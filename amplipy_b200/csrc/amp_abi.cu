@@ -11,6 +11,7 @@
 
 #include "../../include/amplipy_b200.h"
 #include "amp_warp.cuh"
+#include "amp_call.cuh"
 #include "amp_bgzf.cuh"
 #include "amp_ont.cuh"
 #include "amp_deflate.cuh"
@@ -77,196 +78,32 @@ __global__ void __launch_bounds__(AMPO_WARPS * 32, 1) amp_trim_pileup_ont_kernel
 
 __device__ const unsigned char kFixedSyms[8] = {'A', 'C', 'G', 'T', 'N', '-', 0, 0};
 
-__global__ void amp_link_kernel(amp::InsSlot* slots, const unsigned int* entries, const unsigned long long* cursor,
-                                const unsigned char* arena, int* heads) {
-    const unsigned long long n = cursor[1];
-    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n;
-         k += (unsigned long long)gridDim.x * blockDim.x) {
-        const unsigned int s = entries[k];
-        const unsigned char* rec = arena + (slots[s].key & 0xFFFFFFFFFFULL) * 8;
-        const int gpos = ((const int*)rec)[0];
-        slots[s].next = atomicExch(&heads[gpos], (int)s);
-    }
-}
-
-// Calling: sixteen lanes per (sample, position), one allele per lane: lanes 0..5 the fixed symbols A C G T N '-', lanes
-// 6..15 the position's insertion alleles when there are at most ten (with more, the first lane of the group runs the serial
-// form amp::call_position -- the same function the CPU emulation runs for every position).  One float64 division per
-// allele, the allele order (count, then python string order, descending: AmpliPy.py:771) from fifteen shuffles, the
-// position-level facts from ballots.
-#define AMP_CALL_LANES 16
-// Positions with more than ten insertion alleles (indel-rich data: every position of an ONT-like sample): the same
-// results as amp::call_position, with the sixteen lanes of the group sharing the allele list -- lane l owns entries
-// l, l + 16, ... and, for each, walks the whole list once to find its place in the reference's order; the fixed
-// symbols are owned by lanes 0..5.  All lanes walk the same addresses in the same order, so the loads are broadcasts.
-__device__ __forceinline__ bool ins_slot_greater(const amp::CallParams& P, int t, int ct, int c, const amp::Sym& me) {
-    return ct > c || (ct == c && amp::sym_cmp(amp::slot_sym(P, t), me) > 0);
-}
-__device__ __noinline__ void call_long_list(const amp::CallParams& P, long long gp, int sample, int p, int ch, int g0, unsigned gmask) {
-    constexpr int G = AMP_CALL_LANES;
-    const int* cnt = P.counts + (size_t)sample * AMP_NCH * P.Lpad;
-    const int head = P.heads[(size_t)sample * P.Lpad + p];
-    int cfix[AMP_NCH]; long long total = 0;
-#pragma unroll
-    for (int o = 0; o < AMP_NCH; ++o) { cfix[o] = cnt[(size_t)o * P.Lpad + p]; total += cfix[o]; }
-    for (int t = head; t >= 0;) { const amp::InsSlot sl = P.slots[t]; total += sl.count; t = sl.next; }
-    const unsigned char refsym = P.ref_seq[(size_t)sample * (size_t)P.ref_stride + p];
-    int n_alt = 0, alt_fixed = 0;
-    int top_id = -1, top_c = 0;                 // set by the lane that owns the first allele of the order
-    int ref_key = -1, refc = 0; double reff = 0.0;   // 936-937: the last match in visiting order wins
-    if (ch < AMP_NCH) {
-        const int c = cfix[ch];
-        const double f = total ? (double)c / (double)total : 0.0;
-        int rank = -1;
-        if (c) {
-            amp::Sym me; me.p = kFixedSyms + ch; me.len = 1;
-            rank = 0;
-#pragma unroll
-            for (int o = 0; o < AMP_NCH; ++o)
-                if (o != ch && cfix[o]) { amp::Sym os; os.p = kFixedSyms + o; os.len = 1; if (amp::allele_greater(cfix[o], os, c, me)) ++rank; }
-            for (int t = head; t >= 0;) { const amp::InsSlot sl = P.slots[t]; if (sl.count && ins_slot_greater(P, t, sl.count, c, me)) ++rank; t = sl.next; }
-            if (rank == 0) { top_id = ch; top_c = c; }
-            if (kFixedSyms[ch] == refsym) { ref_key = ch; refc = c; reff = f; }
-            else if (f >= P.min_freq_variants) { alt_fixed = 1; ++n_alt; }                        // 938-939
-        }
-        P.fixed_freq[gp * AMP_NCH + ch] = f; P.fixed_rank[gp * AMP_NCH + ch] = rank;
-    }
-    int s = head;
-    for (int k = 0; k < ch && s >= 0; ++k) s = P.slots[s].next;
-    for (int j = ch; s >= 0; j += G) {
-        const int cs = P.slots[s].count;
-        if (cs) {
-            const amp::Sym me = amp::slot_sym(P, s);
-            const double f = (double)cs / (double)total;
-            int rank = 0;
-#pragma unroll
-            for (int o = 0; o < AMP_NCH; ++o)
-                if (cfix[o]) { amp::Sym os; os.p = kFixedSyms + o; os.len = 1; if (amp::allele_greater(cfix[o], os, cs, me)) ++rank; }
-            for (int t = head; t >= 0;) { const amp::InsSlot sl = P.slots[t]; if (t != s && sl.count && ins_slot_greater(P, t, sl.count, cs, me)) ++rank; t = sl.next; }
-            const int kk = P.slot_entry[s];
-            P.ins_freq[kk] = f; P.ins_rank[kk] = rank;
-            if (rank == 0) { top_id = 6 + kk; top_c = cs; }
-            unsigned char is_alt = 0;
-            if (me.len == 1 && me.p[0] == refsym) { if (AMP_NCH + j > ref_key) { ref_key = AMP_NCH + j; refc = cs; reff = f; } }
-            else if (f >= P.min_freq_variants) is_alt = 1;
-            P.ins_alt[kk] = is_alt; n_alt += is_alt;
-        }
-        for (int k = 0; k < G && s >= 0; ++k) s = P.slots[s].next;
-    }
-    // position-level facts
-    const unsigned lanes = (1u << G) - 1u;
-    const unsigned top_m = (__ballot_sync(gmask, top_id >= 0) >> g0) & lanes;
-    const unsigned alt_m = (__ballot_sync(gmask, alt_fixed != 0) >> g0) & lanes;
-    const int top_l = top_m ? __ffs((int)top_m) - 1 : 0;
-    top_id = __shfl_sync(gmask, top_id, g0 + top_l);
-    top_c = __shfl_sync(gmask, top_c, g0 + top_l);
-#pragma unroll
-    for (int d = 1; d < G; d <<= 1) {
-        n_alt += __shfl_xor_sync(gmask, n_alt, d);
-        const int k2 = __shfl_xor_sync(gmask, ref_key, d);
-        const int c2 = __shfl_xor_sync(gmask, refc, d);
-        const double f2 = __shfl_xor_sync(gmask, reff, d);
-        if (k2 > ref_key) { ref_key = k2; refc = c2; reff = f2; }
-    }
-    if (ch == 0) {
-        P.depth[gp] = (int)total;
-        P.top_id[gp] = top_m ? top_id : -1;
-        P.top_count[gp] = top_m ? top_c : 0;
-        unsigned char fl = 0;
-        if (top_m) {
-            const double bf = (double)top_c / (double)total;
-            if (top_c >= P.min_depth_consensus && bf >= P.min_freq_consensus) fl |= 1;            // 928
-        }
-        if (total > 0 && total >= P.min_depth_variants && n_alt != 0) {                           // 940
-            fl |= 2;
-            if (refc >= P.min_depth_variants && reff >= P.min_freq_variants) fl |= 4;             // 948
-        }
-        P.pos_flags[gp] = fl; P.ref_count[gp] = refc; P.alt_mask[gp] = (unsigned char)(alt_m & 0x3Fu);
-    }
-}
-
+// Calling (amp_call.cuh): sixteen lanes per (sample, position)
 __global__ void __launch_bounds__(256) amp_call_kernel(const __grid_constant__ amp::CallParams P) {
-    constexpr int G = AMP_CALL_LANES, NINS = G - AMP_NCH;
     const long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    const long long gp = t / G;
-    const int ch = (int)(t % G);
-    if (gp >= (long long)P.n_samples * P.L) return;             // whole groups: blockDim is a multiple of G
-    const int sample = (int)(gp / P.L), p = (int)(gp - (long long)sample * P.L);
-    const int g0 = threadIdx.x & (32 - G) & 31;               // first lane of this group
-    const unsigned gmask = (G == 32 ? 0xFFFFFFFFu : ((1u << G) - 1u) << g0);
-    // (the fixed symbols' counts and the reference base are independent of the insertion list: loaded first, so that the latencies overlap)
-    const int* cnt = P.counts + (size_t)sample * AMP_NCH * P.Lpad;
-    const int c_fixed = ch < AMP_NCH ? cnt[(size_t)ch * P.Lpad + p] : 0;
-    const unsigned char refsym = P.ref_seq[(size_t)sample * (size_t)P.ref_stride + p];
-    // insertion alleles of the position: lane 6 + j takes the j-th entry of the list
-    int slot = -1, s = P.heads[(size_t)sample * P.Lpad + p];
-    for (int j = 0; j < NINS && s >= 0; ++j) {
-        if (ch == AMP_NCH + j) slot = s;
-        s = P.slots[s].next;
-    }
-    if (s >= 0) {                                             // longer list (uniform within the group)
-        call_long_list(P, gp, sample, p, ch, g0, gmask);
-        return;
-    }
-    int c = c_fixed;
-    amp::Sym me; me.p = kFixedSyms + (ch < AMP_NCH ? ch : 7); me.len = 1;
-    if (ch >= AMP_NCH && slot >= 0) { c = P.slots[slot].count; me = amp::slot_sym(P, slot); }
-    int total = c;
-#pragma unroll
-    for (int d = 1; d < G; d <<= 1) total += __shfl_xor_sync(gmask, total, d);
-    const double f = c ? (double)c / (double)total : 0.0;
-    // index in the sorted allele list = number of alleles that are greater; only alleles that occur take part (one or two at most
-    // positions), so the group walks the set bits of its occupancy mask instead of all sixteen lanes
-    const unsigned lanes = G == 32 ? 0xFFFFFFFFu : (1u << G) - 1u;
-    int rank = 0;
-    for (unsigned occ = (__ballot_sync(gmask, c != 0) >> g0) & lanes; occ; occ &= occ - 1u) {
-        const int o = __ffs((int)occ) - 1;
-        const int co = __shfl_sync(gmask, c, g0 + o);
-        amp::Sym so;
-        so.p = (const unsigned char*)__shfl_sync(gmask, (unsigned long long)me.p, g0 + o);
-        so.len = __shfl_sync(gmask, me.len, g0 + o);
-        if (o != ch && c && amp::allele_greater(co, so, c, me)) ++rank;
-    }
-    if (!c) rank = -1;
-    const bool is_ref = c && me.len == 1 && me.p[0] == refsym;                     // 936-937
-    const bool is_alt = c && !is_ref && f >= P.min_freq_variants;                  // 938-939
-    const unsigned top_m = (__ballot_sync(gmask, rank == 0) >> g0) & lanes;
-    const unsigned ref_m = (__ballot_sync(gmask, is_ref) >> g0) & lanes;
-    const unsigned alt_m = (__ballot_sync(gmask, is_alt) >> g0) & lanes;
-    const int best_l = top_m ? __ffs((int)top_m) - 1 : 0;
-    const int best_c = __shfl_sync(gmask, c, g0 + best_l);
-    const double best_f = __shfl_sync(gmask, f, g0 + best_l);
-    const int kk = slot >= 0 ? P.slot_entry[slot] : -1;       // dense index of the insertion allele (amp_ins_export order)
-    const int best_kk = __shfl_sync(gmask, kk, g0 + best_l);
-    // the reference's loop visits the fixed symbols first, then the insertion alleles: the last match wins (936-937)
-    const int ref_l = ref_m ? 31 - __clz((int)ref_m) : 0;
-    const int refc0 = __shfl_sync(gmask, c, g0 + ref_l);
-    const double reff0 = __shfl_sync(gmask, f, g0 + ref_l);
-    if (ch < AMP_NCH) { P.fixed_freq[gp * AMP_NCH + ch] = f; P.fixed_rank[gp * AMP_NCH + ch] = rank; }
-    else if (slot >= 0 && c) { P.ins_freq[kk] = f; P.ins_rank[kk] = rank; P.ins_alt[kk] = is_alt ? 1 : 0; }
-    if (ch == 0) {
-        const int refc = ref_m ? refc0 : 0;
-        const double reff = ref_m ? reff0 : 0.0;
-        P.depth[gp] = total;
-        P.top_id[gp] = top_m ? (best_l < AMP_NCH ? best_l : 6 + best_kk) : -1;
-        P.top_count[gp] = top_m ? best_c : 0;
-        unsigned char fl = 0;
-        if (top_m && best_c >= P.min_depth_consensus && best_f >= P.min_freq_consensus) fl |= 1;     // 928
-        if (total > 0 && total >= P.min_depth_variants && alt_m != 0) {                             // 940
-            fl |= 2;
-            if (refc >= P.min_depth_variants && reff >= P.min_freq_variants) fl |= 4;               // 948
-        }
-        P.pos_flags[gp] = fl; P.ref_count[gp] = refc; P.alt_mask[gp] = (unsigned char)(alt_m & 0x3Fu);
-    }
+    if (t / AMP_CALL_LANES >= (long long)P.n_samples * P.L) return;   // whole groups: blockDim is a multiple of 16
+    amp::call_thread(P, kFixedSyms, t, (int)(threadIdx.x & 31));
 }
 
-// reset of the insertion table between samples: only the slots that are in use (listed in entries[]) are cleared
-__global__ void amp_clear_slots_kernel(amp::InsSlot* slots, const unsigned int* entries, unsigned long long* cursor) {
+// Reset between samples, one launch: the count matrix (zero) and the list heads (-1) with 16-byte stores, the slots
+// listed in entries[0, cursor[1]) -- the table was zero after amp_create / amp_reset and every slot taken since then is
+// listed there, so clearing those is enough (the full table is tens of MB) -- and, by the last block to finish, the two
+// cursors, the error word and the block counter itself.  Every block reads cursor[1] before it is counted as done.
+__global__ void __launch_bounds__(256) amp_reset_kernel(uint4* counts, unsigned long long counts16, uint4* heads, unsigned long long heads16,
+                                                        amp::InsSlot* slots, const unsigned int* entries, unsigned long long* cursor,
+                                                        unsigned int* err, unsigned int* done) {
     const unsigned long long n = cursor[1];
-    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n;
-         k += (unsigned long long)gridDim.x * blockDim.x) {
+    const unsigned long long tid = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x, nth = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long k = tid; k < counts16; k += nth) counts[k] = make_uint4(0u, 0u, 0u, 0u);
+    for (unsigned long long k = tid; k < heads16; k += nth) heads[k] = make_uint4(~0u, ~0u, ~0u, ~0u);
+    for (unsigned long long k = tid; k < n; k += nth) {
         amp::InsSlot z; z.key = 0; z.count = 0; z.next = 0;
         slots[entries[k]] = z;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        if (atomicAdd(done, 1u) == gridDim.x - 1) { cursor[0] = 0; cursor[1] = 0; *err = 0; *done = 0; }
     }
 }
 
@@ -537,7 +374,7 @@ struct amp_ctx {
     amp::InsTable tab{};
     unsigned long long nslots = 0;
     unsigned int* d_err = nullptr;
-    int* d_heads = nullptr;
+    unsigned int* d_reset_done = nullptr;   // block counter of amp_reset_kernel
     uint32_t* d_scratch = nullptr; size_t scratch_words = 0;
     uint32_t* d_glist = nullptr; size_t glist_words = 0;   // per-CTA generic-read lists of the warp-autonomous kernels
     DevChunk chunk[3];
@@ -761,7 +598,8 @@ int amp_create(const amp_config* cfg, const int32_t* min_primer_start, const int
     CK(cudaMalloc((void**)&c->tab.arena, arena_bytes));
     CK(cudaMalloc((void**)&c->tab.cursor, 16));
     CK(cudaMalloc((void**)&c->d_err, 4));
-    CK(cudaMalloc((void**)&c->d_heads, (size_t)cfg->n_samples * c->Lpad * 4));
+    CK(cudaMalloc((void**)&c->tab.heads, (size_t)cfg->n_samples * c->Lpad * 4));
+    CK(cudaMalloc((void**)&c->d_reset_done, 4));
     c->tab.mask = nslots - 1; c->tab.arena_words = arena_bytes / 8; c->tab.err = c->d_err;
     for (auto& ch : c->chunk) CK(cudaStreamCreateWithFlags(&ch.stream, cudaStreamNonBlocking));
     *out = c;
@@ -777,10 +615,10 @@ int amp_destroy(amp_ctx* c) {
     cudaFree(c->d_min_start); cudaFree(c->d_max_end);
     for (auto& sc : c->scheme) { cudaFree(sc.d_min); cudaFree(sc.d_max); }
     if (c->counts_owned) cudaFree(c->d_counts);
-    cudaFree(c->tab.slots); cudaFree(c->tab.entries); cudaFree(c->tab.slot_entry); cudaFree(c->tab.arena); cudaFree(c->tab.cursor);
+    cudaFree(c->tab.slots); cudaFree(c->tab.entries); cudaFree(c->tab.slot_entry); cudaFree(c->tab.arena); cudaFree(c->tab.cursor); cudaFree(c->tab.heads);
     if (c->defl.stream) cudaStreamDestroy(c->defl.stream);
     cudaFree(c->defl.in); cudaFree(c->defl.slots); cudaFree(c->defl.out); cudaFree(c->defl.bstart); cudaFree(c->defl.off); cudaFree(c->defl.clen); cudaFree(c->defl.crc); cudaFree(c->defl.ctr); cudaFree(c->defl.toks);
-    cudaFree(c->d_err); cudaFree(c->d_heads); cudaFree(c->d_scratch); cudaFree(c->d_glist); cudaFree(c->d_ref); cudaFree(c->d_call); cudaFree(c->d_xbuf);
+    cudaFree(c->d_err); cudaFree(c->d_reset_done); cudaFree(c->d_scratch); cudaFree(c->d_glist); cudaFree(c->d_ref); cudaFree(c->d_call); cudaFree(c->d_xbuf);
     {
         auto& d = c->dec;
         void* ps[] = {d.comp, d.raw, d.in_off, d.out_off, d.out_len, d.tot, d.prefix, d.ctr, d.pos, d.flag, d.tlen, d.cig_off, d.seq_off, d.qual_off,
@@ -804,8 +642,10 @@ int amp_reset(amp_ctx* c) {
     CK(cudaSetDevice(c->cfg.device));
     CK(cudaMemsetAsync(c->d_counts, 0, (size_t)c->cfg.n_samples * AMP_NCH * c->Lpad * 4, 0));
     CK(cudaMemsetAsync(c->tab.slots, 0, c->nslots * sizeof(amp::InsSlot), 0));
+    CK(cudaMemsetAsync(c->tab.heads, 0xFF, (size_t)c->cfg.n_samples * c->Lpad * 4, 0));
     CK(cudaMemsetAsync(c->tab.cursor, 0, 16, 0));
     CK(cudaMemsetAsync(c->d_err, 0, 4, 0));
+    CK(cudaMemsetAsync(c->d_reset_done, 0, 4, 0));
     CK(cudaStreamSynchronize(0));
     return AMP_OK;
 }
@@ -813,14 +653,13 @@ int amp_reset(amp_ctx* c) {
 int amp_reset_async(amp_ctx* c, void* stream) {
     if (!c) return fail(AMP_ERR_ARG, "amp_reset_async: null context");
     CK(cudaSetDevice(c->cfg.device));
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(cudaMemsetAsync(c->d_counts, 0, (size_t)c->cfg.n_samples * AMP_NCH * c->Lpad * 4, st));
-    // the table was zero after amp_create / amp_reset and every slot taken since then is listed in entries[]:
-    // clearing those is enough (the full table is tens of MB)
-    amp_clear_slots_kernel<<<c->sm_count, 256, 0, st>>>(c->tab.slots, c->tab.entries, c->tab.cursor);
+    // counts: n_samples * 6 * Lpad ints and heads: n_samples * Lpad ints, Lpad a multiple of 32 -- whole 16-byte words
+    const unsigned long long counts16 = (unsigned long long)c->cfg.n_samples * AMP_NCH * c->Lpad / 4;
+    const unsigned long long heads16 = (unsigned long long)c->cfg.n_samples * c->Lpad / 4;
+    const unsigned long long grid = std::min<unsigned long long>((counts16 + 255) / 256, (unsigned long long)c->sm_count * 8);
+    amp_reset_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>((uint4*)c->d_counts, counts16, (uint4*)c->tab.heads, heads16,
+                                                                       c->tab.slots, c->tab.entries, c->tab.cursor, c->d_err, c->d_reset_done);
     CK(cudaGetLastError());
-    CK(cudaMemsetAsync(c->tab.cursor, 0, 16, st));
-    CK(cudaMemsetAsync(c->d_err, 0, 4, st));
     return AMP_OK;
 }
 
@@ -961,6 +800,7 @@ int amp_counts_device(amp_ctx* c, int32_t** dev_counts) {
 
 int amp_bind_counts(amp_ctx* c, int32_t* dev_counts) {
     if (!c || !dev_counts) return fail(AMP_ERR_ARG, "amp_bind_counts: null argument");
+    if ((uintptr_t)dev_counts & 15) return fail(AMP_ERR_ARG, "amp_bind_counts: the buffer must be 16-byte aligned");
     CK(cudaSetDevice(c->cfg.device));
     CK(cudaDeviceSynchronize());
     if (c->counts_owned) CK(cudaFree(c->d_counts));
@@ -1084,13 +924,10 @@ int amp_call_device(amp_ctx* c, const amp_call_params* p, void* stream) {
         CK(cudaMalloc((void**)&c->d_call, bytes + 256));
     }
     c->last_launches = 0;
-    CK(cudaMemsetAsync(c->d_heads, 0xFF, S * c->Lpad * 4, st));
-    amp_link_kernel<<<c->sm_count * 4, 256, 0, st>>>(c->tab.slots, c->tab.entries, c->tab.cursor, c->tab.arena, c->d_heads);
-    CK(cudaGetLastError());
     unsigned char* blk = c->d_call;
     amp::CallParams P{};
     P.L = (int)L; P.Lpad = c->Lpad; P.n_samples = (int)S; P.counts = c->d_counts; P.slots = c->tab.slots;
-    P.slot_entry = c->tab.slot_entry; P.arena = c->tab.arena; P.heads = c->d_heads; P.ref_seq = c->d_ref;
+    P.slot_entry = c->tab.slot_entry; P.arena = c->tab.arena; P.heads = c->tab.heads; P.ref_seq = c->d_ref;
     P.ref_stride = c->ref_per_sample ? (long long)c->cfg.ref_len : 0;
     P.min_depth_consensus = p->min_depth_consensus; P.min_freq_consensus = p->min_freq_consensus;
     P.min_depth_variants = p->min_depth_variants; P.min_freq_variants = p->min_freq_variants;
@@ -1098,9 +935,10 @@ int amp_call_device(amp_ctx* c, const amp_call_params* p, void* stream) {
     P.pos_flags = blk + c->o_fl; P.ref_count = (int*)(blk + c->o_refc); P.fixed_freq = (double*)(blk + c->o_ff);
     P.fixed_rank = (int*)(blk + c->o_fr); P.alt_mask = blk + c->o_alt; P.ins_freq = (double*)(blk + c->o_if);
     P.ins_rank = (int*)(blk + c->o_ir); P.ins_alt = blk + c->o_ia;
+    // the insertion lists are current: ins_table_add links every allele it creates
     amp_call_kernel<<<(unsigned)((SL * AMP_CALL_LANES + 255) / 256), 256, 0, st>>>(P);
     CK(cudaGetLastError());
-    c->last_launches = 2;
+    c->last_launches = 1;
     return AMP_OK;
 }
 

@@ -40,6 +40,11 @@ struct uint4 { unsigned int x, y, z, w; };   // host emulation build only
 
 #define AMP_PRAGMA_X(x) _Pragma(#x)
 #define AMP_UNROLL_N(n) AMP_PRAGMA_X(unroll n)
+#if defined(__CUDACC__)
+#define AMP_UNROLL AMP_PRAGMA_X(unroll)
+#else
+#define AMP_UNROLL
+#endif
 
 namespace amp {
 
@@ -823,7 +828,7 @@ AMP_HD int nib_channel(uint32_t nib) {
 }
 
 // ---- insertion-allele hash table ------------------------------------------------------------------
-// slot  : key64 = [tag:24 | arena offset in 8-byte words:40] (0 = empty), count32
+// slot  : key64 = [tag:24 | arena offset in 8-byte words:40] (0 = empty), count32, next = the position's next allele (-1 = last)
 // arena : records {int32 gpos; uint32 len; char text[len]} padded to 8 bytes, write-once
 // Lookups compare the full text, so the hash is only a filter: results are exact.
 struct InsSlot { unsigned long long key; int count; int next; };
@@ -834,6 +839,8 @@ struct InsTable {
     unsigned char* arena; unsigned long long arena_words;
     unsigned long long* cursor;                      // [0] = arena words used, [1] = entries used
     unsigned int* err;
+    int* heads;                                      // [n_samples * Lpad] first slot of the position's allele list, -1 = none;
+                                                     // null: no lists kept (a table whose user links them when it reads them)
 };
 AMP_HD unsigned long long mix64(unsigned long long h) {
     h ^= h >> 30; h *= 0xBF58476D1CE4E5B9ULL; h ^= h >> 27; h *= 0x94D049BB133111EBULL; h ^= h >> 31; return h;
@@ -889,6 +896,9 @@ AMP_HD_NOINLINE void ins_table_add(const InsTable& T, int gpos, int len, const T
                 atomic_add(&T.slots[slot].count, n);
                 const unsigned long long k_new = atomic_add64_warp(&T.cursor[1], 1ULL);
                 T.entries[k_new] = (unsigned int)slot; T.slot_entry[slot] = (int)k_new;
+                // the allele joins its position's list here, where it is created, so the lists are current after every
+                // launch that adds alleles; their order is that of the exchanges (calling does not depend on it)
+                if (T.heads) T.slots[slot].next = atomic_exch(&T.heads[gpos], (int)slot);
                 return;
             }
             k = old;

@@ -651,12 +651,13 @@ AMP_HD void cta_trim_pileup(const KParams& P, unsigned char* smem_base, int bloc
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Calling (AmpliPy.py:756-771, 919-951).  One thread per (sample, position).
+// Calling (AmpliPy.py:756-771, 919-951): the serial form, one thread per (sample, position); the CPU emulation's reference
+// for the kernel's body (amp_call.cuh).
 // ---------------------------------------------------------------------------------------------------
 struct CallParams {
     int L, Lpad, n_samples;
     const int* counts;                 // [n_samples][6][Lpad]
-    const InsSlot* slots;              // insertion table (heads[] / next chains built by link_insertions)
+    const InsSlot* slots;              // insertion table (heads[] / next chains: InsTable, linked by ins_table_add)
     const int* slot_entry;             // slot -> dense allele index k (amp_ins_export order)
     const unsigned char* arena;
     const int* heads;                  // [n_samples * Lpad] slot index of the first insertion allele, -1 = none

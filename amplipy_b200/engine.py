@@ -196,7 +196,7 @@ class Engine:
 
     def reset_async(self, stream=None):
         _check(self.lib.amp_reset_async(self._ctx, ctypes.c_void_p(stream) if stream else None), "amp_reset_async")
-        self.launches += 1            # amp_clear_slots_kernel (the other resets are memsets)
+        self.launches += 1            # amp_reset_kernel
 
     def set_reference(self, ref_seq):
         ref = ref_seq.encode("latin-1") if isinstance(ref_seq, str) else bytes(ref_seq)
