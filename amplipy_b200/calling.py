@@ -46,8 +46,9 @@ class CallResult:
     ins_alt: np.ndarray
 
 
-def consensus_string(res: CallResult, ins: Insertions, sample=0, unknown_symbol="N") -> str:
-    """''.join(consensus_symbols) of AmpliPy.py:920-929, 960."""
+def consensus_string(res: CallResult, ins: Insertions, sample=0, unknown_symbol="N", iupac=None) -> str:
+    """''.join(consensus_symbols) of AmpliPy.py:920-929, 960.  ``iupac``: the IUPAC codes of Engine.call_ivar ([S*L], 0 = keep
+    the reference's symbol) replace the symbols of the positions that pass the consensus gate."""
     L = res.L
     sl = slice(sample * L, (sample + 1) * L)
     top = res.top_id[sl]
@@ -55,6 +56,10 @@ def consensus_string(res: CallResult, ins: Insertions, sample=0, unknown_symbol=
     table = np.frombuffer((FIXED_SYMS + unknown_symbol).encode(), np.uint8)
     idx = np.where(ok & (top >= 0) & (top < 6), top, 6)
     chars = table[idx]
+    if iupac is not None:
+        amb = ok & (iupac[sl] != 0)
+        chars = np.where(amb, iupac[sl], chars).astype(np.uint8)
+        ok = ok & ~amb
     multi = np.flatnonzero(ok & (top >= 6))
     if multi.size == 0:
         return chars.tobytes().decode()

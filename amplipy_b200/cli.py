@@ -8,7 +8,7 @@ import os
 import sys
 from datetime import datetime
 
-from . import alnio, calling, vcf
+from . import alnio, calling, ivar, vcf
 from .primers import InputError, find_overlapping_primers, load_primers, max_primer_len
 
 VERSION = "0.0.2"
@@ -54,6 +54,9 @@ HELP_TEXT_TRIM_PRIMER_POS_OFFSET = ("Primer position offset. Reads that occur at
 HELP_TEXT_TRIM_SLIDING_WINDOW_WIDTH = "Width of sliding window (average quality of this window must be >= minimum quality threshold)"
 HELP_TEXT_UNKNOWN_SYMBOL = "Character to print in regions with less than minimum coverage"
 HELP_TEXT_VARIANTS = "Variant Calls (VCF)"
+HELP_TEXT_TSV = "Variant Calls in iVar's TSV format, with strand counts, mean qualities and Fisher p-values (optional)"
+HELP_TEXT_IUPAC_THRESHOLD = ("Write IUPAC ambiguity codes: the shortest prefix of the sorted alleles whose frequencies reach this "
+                             "threshold (0-1) is coded (optional; 0 = the plain consensus)")
 
 
 def print_log(s='', end='\n'):
@@ -92,6 +95,7 @@ def parse_args(argv=None):
     v.add_argument('-mq', '--min_quality', required=False, type=int, default=DEFAULT_MIN_QUALITY, help=HELP_TEXT_MIN_QUAL)
     v.add_argument('-mf', '--min_freq', required=False, type=float, default=DEFAULT_MIN_FREQ_VARIANTS, help=HELP_TEXT_MIN_FREQ_VARIANTS)
     v.add_argument('-md', '--min_depth', required=False, type=int, default=DEFAULT_MIN_DEPTH_VARIANTS, help=HELP_TEXT_MIN_DEPTH_VARIANTS)
+    v.add_argument('--output_tsv', required=False, type=str, default=None, help=HELP_TEXT_TSV)
 
     c = sub.add_parser("consensus", description=DESCRIPTION, formatter_class=F)
     c.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_TRIMMED)
@@ -101,6 +105,7 @@ def parse_args(argv=None):
     c.add_argument('-mf', '--min_freq', required=False, type=float, default=DEFAULT_MIN_FREQ_CONSENSUS, help=HELP_TEXT_MIN_FREQ_CONSENSUS)
     c.add_argument('-md', '--min_depth', required=False, type=int, default=DEFAULT_MIN_DEPTH_CONSENSUS, help=HELP_TEXT_MIN_DEPTH_CONSENSUS)
     c.add_argument('-n', '--unknown_symbol', required=False, type=str, default=DEFAULT_UNKNOWN_SYMBOL, help=HELP_TEXT_UNKNOWN_SYMBOL)
+    c.add_argument('--iupac_threshold', required=False, type=float, default=None, help=HELP_TEXT_IUPAC_THRESHOLD)
 
     a = sub.add_parser("aio", description=DESCRIPTION, formatter_class=F)
     a.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_UNTRIMMED)
@@ -119,6 +124,8 @@ def parse_args(argv=None):
     a.add_argument('-mdv', '--min_depth_variants', required=False, type=int, default=DEFAULT_MIN_DEPTH_VARIANTS, help=HELP_TEXT_MIN_DEPTH_VARIANTS)
     a.add_argument('-n', '--unknown_symbol', required=False, type=str, default=DEFAULT_UNKNOWN_SYMBOL, help=HELP_TEXT_UNKNOWN_SYMBOL)
     a.add_argument('-e', '--include_no_primer', action='store_true', help=HELP_TEXT_TRIM_INCLUDE_READS_NO_PRIMER)
+    a.add_argument('--output_tsv', required=False, type=str, default=None, help=HELP_TEXT_TSV)
+    a.add_argument('--iupac_threshold', required=False, type=float, default=None, help=HELP_TEXT_IUPAC_THRESHOLD)
     return parser.parse_args(argv)
 
 
@@ -141,20 +148,23 @@ def run_amplipy(untrimmed_reads_fn=None, primer_fn=None, reference_fn=None, trim
                 consensus_fn=None, primer_pos_offset=None, min_length=None, min_quality=None, sliding_window_width=None,
                 min_freq_consensus=None, min_freq_variants=None, min_depth_consensus=None, min_depth_variants=None,
                 unknown_symbol=None, include_no_primer=None, run_trim=False, run_variants=False, run_consensus=False,
-                argv=None, device=0):
-    """Same keyword arguments and behaviour as the reference's run_amplipy (AmpliPy.py:774-963)."""
+                argv=None, device=0, tsv_fn=None, iupac_threshold=None):
+    """Same keyword arguments and behaviour as the reference's run_amplipy (AmpliPy.py:774-963).  Two additions of this
+    project: ``tsv_fn`` (with run_variants) also writes the variants in iVar's TSV format, ``iupac_threshold`` (with
+    run_consensus) writes IUPAC ambiguity codes into the consensus (DESIGN.md 3.7)."""
     argv = list(sys.argv if argv is None else argv)
     try:
         return _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
                     min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
-                    min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device)
+                    min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
+                    tsv_fn if run_variants else None, iupac_threshold if run_consensus else None)
     except InputError as e:
         error(str(e))
 
 
 def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
          min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
-         unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device):
+         unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn=None, iupac_threshold=None):
     # validity checks (AmpliPy.py:837-854)
     if primer_pos_offset is not None and primer_pos_offset < 0:
         error("%s: %s" % (ERROR_TEXT_NEGATIVE_PRIMER_POS_OFFSET, primer_pos_offset))
@@ -174,6 +184,8 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         error("%s: %s" % (ERROR_TEXT_INVALID_MIN_DEPTH, min_depth_variants))
     if unknown_symbol is not None and len(unknown_symbol) != 1:
         error("%s: %s" % (ERROR_TEXT_INVALID_UNKNOWN_SYMBOL_LENGTH, unknown_symbol))
+    if iupac_threshold is not None and not (0 <= iupac_threshold <= 1):
+        error("%s: %s" % (ivar.ERROR_TEXT_INVALID_IUPAC_THRESHOLD, iupac_threshold))
 
     # mode banner (AmpliPy.py:857-866)
     if not (run_trim or run_variants or run_consensus):
@@ -207,18 +219,26 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
     if variants_fn is not None:
         print_log("Output variants VCF: %s" % variants_fn)
         vcf.check_output_path(variants_fn)
+    if tsv_fn is not None:
+        print_log("Output variants TSV: %s" % tsv_fn)
+        ivar.check_output_path(tsv_fn)
     import threading
     import time as _time
     tm = {}
     from .engine import AmpError, Engine, TrimResult
 
+    qstats = tsv_fn is not None      # the strand / quality pass runs only for the TSV
+
     def make_engine(indel_rich):
-        return Engine(ref_len=L, primer_tables=tables, max_primer_len=mpl,
-                      min_quality=DEFAULT_MIN_QUALITY if min_quality is None else min_quality,
-                      sliding_window_width=DEFAULT_SLIDING_WINDOW_WIDTH if sliding_window_width is None else sliding_window_width,
-                      min_length=DEFAULT_MIN_LENGTH if min_length is None else min_length,
-                      include_no_primer=bool(include_no_primer), device=device,
-                      ins_slots=(1 << 24) if indel_rich else 0, ins_arena_bytes=(1 << 30) if indel_rich else 0)
+        e = Engine(ref_len=L, primer_tables=tables, max_primer_len=mpl,
+                   min_quality=DEFAULT_MIN_QUALITY if min_quality is None else min_quality,
+                   sliding_window_width=DEFAULT_SLIDING_WINDOW_WIDTH if sliding_window_width is None else sliding_window_width,
+                   min_length=DEFAULT_MIN_LENGTH if min_length is None else min_length,
+                   include_no_primer=bool(include_no_primer), device=device,
+                   ins_slots=(1 << 24) if indel_rich else 0, ins_arena_bytes=(1 << 30) if indel_rich else 0)
+        if qstats or iupac_threshold is not None:
+            e.enable_qstats()
+        return e
     pile = run_variants or run_consensus
     _t = _time.perf_counter()
     aln = eng = trim = None
@@ -249,7 +269,7 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         print_log("Processing reads...")
         try:
             info = eng.decode_bam(raw, layout)
-            outs = eng.process_decoded(trim=run_trim, pileup=pile, download=not dev_bam_out)
+            outs = eng.process_decoded(trim=run_trim, pileup=pile, download=not dev_bam_out, **({"qstats": True} if qstats else {}))
             n_reads = info["n"]
         except AmpError:
             eng.close()
@@ -276,7 +296,7 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         eng = make_engine(indel_rich)
         print_log("Processing reads...")
         _t = _time.perf_counter()
-        trim = eng.process(aln.batch, trim=run_trim, pileup=pile)
+        trim = eng.process(aln.batch, trim=run_trim, pileup=pile, **({"qstats": True} if qstats else {}))
         eng.raise_on_device_errors()
         tm["gpu_process"] = _time.perf_counter() - _t
         n_reads = aln.n
@@ -314,8 +334,17 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
                        DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants)
         if run_variants:
             vcf.write_vcf(variants_fn, ref_id, VERSION, argv, calling.variant_records(res, ins, ref_seq, counts))
+        if tsv_fn is not None:
+            iv = eng.call_ivar(DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
+                               DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants)
+            ivar.write_tsv(tsv_fn, ivar.tsv_rows(res, ins, iv, eng.qstats(0), ref_id, ref_seq, counts))
+        iupac = None
+        if iupac_threshold is not None:
+            iupac = eng.call_ivar(DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
+                                  DEFAULT_MIN_FREQ_CONSENSUS if min_freq_consensus is None else min_freq_consensus,
+                                  iupac_threshold).iupac
         if run_consensus:
-            text = '>sample\n%s\n' % calling.consensus_string(res, ins, 0, unknown_symbol)
+            text = '>sample\n%s\n' % calling.consensus_string(res, ins, 0, unknown_symbol, iupac=iupac)
             if consensus_fn.lower() == 'stdout':
                 sys.stdout.write(text)
             elif consensus_fn.lower().endswith('.gz'):
@@ -348,11 +377,11 @@ def main(argv=None):
     elif args.command == 'variants':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, variants_fn=args.output,
                     min_quality=args.min_quality, min_freq_variants=args.min_freq, min_depth_variants=args.min_depth,
-                    run_variants=True, argv=full_argv)
+                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv)
     elif args.command == 'consensus':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, consensus_fn=args.output,
                     min_quality=args.min_quality, min_freq_consensus=args.min_freq, min_depth_consensus=args.min_depth,
-                    unknown_symbol=args.unknown_symbol, run_consensus=True, argv=full_argv)
+                    unknown_symbol=args.unknown_symbol, run_consensus=True, argv=full_argv, iupac_threshold=args.iupac_threshold)
     elif args.command == 'aio':
         run_amplipy(untrimmed_reads_fn=args.input, primer_fn=args.primer, reference_fn=args.reference,
                     trimmed_reads_fn=args.output_trimmed_reads, variants_fn=args.output_variants,
@@ -361,7 +390,8 @@ def main(argv=None):
                     min_freq_consensus=args.min_freq_consensus, min_freq_variants=args.min_freq_variants,
                     min_depth_consensus=args.min_depth_consensus, min_depth_variants=args.min_depth_variants,
                     unknown_symbol=args.unknown_symbol, include_no_primer=args.include_no_primer, run_trim=True,
-                    run_variants=True, run_consensus=True, argv=full_argv)
+                    run_variants=True, run_consensus=True, argv=full_argv, tsv_fn=args.output_tsv,
+                    iupac_threshold=args.iupac_threshold)
 
 
 if __name__ == "__main__":

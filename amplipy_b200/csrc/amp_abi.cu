@@ -15,9 +15,11 @@
 #include "amp_bgzf.cuh"
 #include "amp_ont.cuh"
 #include "amp_deflate.cuh"
+#include "amp_ivar.cuh"
 
 static_assert(AMP_F_TRIM_START == AMP_FLAG_TRIM_START && AMP_F_KEEP == AMP_FLAG_KEEP && AMP_F_SKIPPED == AMP_FLAG_SKIPPED &&
-                  AMP_F_ERROR == AMP_FLAG_ERROR && AMP_E_ARENA_FULL == AMP_DEVERR_ARENA_FULL,
+                  AMP_F_ERROR == AMP_FLAG_ERROR && AMP_E_ARENA_FULL == AMP_DEVERR_ARENA_FULL &&
+                  AMP_E_QSTATS_MISS == AMP_DEVERR_QSTATS_MISS,
               "flag constants out of sync with include/amplipy_b200.h");
 static_assert(sizeof(amp::Seg) == 16 && sizeof(amp::InsSlot) == 16, "layout");
 
@@ -85,20 +87,48 @@ __global__ void __launch_bounds__(256) amp_call_kernel(const __grid_constant__ a
     amp::call_thread(P, kFixedSyms, t, (int)(threadIdx.x & 31));
 }
 
+// Strand / quality pass (amp_ivar.cuh): one CTA per AMP_QS_READS reads, after the fused kernel on the same stream
+__global__ void __launch_bounds__(AMP_QS_READS) amp_qstats_kernel(const __grid_constant__ amp::QStatsParams P) {
+    __shared__ int trev[AMP_NCH * AMP_QS_WT], tq[AMP_NCH * AMP_QS_WT];
+    __shared__ int lo;
+    amp::cta_qstats(P, trev, tq, &lo, (int)blockIdx.x, (int)blockDim.x);
+}
+
+// iVar calling (amp_ivar.cuh): one thread per (sample, position), after amp_call_kernel on its outputs
+__global__ void __launch_bounds__(256) amp_ivar_kernel(const __grid_constant__ amp::IvarParams P) {
+    const long long gp = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (gp < (long long)P.n_samples * P.L) amp::ivar_position(P, gp);
+}
+
+// the per-slot stats of the insertion alleles in amp_ins_export order
+__global__ void amp_qstats_gather_kernel(const unsigned int* entries, unsigned long long n, const int* ins_rev, const unsigned long long* ins_qsum,
+                                         const unsigned char* ins_head, int* o_rev, unsigned long long* o_qsum, unsigned char* o_head) {
+    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n; k += (unsigned long long)gridDim.x * blockDim.x) {
+        const unsigned int s = entries[k];
+        o_rev[k] = ins_rev[s]; o_qsum[k] = ins_qsum[s]; o_head[k] = ins_head[s];
+    }
+}
+
 // Reset between samples, one launch: the count matrix (zero) and the list heads (-1) with 16-byte stores, the slots
 // listed in entries[0, cursor[1]) -- the table was zero after amp_create / amp_reset and every slot taken since then is
 // listed there, so clearing those is enough (the full table is tens of MB) -- and, by the last block to finish, the two
 // cursors, the error word and the block counter itself.  Every block reads cursor[1] before it is counted as done.
+// STATS: the strand / quality sums are enabled; their per-position sums and the listed slots' sums are zeroed too.
+template <bool STATS>
 __global__ void __launch_bounds__(256) amp_reset_kernel(uint4* counts, unsigned long long counts16, uint4* heads, unsigned long long heads16,
                                                         amp::InsSlot* slots, const unsigned int* entries, unsigned long long* cursor,
-                                                        unsigned int* err, unsigned int* done) {
+                                                        unsigned int* err, unsigned int* done, uint4* rev, uint4* qsum, unsigned long long stats16,
+                                                        int* ins_rev, unsigned long long* ins_qsum, unsigned char* ins_head) {
     const unsigned long long n = cursor[1];
     const unsigned long long tid = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x, nth = (unsigned long long)gridDim.x * blockDim.x;
     for (unsigned long long k = tid; k < counts16; k += nth) counts[k] = make_uint4(0u, 0u, 0u, 0u);
     for (unsigned long long k = tid; k < heads16; k += nth) heads[k] = make_uint4(~0u, ~0u, ~0u, ~0u);
+    if (STATS)
+        for (unsigned long long k = tid; k < stats16; k += nth) { rev[k] = make_uint4(0u, 0u, 0u, 0u); qsum[2 * k] = qsum[2 * k + 1] = make_uint4(0u, 0u, 0u, 0u); }
     for (unsigned long long k = tid; k < n; k += nth) {
         amp::InsSlot z; z.key = 0; z.count = 0; z.next = 0;
         slots[entries[k]] = z;
+        if (STATS) { ins_rev[entries[k]] = 0; ins_qsum[entries[k]] = 0; ins_head[entries[k]] = 0; }
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -409,6 +439,11 @@ struct amp_ctx {
     unsigned char* d_ref = nullptr;     // reference characters (amp_set_reference)
     unsigned char* d_call = nullptr;    // calling outputs (one block, offsets below)
     size_t o_depth = 0, o_top = 0, o_topc = 0, o_fl = 0, o_refc = 0, o_ff = 0, o_fr = 0, o_alt = 0, o_if = 0, o_ir = 0, o_ia = 0;
+    // strand / quality stats (amp_qstats_enable): [n_samples][6][Lpad] sums and per-slot sums of the insertion alleles
+    int* d_rev = nullptr; unsigned long long* d_qsum = nullptr;
+    int* d_ins_rev = nullptr; unsigned long long* d_ins_qsum = nullptr; unsigned char* d_ins_head = nullptr;
+    unsigned char* d_ivar = nullptr;    // iVar calling outputs (one block, offsets below)
+    size_t o_iu = 0, o_fmq = 0, o_fpv = 0, o_imq = 0, o_ipv = 0;
 };
 
 namespace {
@@ -431,8 +466,8 @@ bool has_scheme(const amp_ctx* c, int sample) {
 // words of the per-CTA generic-read lists + their counters for a launch over n reads
 size_t glist_words_for(const amp_ctx* c, long long n) { return (size_t)n + 33 * ((size_t)c->sm_count + 1) + (size_t)c->sm_count + 64; }
 
-int launch_process(amp_ctx* c, const amp::BatchPtrs& b, long long sum_cig, long long max_cig, long long sum_qual, int mode,
-                   int sample, const amp::TrimOut& o, uint32_t* scratch, uint32_t* glist, cudaStream_t st) {
+int launch_fused(amp_ctx* c, const amp::BatchPtrs& b, long long sum_cig, long long max_cig, long long sum_qual, int mode,
+                 int sample, const amp::TrimOut& o, uint32_t* scratch, uint32_t* glist, cudaStream_t st) {
     if (b.n <= 0) return AMP_OK;
     amp::KParams P{};
     P.b = b; P.o = o;
@@ -443,7 +478,7 @@ int launch_process(amp_ctx* c, const amp::BatchPtrs& b, long long sum_cig, long 
         P.tp.L = sc.L; P.tp.min_primer_start = sc.d_min; P.tp.max_primer_end = sc.d_max; P.tp.max_primer_len = sc.mpl;
     } P.tp.min_quality = c->cfg.min_quality; P.tp.window = c->cfg.sliding_window;
     P.tp.min_length = c->cfg.min_length; P.tp.include_no_primer = c->cfg.include_no_primer;
-    P.mode = mode;
+    P.mode = mode & (AMP_MODE_TRIM | AMP_MODE_PILEUP);
     P.counts = c->d_counts + (size_t)sample * AMP_NCH * c->Lpad;
     P.Lpad = c->Lpad; P.gpos_base = sample * c->Lpad;
     P.tab = c->tab; P.err = c->d_err;
@@ -560,6 +595,32 @@ int launch_process(amp_ctx* c, const amp::BatchPtrs& b, long long sum_cig, long 
     return AMP_OK;
 }
 
+// the fused kernel, then (AMP_MODE_QSTATS) the strand / quality pass over the same reads on the same stream
+int launch_process(amp_ctx* c, const amp::BatchPtrs& b, long long sum_cig, long long max_cig, long long sum_qual, int mode,
+                   int sample, const amp::TrimOut& o, uint32_t* scratch, uint32_t* glist, cudaStream_t st) {
+    int rc = launch_fused(c, b, sum_cig, max_cig, sum_qual, mode, sample, o, scratch, glist, st);
+    if (rc || !(mode & AMP_MODE_QSTATS) || b.n <= 0) return rc;
+    amp::QStatsParams Q{};
+    Q.b = b; Q.o = o; Q.trimmed = (mode & AMP_MODE_TRIM) ? 1 : 0;
+    Q.L = c->cfg.ref_len;
+    if ((size_t)sample < c->scheme.size() && c->scheme[sample].L > 0) Q.L = c->scheme[sample].L;   // as launch_fused
+    Q.Lpad = c->Lpad; Q.minq = c->cfg.min_quality; Q.gpos_base = sample * c->Lpad;
+    Q.rev = c->d_rev + (size_t)sample * AMP_NCH * c->Lpad; Q.qsum = c->d_qsum + (size_t)sample * AMP_NCH * c->Lpad;
+    Q.tab = c->tab; Q.ins_rev = c->d_ins_rev; Q.ins_qsum = c->d_ins_qsum; Q.ins_head = c->d_ins_head; Q.err = c->d_err;
+    amp_qstats_kernel<<<(unsigned)((b.n + AMP_QS_READS - 1) / AMP_QS_READS), AMP_QS_READS, 0, st>>>(Q);
+    CK(cudaGetLastError());
+    c->last_launches += 1;
+    return AMP_OK;
+}
+
+// AMP_MODE_QSTATS needs AMP_MODE_PILEUP and amp_qstats_enable
+int check_qstats_mode(const amp_ctx* c, int mode, const char* who) {
+    if (!(mode & AMP_MODE_QSTATS)) return AMP_OK;
+    if (!(mode & AMP_MODE_PILEUP)) return fail(AMP_ERR_ARG, who, "AMP_MODE_QSTATS needs AMP_MODE_PILEUP");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, who, "AMP_MODE_QSTATS needs amp_qstats_enable first");
+    return AMP_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -618,6 +679,7 @@ int amp_destroy(amp_ctx* c) {
     cudaFree(c->tab.slots); cudaFree(c->tab.entries); cudaFree(c->tab.slot_entry); cudaFree(c->tab.arena); cudaFree(c->tab.cursor); cudaFree(c->tab.heads);
     if (c->defl.stream) cudaStreamDestroy(c->defl.stream);
     cudaFree(c->defl.in); cudaFree(c->defl.slots); cudaFree(c->defl.out); cudaFree(c->defl.bstart); cudaFree(c->defl.off); cudaFree(c->defl.clen); cudaFree(c->defl.crc); cudaFree(c->defl.ctr); cudaFree(c->defl.toks);
+    cudaFree(c->d_rev); cudaFree(c->d_qsum); cudaFree(c->d_ins_rev); cudaFree(c->d_ins_qsum); cudaFree(c->d_ins_head); cudaFree(c->d_ivar);
     cudaFree(c->d_err); cudaFree(c->d_reset_done); cudaFree(c->d_scratch); cudaFree(c->d_glist); cudaFree(c->d_ref); cudaFree(c->d_call); cudaFree(c->d_xbuf);
     {
         auto& d = c->dec;
@@ -646,6 +708,12 @@ int amp_reset(amp_ctx* c) {
     CK(cudaMemsetAsync(c->tab.cursor, 0, 16, 0));
     CK(cudaMemsetAsync(c->d_err, 0, 4, 0));
     CK(cudaMemsetAsync(c->d_reset_done, 0, 4, 0));
+    if (c->d_rev) {
+        const size_t n = (size_t)c->cfg.n_samples * AMP_NCH * c->Lpad;
+        CK(cudaMemsetAsync(c->d_rev, 0, n * 4, 0)); CK(cudaMemsetAsync(c->d_qsum, 0, n * 8, 0));
+        CK(cudaMemsetAsync(c->d_ins_rev, 0, c->nslots * 4, 0)); CK(cudaMemsetAsync(c->d_ins_qsum, 0, c->nslots * 8, 0));
+        CK(cudaMemsetAsync(c->d_ins_head, 0, c->nslots, 0));
+    }
     CK(cudaStreamSynchronize(0));
     return AMP_OK;
 }
@@ -657,8 +725,10 @@ int amp_reset_async(amp_ctx* c, void* stream) {
     const unsigned long long counts16 = (unsigned long long)c->cfg.n_samples * AMP_NCH * c->Lpad / 4;
     const unsigned long long heads16 = (unsigned long long)c->cfg.n_samples * c->Lpad / 4;
     const unsigned long long grid = std::min<unsigned long long>((counts16 + 255) / 256, (unsigned long long)c->sm_count * 8);
-    amp_reset_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>((uint4*)c->d_counts, counts16, (uint4*)c->tab.heads, heads16,
-                                                                       c->tab.slots, c->tab.entries, c->tab.cursor, c->d_err, c->d_reset_done);
+    auto* k = c->d_rev ? amp_reset_kernel<true> : amp_reset_kernel<false>;
+    k<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>((uint4*)c->d_counts, counts16, (uint4*)c->tab.heads, heads16, c->tab.slots, c->tab.entries,
+                                                        c->tab.cursor, c->d_err, c->d_reset_done, (uint4*)c->d_rev, (uint4*)c->d_qsum, counts16,
+                                                        c->d_ins_rev, c->d_ins_qsum, c->d_ins_head);
     CK(cudaGetLastError());
     return AMP_OK;
 }
@@ -681,6 +751,7 @@ int amp_process_device(amp_ctx* c, const amp_batch* b, int64_t sum_cigar_ops, in
     if (sample < 0 || sample >= c->cfg.n_samples) return fail(AMP_ERR_ARG, "amp_process_device: sample out of range");
     if ((mode & AMP_MODE_TRIM) && (!o || !has_scheme(c, sample))) return fail(AMP_ERR_ARG, "amp_process_device: trimming needs primer tables and an output block");
     if (!(mode & (AMP_MODE_TRIM | AMP_MODE_PILEUP))) return fail(AMP_ERR_ARG, "amp_process_device: empty mode");
+    if (int rc = check_qstats_mode(c, mode, "amp_process_device")) return rc;
     CK(cudaSetDevice(c->cfg.device));
     c->last_launches = 0;
     cudaStream_t st = (cudaStream_t)stream;
@@ -724,6 +795,7 @@ int amp_process_host(amp_ctx* c, const amp_batch* b, int mode, int sample, const
     if (sample < 0 || sample >= c->cfg.n_samples) return fail(AMP_ERR_ARG, "amp_process_host: sample out of range");
     if ((mode & AMP_MODE_TRIM) && (!o || !has_scheme(c, sample))) return fail(AMP_ERR_ARG, "amp_process_host: trimming needs primer tables and an output block");
     if (!(mode & (AMP_MODE_TRIM | AMP_MODE_PILEUP))) return fail(AMP_ERR_ARG, "amp_process_host: empty mode");
+    if (int rc = check_qstats_mode(c, mode, "amp_process_host")) return rc;
     CK(cudaSetDevice(c->cfg.device));
     c->last_launches = 0;
     const bool trim = mode & AMP_MODE_TRIM, pile = mode & AMP_MODE_PILEUP;
@@ -972,6 +1044,104 @@ int amp_call(amp_ctx* c, const char* ref_seq, const amp_call_params* p, const am
     return AMP_OK;
 }
 
+int amp_qstats_enable(amp_ctx* c) {
+    if (!c) return fail(AMP_ERR_ARG, "amp_qstats_enable: null context");
+    if (c->d_rev) return AMP_OK;
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    const size_t n = (size_t)c->cfg.n_samples * AMP_NCH * c->Lpad;
+    CK(cudaMalloc((void**)&c->d_rev, n * 4)); CK(cudaMalloc((void**)&c->d_qsum, n * 8));
+    CK(cudaMalloc((void**)&c->d_ins_rev, c->nslots * 4)); CK(cudaMalloc((void**)&c->d_ins_qsum, c->nslots * 8));
+    CK(cudaMalloc((void**)&c->d_ins_head, c->nslots));
+    CK(cudaMemset(c->d_rev, 0, n * 4)); CK(cudaMemset(c->d_qsum, 0, n * 8));
+    CK(cudaMemset(c->d_ins_rev, 0, c->nslots * 4)); CK(cudaMemset(c->d_ins_qsum, 0, c->nslots * 8)); CK(cudaMemset(c->d_ins_head, 0, c->nslots));
+    return AMP_OK;
+}
+
+int amp_qstats_host(amp_ctx* c, int sample, int32_t* rev, int64_t* qsum, int32_t* ins_rev, int64_t* ins_qsum, uint8_t* ins_head) {
+    if (!c || sample < 0 || sample >= c->cfg.n_samples) return fail(AMP_ERR_ARG, "amp_qstats_host: bad argument");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, "amp_qstats_host: amp_qstats_enable has not been called");
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    const size_t L = (size_t)c->cfg.ref_len, base = (size_t)sample * AMP_NCH * c->Lpad;
+    if (rev) CK(cudaMemcpy2D(rev, L * 4, c->d_rev + base, (size_t)c->Lpad * 4, L * 4, AMP_NCH, cudaMemcpyDeviceToHost));
+    if (qsum) CK(cudaMemcpy2D(qsum, L * 8, c->d_qsum + base, (size_t)c->Lpad * 8, L * 8, AMP_NCH, cudaMemcpyDeviceToHost));
+    unsigned long long cur[2];
+    CK(cudaMemcpy(cur, c->tab.cursor, 16, cudaMemcpyDeviceToHost));
+    const unsigned long long n = cur[1];
+    if (n == 0 || !(ins_rev || ins_qsum || ins_head)) return AMP_OK;
+    {
+        int rc = dev_grow(&c->d_xbuf, &c->xbuf_bytes, (size_t)n * 13 + 64);
+        if (rc) return rc;
+    }
+    unsigned long long* d_q = (unsigned long long*)c->d_xbuf;
+    int* d_r = (int*)(c->d_xbuf + (size_t)n * 8);
+    unsigned char* d_h = c->d_xbuf + (size_t)n * 12;
+    amp_qstats_gather_kernel<<<(unsigned)std::min<unsigned long long>((n + 255) / 256, 1184), 256>>>(c->tab.entries, n, c->d_ins_rev, c->d_ins_qsum,
+                                                                                                    c->d_ins_head, d_r, d_q, d_h);
+    CK(cudaGetLastError());
+    if (ins_rev) CK(cudaMemcpy(ins_rev, d_r, n * 4, cudaMemcpyDeviceToHost));
+    if (ins_qsum) CK(cudaMemcpy(ins_qsum, d_q, n * 8, cudaMemcpyDeviceToHost));
+    if (ins_head) CK(cudaMemcpy(ins_head, d_h, n, cudaMemcpyDeviceToHost));
+    return AMP_OK;
+}
+
+// device-side iVar calling on the outputs amp_call_device left in the context; asynchronous on `stream`
+int amp_call_ivar_device(amp_ctx* c, const amp_ivar_params* p, void* stream) {
+    if (!c || !p) return fail(AMP_ERR_ARG, "amp_call_ivar_device: null argument");
+    if (!(p->iupac_threshold >= 0.0 && p->iupac_threshold <= 1.0)) return fail(AMP_ERR_ARG, "amp_call_ivar_device: iupac_threshold must be in [0, 1]");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, "amp_call_ivar_device: amp_qstats_enable has not been called");
+    if (!c->d_call) return fail(AMP_ERR_STATE, "amp_call_ivar_device: amp_call / amp_call_device has not been called");
+    CK(cudaSetDevice(c->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t L = (size_t)c->cfg.ref_len, S = (size_t)c->cfg.n_samples, SL = S * L;
+    if (!c->d_ivar) {
+        size_t bytes = 0;
+        auto take = [&](size_t n) { size_t o = bytes; bytes += (n + 255) & ~(size_t)255; return o; };
+        c->o_iu = take(SL); c->o_fmq = take(SL * 6 * 4); c->o_fpv = take(SL * 6 * 8); c->o_imq = take(c->nslots * 4); c->o_ipv = take(c->nslots * 8);
+        CK(cudaMalloc((void**)&c->d_ivar, bytes + 256));
+    }
+    unsigned char* blk = c->d_call;
+    unsigned char* out = c->d_ivar;
+    amp::IvarParams P{};
+    P.L = (int)L; P.Lpad = c->Lpad; P.n_samples = (int)S; P.counts = c->d_counts; P.qsum = c->d_qsum;
+    P.slots = c->tab.slots; P.slot_entry = c->tab.slot_entry; P.arena = c->tab.arena; P.heads = c->tab.heads; P.ins_qsum = c->d_ins_qsum;
+    P.ref_seq = c->d_ref; P.ref_stride = c->ref_per_sample ? (long long)c->cfg.ref_len : 0;
+    P.depth = (const int*)(blk + c->o_depth); P.top_id = (const int*)(blk + c->o_top); P.top_count = (const int*)(blk + c->o_topc);
+    P.fixed_freq = (const double*)(blk + c->o_ff); P.fixed_rank = (const int*)(blk + c->o_fr);
+    P.ins_freq = (const double*)(blk + c->o_if); P.ins_rank = (const int*)(blk + c->o_ir);
+    P.min_depth = p->min_depth; P.min_freq = p->min_freq; P.iupac_threshold = p->iupac_threshold;
+    P.iupac = out + c->o_iu; P.fixed_mq = (int*)(out + c->o_fmq); P.fixed_pval = (double*)(out + c->o_fpv);
+    P.ins_mq = (int*)(out + c->o_imq); P.ins_pval = (double*)(out + c->o_ipv);
+    amp_ivar_kernel<<<(unsigned)((SL + 255) / 256), 256, 0, st>>>(P);
+    CK(cudaGetLastError());
+    c->last_launches = 1;
+    return AMP_OK;
+}
+
+int amp_call_ivar(amp_ctx* c, const amp_ivar_params* p, uint8_t* iupac, int32_t* fixed_mq, double* fixed_pval, int32_t* ins_mq,
+                  double* ins_pval) {
+    if (!c || !p) return fail(AMP_ERR_ARG, "amp_call_ivar: null argument");
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    cudaStream_t st = c->chunk[0].stream;
+    int rc;
+    if ((rc = amp_call_ivar_device(c, p, st))) return rc;
+    const size_t SL = (size_t)c->cfg.n_samples * c->cfg.ref_len;
+    unsigned long long cur[2];
+    CK(cudaMemcpyAsync(cur, c->tab.cursor, 16, cudaMemcpyDeviceToHost, st));
+    unsigned char* out = c->d_ivar;
+    if (iupac) CK(cudaMemcpyAsync(iupac, out + c->o_iu, SL, cudaMemcpyDeviceToHost, st));
+    if (fixed_mq) CK(cudaMemcpyAsync(fixed_mq, out + c->o_fmq, SL * 6 * 4, cudaMemcpyDeviceToHost, st));
+    if (fixed_pval) CK(cudaMemcpyAsync(fixed_pval, out + c->o_fpv, SL * 6 * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const size_t K = (size_t)cur[1];
+    if (K && ins_mq) CK(cudaMemcpyAsync(ins_mq, out + c->o_imq, K * 4, cudaMemcpyDeviceToHost, st));
+    if (K && ins_pval) CK(cudaMemcpyAsync(ins_pval, out + c->o_ipv, K * 8, cudaMemcpyDeviceToHost, st));
+    if (K) CK(cudaStreamSynchronize(st));
+    return AMP_OK;
+}
+
 // The blocks of a byte stream that is already in device memory (readable up to d_in + n_bytes + 8): deflate + pack kernels, then the
 // BGZF blocks and the EOF block to the host.  Returns the bytes written to out or a negative error code.
 static int64_t deflate_device(amp_ctx* c, const uint8_t* d_in, int64_t n_bytes, const int64_t* bstart, int64_t n_blocks, uint8_t* out, int64_t out_cap,
@@ -1183,6 +1353,7 @@ int amp_nccl_allgather(void* comm, const void* dev_send, void* dev_recv, int64_t
 // one ncclAllReduce(sum, int32) over the whole [n_samples][6][lpad] block, in place, asynchronous on `stream`
 int amp_allreduce_counts(amp_ctx* c, void* comm, void* stream) {
     if (!c || !comm) return fail(AMP_ERR_ARG, "amp_allreduce_counts: null argument");
+    if (c->d_rev) return fail(AMP_ERR_STATE, "amp_allreduce_counts: the strand / quality stats are not exchanged across ranks");
     NCCL_OR_FAIL(a);
     CK(cudaSetDevice(c->cfg.device));
     const size_t n = (size_t)c->cfg.n_samples * AMP_NCH * (size_t)c->Lpad;
@@ -1197,6 +1368,7 @@ int64_t amp_ins_slot_bytes(int64_t cap_entries, int64_t cap_arena_bytes) {
 }
 int amp_ins_pack_device(amp_ctx* c, void* dev_slot, int64_t cap_entries, int64_t cap_arena_bytes, void* stream) {
     if (!c || !dev_slot || cap_entries < 0 || cap_arena_bytes < 0) return fail(AMP_ERR_ARG, "amp_ins_pack_device: bad argument");
+    if (c->d_rev) return fail(AMP_ERR_STATE, "amp_ins_pack_device: the strand / quality stats are not exchanged across ranks");
     CK(cudaSetDevice(c->cfg.device));
     amp_ins_pack_kernel<<<c->sm_count * 2, 512, 0, (cudaStream_t)stream>>>(c->tab, (unsigned long long*)dev_slot, (unsigned long long)cap_entries,
                                                                           (unsigned long long)((cap_arena_bytes + 7) / 8));
@@ -1363,6 +1535,7 @@ int amp_process_decoded(amp_ctx* c, int mode, int sample, const amp_trim_out* ho
     if (sample < 0 || sample >= c->cfg.n_samples) return fail(AMP_ERR_ARG, "amp_process_decoded: sample out of range");
     if ((mode & AMP_MODE_TRIM) && !has_scheme(c, sample)) return fail(AMP_ERR_ARG, "amp_process_decoded: trimming needs primer tables");
     if (!(mode & (AMP_MODE_TRIM | AMP_MODE_PILEUP))) return fail(AMP_ERR_ARG, "amp_process_decoded: empty mode");
+    if (int rc = check_qstats_mode(c, mode, "amp_process_decoded")) return rc;
     CK(cudaSetDevice(c->cfg.device));
     cudaStream_t sc = c->chunk[0].stream;
     const bool trim = mode & AMP_MODE_TRIM;

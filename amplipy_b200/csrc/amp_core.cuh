@@ -31,6 +31,7 @@
 #define AMP_E_CIGAR 8        // query-consuming ops exceed l_seq / unsupported op
 #define AMP_E_TABLE_FULL 16  // insertion hash table full
 #define AMP_E_ARENA_FULL 32  // insertion string arena full
+#define AMP_E_QSTATS_MISS 64 // strand / quality pass: an insertion allele the pileup did not add (amp_ivar.cuh)
 
 #define AMP_NCH 6            // channels A C G T N '-'
 
@@ -848,10 +849,28 @@ AMP_HD unsigned long long mix64(unsigned long long h) {
 // text getter: text(i) -> i-th character of the key; text.word(i, len) -> characters i .. i+3 packed little-endian
 // (i a multiple of 4, zero beyond len).  Keys are hashed, stored and compared a word at a time: insertion alleles that
 // run to the end of the read (exit (B) of the state machine) are hundreds of characters long.
+// The key's hash is built from these three steps (ins_table_add interleaves the middle one with writing a long key's record)
+AMP_HD unsigned long long ins_hash_init(int gpos) { return (0xCBF29CE484222325ULL ^ (unsigned long long)(unsigned int)gpos) * 0x100000001B3ULL; }
+AMP_HD unsigned long long ins_hash_word(unsigned long long h, unsigned int w) { return (h ^ w) * 0x100000001B3ULL; }
+AMP_HD unsigned long long ins_hash_final(unsigned long long h, int len) { return mix64(h ^ ((unsigned long long)len << 32)); }
+// slot key k (tag matched) names the record of exactly this key
+template <class Text>
+AMP_HD bool ins_rec_equal(const InsTable& T, unsigned long long k, int gpos, int len, const Text& text) {
+    fence();
+    const unsigned char* rec = T.arena + (k & 0xFFFFFFFFFFULL) * 8;
+    const unsigned long long hdr = ld_cg64((const unsigned long long*)rec);
+    if ((int)(hdr & 0xFFFFFFFFu) != gpos || (unsigned int)(hdr >> 32) != (unsigned int)len) return false;
+    bool same = true;
+    for (int i = 0; i < len && same; i += 4) {
+        unsigned int w = ld_cg32((const unsigned int*)(rec + 8 + i));
+        if (len - i < 4) w &= (1u << (8 * (len - i))) - 1u;
+        same = w == text.word(i, len);
+    }
+    return same;
+}
 template <class Text>
 AMP_HD_NOINLINE void ins_table_add(const InsTable& T, int gpos, int len, const Text& text, int n) {
-    unsigned long long h = 0xCBF29CE484222325ULL ^ (unsigned long long)(unsigned int)gpos;
-    h *= 0x100000001B3ULL;
+    unsigned long long h = ins_hash_init(gpos);
     long long my_off = -1;
 #ifndef AMP_KEY_SPEC
 #define AMP_KEY_SPEC 32
@@ -868,14 +887,14 @@ AMP_HD_NOINLINE void ins_table_add(const InsTable& T, int gpos, int len, const T
         for (int i = 0; i < len; i += 4) {
             const unsigned int w = text.word(i, len);
             ((unsigned int*)(rec + 8))[i >> 2] = w;
-            h ^= w; h *= 0x100000001B3ULL;
+            h = ins_hash_word(h, w);
         }
         fence();
         my_off = (long long)off;
     } else {
-        for (int i = 0; i < len; i += 4) { h ^= text.word(i, len); h *= 0x100000001B3ULL; }
+        for (int i = 0; i < len; i += 4) h = ins_hash_word(h, text.word(i, len));
     }
-    h = mix64(h ^ ((unsigned long long)len << 32));
+    h = ins_hash_final(h, len);
     const unsigned long long tag = (h >> 40) | 0x800000ULL;            // never zero
     unsigned long long slot = h & T.mask;
     for (unsigned long long probes = 0; probes <= T.mask; ++probes, slot = (slot + 1) & T.mask) {
@@ -903,28 +922,32 @@ AMP_HD_NOINLINE void ins_table_add(const InsTable& T, int gpos, int len, const T
             }
             k = old;
         }
-        if ((k >> 40) == tag) {
-            fence();
-            const unsigned char* rec = T.arena + (k & 0xFFFFFFFFFFULL) * 8;
-            const unsigned long long hdr = ld_cg64((const unsigned long long*)rec);
-            if ((int)(hdr & 0xFFFFFFFFu) == gpos && (unsigned int)(hdr >> 32) == (unsigned int)len) {
-                bool same = true;
-                for (int i = 0; i < len && same; i += 4) {
-                    unsigned int w = ld_cg32((const unsigned int*)(rec + 8 + i));
-                    if (len - i < 4) w &= (1u << (8 * (len - i))) - 1u;
-                    same = w == text.word(i, len);
-                }
-                if (same) { atomic_add(&T.slots[slot].count, n); return; }
-            }
-        }
+        if ((k >> 40) == tag && ins_rec_equal(T, k, gpos, len, text)) { atomic_add(&T.slots[slot].count, n); return; }
     }
     atomic_or(T.err, AMP_E_TABLE_FULL);
+}
+// The slot of an allele that is already in the table, -1 if it is not: the same hash and comparison as ins_table_add, nothing
+// is written.
+template <class Text>
+AMP_HD int ins_table_find(const InsTable& T, int gpos, int len, const Text& text) {
+    unsigned long long h = ins_hash_init(gpos);
+    for (int i = 0; i < len; i += 4) h = ins_hash_word(h, text.word(i, len));
+    h = ins_hash_final(h, len);
+    const unsigned long long tag = (h >> 40) | 0x800000ULL;
+    unsigned long long slot = h & T.mask;
+    for (unsigned long long probes = 0; probes <= T.mask; ++probes, slot = (slot + 1) & T.mask) {
+        const unsigned long long k = ld_cg64(&T.slots[slot].key);
+        if (k == 0) return -1;
+        if ((k >> 40) == tag && ins_rec_equal(T, k, gpos, len, text)) return (int)slot;
+    }
+    return -1;
 }
 
 // ---- pileup plan: walk the (trimmed) CIGAR exactly as update_base_counts walks get_aligned_pairs() ----
 // Sink interface:  match(rpos, q, len)   aligned run (quality filter applied when counting)
 //                  del(rpos, len)        D / N run -> '-' channel, unconditional (714-715)
-//                  ins(pos, s_begin, s_len)   insertion allele = query_seq[s_begin : s_begin + s_len]
+//                  ins(pos, s_begin, s_len, q0)   insertion allele = query_seq[s_begin : s_begin + s_len]; q0 = the first
+//                                        inserted base that passed the gates 718 / 722 (s_begin == q0: the key of 735-736)
 // Returns AMP_E_* bits (0 = ok).
 template <class Sink>
 AMP_HD int plan_read(const uint32_t* c, int nc, int pos, int l_seq, const uint8_t* qual, int minq, int L, Sink& sink) {
@@ -940,7 +963,7 @@ AMP_HD int plan_read(const uint32_t* c, int nc, int pos, int l_seq, const uint8_
     // key slice [q0-1 : end) with python's negative-index wrap for q0 == 0
 #define AMP_KEY(end_, at_) do { int b_ = q0 - 1; if (b_ < 0) { b_ += l_seq; if (b_ < 0) b_ = 0; } \
         int e_ = (end_) < l_seq ? (end_) : l_seq; int n_ = e_ - b_; if (n_ < 0) n_ = 0; \
-        int p_ = (at_) - 1; if (p_ < 0) p_ = 0; if (p_ >= L) return AMP_E_COORD; sink.ins(p_, b_, n_); q0 = -1; } while (0)
+        int p_ = (at_) - 1; if (p_ < 0) p_ = 0; if (p_ >= L) return AMP_E_COORD; sink.ins(p_, b_, n_, q0); q0 = -1; } while (0)
     for (int k = 0; k < nc; ++k) {
         const uint32_t op = c_op(c[k]); const int n = c_len(c[k]);
         if (op == OP_H || n == 0) continue;
@@ -948,7 +971,7 @@ AMP_HD int plan_read(const uint32_t* c, int nc, int pos, int l_seq, const uint8_
             if (r + n > L) return AMP_E_COORD;
             if (q + n > l_seq) return AMP_E_CIGAR;
             if (q0 >= 0) {                                    // exit (A)/(A'): next pair is a match
-                if (r == 0) { int e_ = q + 1 < l_seq ? q + 1 : l_seq; sink.ins(0, q0, e_ - q0); q0 = -1; }   // 735-736
+                if (r == 0) { int e_ = q + 1 < l_seq ? q + 1 : l_seq; sink.ins(0, q0, e_ - q0, q0); q0 = -1; }   // 735-736
                 else AMP_KEY(q, r);
             }
             sink.match(r, q, n);

@@ -197,7 +197,7 @@ struct TileSink {
             return w;
         }
     };
-    AMP_HD void ins(int pos, int b, int n) {
+    AMP_HD void ins(int pos, int b, int n, int /*q0*/ = 0) {
         if (n == 1) {   // one-character key == that base's own dict entry (AmpliPy.py:745-746)
             int ch = nib_channel(nib_at(seq_read, (uint32_t)b));
             if (ch >= 0) { atomic_add(&P->counts[(size_t)ch * P->Lpad + pos], 1); return; }
@@ -258,7 +258,7 @@ struct DirectSink {
         }
     }
     AMP_HD void del(int rpos, int n) { for (int j = 0; j < n; ++j) count_add(*P, sm.cnt, wbase, 5, rpos + j); }   // 714-715
-    AMP_HD void ins(int pos, int b, int n) {
+    AMP_HD void ins(int pos, int b, int n, int /*q0*/ = 0) {
         if (n == 1) {
             int ch = nib_channel(nib_at(seq_read, (uint32_t)b));
             if (ch >= 0) { atomic_add(&P->counts[(size_t)ch * P->Lpad + pos], 1); return; }
@@ -292,7 +292,7 @@ struct RecordSink {
         if (nrun < AMP_REC_RUNS && n < 32768) { rp[nrun] = rpos; ql[nrun] = 0x8000u | (uint32_t)n; ++nrun; steps += n; }
         else d.del(rpos, n);
     }
-    AMP_HD void ins(int pos, int b, int n) {
+    AMP_HD void ins(int pos, int b, int n, int /*q0*/ = 0) {
         if (nins < AMP_REC_INS && b < 65536 && n < 65536) { ip[nins] = pos; ib[nins] = ((uint32_t)b << 16) | (uint32_t)n; ++nins; }
         else d.ins(pos, b, n);
     }

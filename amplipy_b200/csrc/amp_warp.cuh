@@ -468,7 +468,7 @@ struct WarpSink7 {
     }
     AMP_HD void match(int rpos, int q, int n) { push(rpos, n, q); }
     AMP_HD void del(int rpos, int n) { push(rpos, (int)(0x80000000u | (unsigned)n), 0); }
-    AMP_WD void ins(int pos, int b, int n) { ins_defer(*P, wm.ctrl, so0, pos, b, n); }
+    AMP_WD void ins(int pos, int b, int n, int /*q0*/) { ins_defer(*P, wm.ctrl, so0, pos, b, n); }
 };
 
 // one base outside the tile (or of an unstaged run): straight to the global matrix.  row = BAM nibble, or AMP7_DEL_CODE

@@ -18,18 +18,20 @@ import numpy as np
 
 from .batch import ReadBatch
 from .calling import CallResult, Insertions
+from .ivar import IvarResult, QStats
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AMP_LIB_OVERRIDE") or os.path.join(_HERE, "csrc", "libamplipy_b200.so")   # override: tuning experiments only
 
-MODE_TRIM, MODE_PILEUP = 1, 2
+MODE_TRIM, MODE_PILEUP, MODE_QSTATS = 1, 2, 4
 F_TRIM_START, F_TRIM_END, F_TRIM_QUAL, F_KEEP, F_SKIPPED, F_ERROR = 1, 2, 4, 8, 16, 32
 DEVERR_NAMES = {1: "read outside the reference (IndexError in AmpliPy.py:450-451)",
                 2: "aligned base not in ACGTN (KeyError in AmpliPy.py:753)",
                 4: "insertion runs to the end of the alignment (IndexError in AmpliPy.py:734)",
                 8: "CIGAR consumes more query than l_seq / unsupported op",
                 16: "insertion hash table full (raise ins_slots)",
-                32: "insertion string arena full (raise ins_arena_bytes)"}
+                32: "insertion string arena full (raise ins_arena_bytes)",
+                64: "strand / quality pass met an insertion allele the pileup did not add"}
 
 EXPORTED_SYMBOLS = [
     "amp_last_error", "amp_abi_version", "amp_create", "amp_destroy", "amp_reset", "amp_error_flags", "amp_lpad",
@@ -39,7 +41,8 @@ EXPORTED_SYMBOLS = [
     "amp_nccl_unique_id", "amp_nccl_comm_init", "amp_nccl_comm_destroy", "amp_nccl_allgather", "amp_allreduce_counts",
     "amp_ins_slot_bytes", "amp_ins_pack_device", "amp_ins_merge_packed", "amp_reserve", "amp_counts_copy_device",
     "amp_bam_decode_host", "amp_process_decoded", "amp_decoded_copy_host", "amp_counts_upload", "amp_bgzf_deflate_host", "amp_decoded_write_bam",
-    "amp_set_scheme", "amp_get_scheme", "amp_set_sample_reference"]
+    "amp_set_scheme", "amp_get_scheme", "amp_set_sample_reference", "amp_qstats_enable", "amp_qstats_host", "amp_call_ivar",
+    "amp_call_ivar_device"]
 
 
 class AmpConfig(ctypes.Structure):
@@ -74,6 +77,10 @@ class AmpBatchOut(ctypes.Structure):
 class AmpCallParams(ctypes.Structure):
     _fields_ = [("min_depth_consensus", ctypes.c_int32), ("min_freq_consensus", ctypes.c_double),
                 ("min_depth_variants", ctypes.c_int32), ("min_freq_variants", ctypes.c_double)]
+
+
+class AmpIvarParams(ctypes.Structure):
+    _fields_ = [("min_depth", ctypes.c_int32), ("min_freq", ctypes.c_double), ("iupac_threshold", ctypes.c_double)]
 
 
 class AmpCallOut(ctypes.Structure):
@@ -253,9 +260,10 @@ class Engine:
         return (np.zeros(n, np.int32), np.zeros(n, np.uint16), np.zeros(n, np.uint8),
                 np.zeros(int(batch.cig_off[-1]) + 3 * n, np.uint32))
 
-    def process(self, batch, trim=True, pileup=True, sample=0, out=None, first=0, n=None):
-        """H2D + fused kernel + D2H through amp_process_host.  Returns TrimResult when trim=True."""
-        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0)
+    def process(self, batch, trim=True, pileup=True, sample=0, out=None, first=0, n=None, qstats=False):
+        """H2D + fused kernel + D2H through amp_process_host.  Returns TrimResult when trim=True.  ``qstats=True``: the
+        strand / quality pass runs on the same reads (enable_qstats first)."""
+        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0) | (MODE_QSTATS if qstats else 0)
         n = batch.n - first if n is None else n
         hb = AmpBatch(first, n, _ptr(batch.pos), _ptr(batch.flag), _ptr(batch.tlen), _ptr(batch.cig_off),
                       _ptr(batch.cigar), _ptr(batch.seq_off), _ptr(batch.seq), _ptr(batch.qual_off), _ptr(batch.qual))
@@ -312,9 +320,10 @@ class Engine:
         return d
 
     def process_device(self, d, trim=True, pileup=True, sample=0, stream=None, first=0, n=None, sum_cig=None,
-                       sum_qual=None):
-        """Launch the fused kernel on a batch already resident in HBM (asynchronous on ``stream``)."""
-        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0)
+                       sum_qual=None, qstats=False):
+        """Launch the fused kernel on a batch already resident in HBM (asynchronous on ``stream``); ``qstats=True``: and the
+        strand / quality pass after it."""
+        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0) | (MODE_QSTATS if qstats else 0)
         n = d["n"] - first if n is None else n
         p = lambda t: ctypes.c_void_p(t.data_ptr())
         db = AmpBatch(first, n, p(d["pos"]), p(d["flag"]), p(d["tlen"]), p(d["cig_off"]), p(d["cigar"]),
@@ -416,10 +425,10 @@ class Engine:
         n, sc = self._decoded["n"], self._decoded["sum_cig"]
         return (np.zeros(n, np.int32), np.zeros(n, np.uint16), np.zeros(n, np.uint8), np.zeros(sc + 3 * n, np.uint32))
 
-    def process_decoded(self, trim=True, pileup=True, sample=0, out=None, download=True):
+    def process_decoded(self, trim=True, pileup=True, sample=0, out=None, download=True, qstats=False):
         """Fused kernel on the batch decode_bam left in HBM; trim outputs copied to ``out`` (alloc_decoded_trim_out), or left on the
-        device only (``download=False``: decoded_write_bam is their consumer)."""
-        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0)
+        device only (``download=False``: decoded_write_bam is their consumer).  ``qstats=True``: the strand / quality pass too."""
+        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0) | (MODE_QSTATS if qstats else 0)
         to = None
         if trim and download:
             if out is None:
@@ -496,6 +505,46 @@ class Engine:
                                              ctypes.c_int64(cap_entries), ctypes.c_int64(cap_arena_bytes),
                                              ctypes.c_void_p(stream) if stream else None), "amp_ins_merge_packed")
         self.launches += 1
+
+    # ---------------------------------------------------------------- iVar-format outputs (DESIGN.md 3.7)
+    def enable_qstats(self):
+        """Allocate the strand / quality sums (amp_qstats_enable); process(..., qstats=True) fills them."""
+        _check(self.lib.amp_qstats_enable(self._ctx), "amp_qstats_enable")
+
+    def qstats(self, sample=0):
+        """The strand / quality sums of one sample: rev / qsum [6, L] and, in insertions() order (all samples), ins_rev /
+        ins_qsum / ins_head."""
+        n = ctypes.c_int64(0)
+        nch = ctypes.c_int64(0)
+        _check(self.lib.amp_ins_count(self._ctx, ctypes.byref(n), ctypes.byref(nch)), "amp_ins_count")
+        k = int(n.value)
+        q = QStats(np.empty((6, self.L), np.int32), np.empty((6, self.L), np.int64), np.zeros(max(k, 1), np.int32),
+                   np.zeros(max(k, 1), np.int64), np.zeros(max(k, 1), np.uint8))
+        _check(self.lib.amp_qstats_host(self._ctx, int(sample), _ptr(q.rev), _ptr(q.qsum), _ptr(q.ins_rev), _ptr(q.ins_qsum),
+                                        _ptr(q.ins_head)), "amp_qstats_host")
+        q.ins_rev, q.ins_qsum, q.ins_head = q.ins_rev[:k], q.ins_qsum[:k], q.ins_head[:k]
+        return q
+
+    def call_ivar(self, min_depth=1, min_freq=0.03, iupac_threshold=0.0):
+        """Mean qualities, Fisher p-values and IUPAC codes (amp_call_ivar) on the outputs of the last ``call``."""
+        n = ctypes.c_int64(0)
+        nch = ctypes.c_int64(0)
+        _check(self.lib.amp_ins_count(self._ctx, ctypes.byref(n), ctypes.byref(nch)), "amp_ins_count")
+        k = max(int(n.value), 1)
+        SL = self.n_samples * self.L
+        r = IvarResult(np.empty(SL, np.uint8), np.empty((SL, 6), np.int32), np.empty((SL, 6), np.float64), np.zeros(k, np.int32),
+                       np.full(k, np.nan))
+        p = AmpIvarParams(int(min_depth), float(min_freq), float(iupac_threshold))
+        _check(self.lib.amp_call_ivar(self._ctx, ctypes.byref(p), _ptr(r.iupac), _ptr(r.fixed_mq), _ptr(r.fixed_pval),
+                                      _ptr(r.ins_mq), _ptr(r.ins_pval)), "amp_call_ivar")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        return r
+
+    def call_ivar_device(self, min_depth=1, min_freq=0.03, iupac_threshold=0.0, stream=None):
+        p = AmpIvarParams(int(min_depth), float(min_freq), float(iupac_threshold))
+        _check(self.lib.amp_call_ivar_device(self._ctx, ctypes.byref(p), ctypes.c_void_p(stream) if stream else None),
+               "amp_call_ivar_device")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
 
     def _call_buffers(self, n_ins, pinned):
         """Result arrays of ``call``: fresh numpy arrays, or (``pinned``) page-locked arrays owned by the engine and reused."""

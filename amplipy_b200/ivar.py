@@ -1,0 +1,115 @@
+"""iVar-format outputs (DESIGN.md 3.7): the variants TSV and the IUPAC-ambiguity consensus.  AmpliPy itself has neither.
+
+The per-allele numbers (strand and quality sums, mean qualities, Fisher p-values, IUPAC codes) are computed on the device
+(``Engine.enable_qstats`` / ``process(..., qstats=True)`` / ``Engine.call_ivar``); this module only selects rows and formats.
+"""
+import gzip
+import math
+import os
+from dataclasses import dataclass
+
+import numpy as np
+
+from .calling import FIXED_SYMS
+from .primers import InputError
+
+ERROR_TEXT_FILE_EXISTS = "File already exists"
+ERROR_TEXT_INVALID_IUPAC_THRESHOLD = "IUPAC threshold must be between 0 and 1"
+TSV_HEADER = ("REGION", "POS", "REF", "ALT", "REF_DP", "REF_RV", "REF_QUAL", "ALT_DP", "ALT_RV", "ALT_QUAL", "ALT_FREQ", "TOTAL_DP",
+              "PVAL", "PASS", "GFF_FEATURE", "REF_CODON", "REF_AA", "ALT_CODON", "ALT_AA", "POS_AA")
+PASS_PVAL = 0.05
+
+
+@dataclass
+class QStats:
+    """Strand / quality sums of one sample (``amp_qstats_host``); the insertion arrays are in ``insertions()`` order."""
+    rev: np.ndarray         # i32[6, L] increments of the count matrix from reverse-strand reads
+    qsum: np.ndarray        # i64[6, L] phred qualities of the counted bases ('-' row: 0)
+    ins_rev: np.ndarray     # i32[K]
+    ins_qsum: np.ndarray    # i64[K] quality of each event's first inserted base
+    ins_head: np.ndarray    # u8[K] 1: the allele's key is the one AmpliPy.py:735-736 builds at position 0
+
+
+@dataclass
+class IvarResult:
+    """``amp_call_ivar`` outputs for all samples."""
+    iupac: np.ndarray       # u8[S*L] IUPAC code, 0 = the reference's own consensus symbol
+    fixed_mq: np.ndarray    # i32[S*L, 6] mean quality of A C G T N '-'
+    fixed_pval: np.ndarray  # f64[S*L, 6] NaN = no TSV row
+    ins_mq: np.ndarray      # i32[K]
+    ins_pval: np.ndarray    # f64[K]
+
+
+def check_output_path(path):
+    """The TSV refuses to overwrite, like the other outputs."""
+    if path.lower() != "stdout" and os.path.isfile(path):
+        raise InputError("%s: %s" % (ERROR_TEXT_FILE_EXISTS, path))
+
+
+def check_iupac_threshold(t):
+    if t is not None and not (0 <= t <= 1):
+        raise InputError("%s: %s" % (ERROR_TEXT_INVALID_IUPAC_THRESHOLD, t))
+
+
+def alt_text(sym, ref_char, head=False):
+    """iVar's ALT column: a base as is, '-' as '-' + REF (a 1-bp deletion at the deleted base itself), an insertion key s as
+    '+' + s[1:] (its first character is the anchor base), the key of AmpliPy.py:735-736 (``head``) as '+' + s[:-1]."""
+    if sym == "-":
+        return "-" + ref_char
+    if len(sym) == 1 and sym in FIXED_SYMS:
+        return sym
+    return "+" + (sym[:-1] if head else sym[1:])
+
+
+def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0):
+    """The TSV rows of one sample: every allele with a p-value (count > 0, symbol != the FASTA character, freq >= min_freq, depth
+    >= min_depth), in position order, then in the reference's allele order (AmpliPy.py:771)."""
+    L = res.L
+    base = sample * L
+    fpv = iv.fixed_pval[base:base + L]
+    ins_rows = {}
+    if ins.k:
+        sel = np.flatnonzero((ins.sample == sample) & ~np.isnan(iv.ins_pval[:ins.k]))
+        for k in sel.tolist():
+            ins_rows.setdefault(int(ins.pos[k]), []).append(k)
+    pos = sorted(set(np.flatnonzero(~np.isnan(fpv).all(axis=1)).tolist()) | set(ins_rows))
+    out = []
+    for p in pos:
+        gp = base + p
+        D = int(res.depth[gp])
+        ref_char = ref_seq[p]
+        rch = "ACGTN".find(ref_char) if ref_char else -1
+        ref_dp = int(counts[rch, p]) if rch >= 0 else 0
+        ref_rv = int(qs.rev[rch, p]) if rch >= 0 else 0
+        ref_q = int(iv.fixed_mq[gp, rch]) if rch >= 0 else 0
+        alts = []   # (rank, ALT, count, rev, mq, pval)
+        for ch in range(6):
+            if not math.isnan(fpv[p, ch]):
+                alts.append((int(res.fixed_rank[gp, ch]), alt_text(FIXED_SYMS[ch], ref_char), int(counts[ch, p]), int(qs.rev[ch, p]),
+                             int(iv.fixed_mq[gp, ch]), float(fpv[p, ch])))
+        for k in ins_rows.get(p, ()):
+            alts.append((int(res.ins_rank[k]), alt_text(ins.strs[k], ref_char, bool(qs.ins_head[k])), int(ins.count[k]),
+                         int(qs.ins_rev[k]), int(iv.ins_mq[k]), float(iv.ins_pval[k])))
+        alts.sort(key=lambda a: a[0])
+        for _, alt, c, rv, mq, pv in alts:
+            out.append((ref_id, p + 1, ref_char, alt, ref_dp, ref_rv, ref_q, c, rv, mq, c / D, D, pv, pv <= PASS_PVAL))
+    return out
+
+
+def format_row(r):
+    ref_id, pos, ref, alt, ref_dp, ref_rv, ref_q, c, rv, mq, freq, D, pv, ok = r
+    return "\t".join([ref_id, str(pos), ref, alt, str(ref_dp), str(ref_rv), str(ref_q), str(c), str(rv), str(mq), repr(freq), str(D),
+                      repr(pv), "TRUE" if ok else "FALSE"] + ["NA"] * 6)
+
+
+def write_tsv(path, rows):
+    text = "\t".join(TSV_HEADER) + "\n" + "".join(format_row(r) + "\n" for r in rows)
+    if path.lower() == "stdout":
+        import sys
+        sys.stdout.write(text)
+    elif path.lower().endswith(".gz"):
+        with gzip.open(path, "wt") as f:
+            f.write(text)
+    else:
+        with open(path, "w") as f:
+            f.write(text)

@@ -51,10 +51,12 @@ extern "C" {
 #define AMP_DEVERR_CIGAR 8
 #define AMP_DEVERR_TABLE_FULL 16
 #define AMP_DEVERR_ARENA_FULL 32
+#define AMP_DEVERR_QSTATS_MISS 64   /* strand / quality pass: an insertion allele the pileup did not add (never expected) */
 
 /* mode bits for amp_process_* */
 #define AMP_MODE_TRIM 1      /* trim_read, AmpliPy.py:426-687 (+ gate 902/910) */
 #define AMP_MODE_PILEUP 2    /* update_base_counts, AmpliPy.py:690-753 */
+#define AMP_MODE_QSTATS 4    /* with AMP_MODE_PILEUP, after amp_qstats_enable: strand / quality sums of the same events */
 
 typedef struct amp_ctx amp_ctx;
 
@@ -153,6 +155,30 @@ int amp_call(amp_ctx* ctx, const char* ref_seq, const amp_call_params* p, const 
  * in context-owned HBM buffers; asynchronous on `stream` */
 int amp_set_reference(amp_ctx* ctx, const char* ref_seq);
 int amp_call_device(amp_ctx* ctx, const amp_call_params* p, void* stream);
+
+/* ---- iVar-format outputs (the reference has none; DESIGN.md 3.7).  amp_qstats_enable allocates and zeroes, per (sample, channel,
+ * position), rev = the count matrix's increments from reverse-strand reads (flag & 0x10) and qsum = the phred qualities of the
+ * counted A C G T N bases ('-' carries none), plus the same two sums per insertion allele (an event's quality = that of the first
+ * inserted base past the gates 718 / 722).  amp_process_* with AMP_MODE_PILEUP | AMP_MODE_QSTATS then runs a second pass over the
+ * same reads after the fused kernel; amp_reset / amp_reset_async zero the sums.  The sums are not exchanged across ranks:
+ * amp_allreduce_counts and amp_ins_pack_device return AMP_ERR_STATE on a context with them enabled.
+ * amp_qstats_host: host arrays rev [6][L], qsum [6][L] of one sample, and ins_rev / ins_qsum / ins_head [n_alleles] in
+ * amp_ins_export order (ins_head[k] = 1: an event of allele k is the key of AmpliPy.py:735-736); any pointer may be NULL.
+ * amp_call_ivar (after amp_call): per allele mean quality mq = floor(qsum / count) ('-': the position's mean base quality) and,
+ * for the alleles that get a TSV row (count > 0, symbol != the FASTA character, freq >= min_freq, depth >= min_depth; NaN
+ * otherwise), PVAL = the left tail of Fisher's exact test on [[e, D - e], [a, D - a]], e = floor(D * 10^(-mq/10)); and per
+ * (sample, position) an IUPAC code (0 = the reference's own consensus symbol) from the shortest prefix of the sorted allele
+ * list whose frequencies reach iupac_threshold.  Per-allele outputs are indexed like amp_ins_export. */
+typedef struct {
+    int32_t min_depth; double min_freq;   /* TSV rows, and the consensus gate of AmpliPy.py:928 for the IUPAC code */
+    double iupac_threshold;               /* [0, 1]; 0 = the reference's consensus */
+} amp_ivar_params;
+int amp_qstats_enable(amp_ctx* ctx);
+int amp_qstats_host(amp_ctx* ctx, int sample, int32_t* rev, int64_t* qsum, int32_t* ins_rev, int64_t* ins_qsum, uint8_t* ins_head);
+int amp_call_ivar(amp_ctx* ctx, const amp_ivar_params* p, uint8_t* iupac /* [S*L] */, int32_t* fixed_mq /* [S*L*6] */,
+                  double* fixed_pval /* [S*L*6] */, int32_t* ins_mq, double* ins_pval);
+/* the same kernel on the outputs amp_call_device left in HBM; results stay in context-owned buffers; asynchronous on `stream` */
+int amp_call_ivar_device(amp_ctx* ctx, const amp_ivar_params* p, void* stream);
 
 /* ---- deep-sample mode: one sample's reads sharded over ranks (SURVEY.md 8e; the reference has no counterpart, its loop
  * AmpliPy.py:896-915 is sequential).  After every rank has processed its read range:
