@@ -496,8 +496,9 @@ def _bam_tags_to_sam(b):
     return out
 
 
-def write_bam(path, header_text, refs, batch, names=None, mapq=60, threads=0, level=1):
-    """Serialise a ReadBatch as a BAM file (synthetic inputs for tests / benchmarks; read names r<i>)."""
+def write_bam(path, header_text, refs, batch, names=None, mapq=60, threads=0, level=1, refid=None):
+    """Serialise a ReadBatch as a BAM file (synthetic inputs for tests / benchmarks; read names r<i>).  ``refid``: the refID of
+    every read (also its mate's, for paired reads); default 0, and -1 for unmapped reads."""
     lib = hostio()
     b = batch
     nblob = noff = None
@@ -511,6 +512,14 @@ def write_bam(path, header_text, refs, batch, names=None, mapq=60, threads=0, le
             _p(b.qual), int(mapq), _p(nblob), _p(noff))
     size = int(lib.amp_bam_serialize(*args, None, None))
     body = np.empty(size + 8, np.uint8)
-    lib.amp_bam_serialize(*args, _p(body), None)
+    rec_off = np.empty(b.n + 1, np.int64)
+    lib.amp_bam_serialize(*args, _p(body), _p(rec_off))
+    if refid is not None:
+        rid = np.ascontiguousarray(refid, np.int32)
+        assert rid.shape == (b.n,)
+        at = rec_off[:-1, None] + np.arange(4)
+        body[at + 4] = rid.view(np.uint8).reshape(-1, 4)
+        paired = np.flatnonzero(b.flag & 1)
+        body[at[paired] + 24] = rid[paired].view(np.uint8).reshape(-1, 4)
     with open(path, "wb") as f:
         f.write(_bam_file_bytes(_bam_header_bytes(header_text, refs), body[:size], level, threads))

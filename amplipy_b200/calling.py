@@ -46,11 +46,12 @@ class CallResult:
     ins_alt: np.ndarray
 
 
-def consensus_string(res: CallResult, ins: Insertions, sample=0, unknown_symbol="N", iupac=None) -> str:
+def consensus_string(res: CallResult, ins: Insertions, sample=0, unknown_symbol="N", iupac=None, L=None) -> str:
     """''.join(consensus_symbols) of AmpliPy.py:920-929, 960.  ``iupac``: the IUPAC codes of Engine.call_ivar ([S*L], 0 = keep
-    the reference's symbol) replace the symbols of the positions that pass the consensus gate."""
-    L = res.L
-    sl = slice(sample * L, (sample + 1) * L)
+    the reference's symbol) replace the symbols of the positions that pass the consensus gate.  ``L``: the sample's own reference
+    length when it is shorter than the context's (a contig of a multi-record FASTA)."""
+    L = res.L if L is None else L
+    sl = slice(sample * res.L, sample * res.L + L)
     top = res.top_id[sl]
     ok = (res.pos_flags[sl] & 1) != 0
     table = np.frombuffer((FIXED_SYMS + unknown_symbol).encode(), np.uint8)
@@ -74,12 +75,12 @@ def consensus_string(res: CallResult, ins: Insertions, sample=0, unknown_symbol=
     return "".join(out)
 
 
-def variant_records(res: CallResult, ins: Insertions, ref_seq: str, counts: np.ndarray, sample=0):
+def variant_records(res: CallResult, ins: Insertions, ref_seq: str, counts: np.ndarray, sample=0, L=None):
     """[(pos0, ref, [alts], DP, REF_DP, [ALT_DP], REF_FREQ, [ALT_FREQ], GT tuple)] in reference order
     (AmpliPy.py:932-951): ALT alleles follow the reference's sort (count, freq, symbol descending).
-    ``counts`` = this sample's int32[6, L] count matrix (ALT_DP of the fixed symbols)."""
-    L = res.L
-    base = sample * L
+    ``counts`` = this sample's int32[6, L] count matrix (ALT_DP of the fixed symbols); ``L`` as in consensus_string."""
+    L = res.L if L is None else L
+    base = sample * res.L
     flags = res.pos_flags[base:base + L]
     emit = np.flatnonzero(flags & 2)
     by_pos = {}

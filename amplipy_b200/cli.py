@@ -9,7 +9,7 @@ import sys
 from datetime import datetime
 
 from . import alnio, calling, ivar, vcf
-from .primers import InputError, find_overlapping_primers, load_primers, max_primer_len
+from .primers import InputError, find_overlapping_primers, load_primers, load_primers_by_contig, max_primer_len
 
 VERSION = "0.0.2"
 DESCRIPTION = "\nAmpliPy: Python toolkit for viral amplicon sequencing\n"
@@ -55,6 +55,14 @@ HELP_TEXT_TRIM_SLIDING_WINDOW_WIDTH = "Width of sliding window (average quality 
 HELP_TEXT_UNKNOWN_SYMBOL = "Character to print in regions with less than minimum coverage"
 HELP_TEXT_VARIANTS = "Variant Calls (VCF)"
 HELP_TEXT_TSV = "Variant Calls in iVar's TSV format, with strand counts, mean qualities and Fisher p-values (optional)"
+HELP_TEXT_MULTI_CONTIG = ("Every record of the reference FASTA is a contig (e.g. the segments of a segmented virus): reads, primers "
+                          "and outputs are taken per contig by name")
+ERROR_TEXT_EMPTY_FASTA_RECORD = "Empty sequence in FASTA file"
+ERROR_TEXT_DUPLICATE_FASTA_ID = "Duplicate sequence ID in FASTA file"
+ERROR_TEXT_LENGTH_MISMATCH = "Sequence length in the alignment header differs from the reference FASTA"
+ERROR_TEXT_UNKNOWN_CONTIG = "Reads on a sequence that is not in the reference FASTA"
+ERROR_TEXT_UNMAPPED_NO_FLAG = "Read without a reference sequence is not flagged unmapped (flag 4)"
+ERROR_TEXT_BAD_REFID = "Read reference ID outside the alignment header"
 HELP_TEXT_IUPAC_THRESHOLD = ("Write IUPAC ambiguity codes: the shortest prefix of the sorted alleles whose frequencies reach this "
                              "threshold (0-1) is coded (optional; 0 = the plain consensus)")
 
@@ -81,6 +89,7 @@ def parse_args(argv=None):
     t.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_UNTRIMMED)
     t.add_argument('-p', '--primer', required=True, type=str, help=HELP_TEXT_PRIMER)
     t.add_argument('-r', '--reference', required=True, type=str, help=HELP_TEXT_REFERENCE)
+    t.add_argument('--multi_contig', action='store_true', help=HELP_TEXT_MULTI_CONTIG)
     t.add_argument('-o', '--output', required=False, type=str, default='stdout', help=HELP_TEXT_READS_TRIMMED)
     t.add_argument('-x', '--primer_pos_offset', required=False, type=int, default=DEFAULT_PRIMER_POS_OFFSET, help=HELP_TEXT_TRIM_PRIMER_POS_OFFSET)
     t.add_argument('-ml', '--min_length', required=False, type=int, default=DEFAULT_MIN_LENGTH, help=HELP_TEXT_TRIM_MIN_LENGTH)
@@ -91,6 +100,7 @@ def parse_args(argv=None):
     v = sub.add_parser("variants", description=DESCRIPTION, formatter_class=F)
     v.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_TRIMMED)
     v.add_argument('-r', '--reference', required=True, type=str, help=HELP_TEXT_REFERENCE)
+    v.add_argument('--multi_contig', action='store_true', help=HELP_TEXT_MULTI_CONTIG)
     v.add_argument('-o', '--output', required=False, type=str, default='stdout', help=HELP_TEXT_VARIANTS)
     v.add_argument('-mq', '--min_quality', required=False, type=int, default=DEFAULT_MIN_QUALITY, help=HELP_TEXT_MIN_QUAL)
     v.add_argument('-mf', '--min_freq', required=False, type=float, default=DEFAULT_MIN_FREQ_VARIANTS, help=HELP_TEXT_MIN_FREQ_VARIANTS)
@@ -100,6 +110,7 @@ def parse_args(argv=None):
     c = sub.add_parser("consensus", description=DESCRIPTION, formatter_class=F)
     c.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_TRIMMED)
     c.add_argument('-r', '--reference', required=True, type=str, help=HELP_TEXT_REFERENCE)
+    c.add_argument('--multi_contig', action='store_true', help=HELP_TEXT_MULTI_CONTIG)
     c.add_argument('-o', '--output', required=False, type=str, default='stdout', help=HELP_TEXT_CONSENSUS)
     c.add_argument('-mq', '--min_quality', required=False, type=int, default=DEFAULT_MIN_QUALITY, help=HELP_TEXT_MIN_QUAL)
     c.add_argument('-mf', '--min_freq', required=False, type=float, default=DEFAULT_MIN_FREQ_CONSENSUS, help=HELP_TEXT_MIN_FREQ_CONSENSUS)
@@ -111,6 +122,7 @@ def parse_args(argv=None):
     a.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_UNTRIMMED)
     a.add_argument('-p', '--primer', required=True, type=str, help=HELP_TEXT_PRIMER)
     a.add_argument('-r', '--reference', required=True, type=str, help=HELP_TEXT_REFERENCE)
+    a.add_argument('--multi_contig', action='store_true', help=HELP_TEXT_MULTI_CONTIG)
     a.add_argument('-ot', '--output_trimmed_reads', required=True, type=str, help=HELP_TEXT_READS_TRIMMED)
     a.add_argument('-ov', '--output_variants', required=True, type=str, help=HELP_TEXT_VARIANTS)
     a.add_argument('-oc', '--output_consensus', required=True, type=str, help=HELP_TEXT_CONSENSUS)
@@ -144,27 +156,118 @@ def load_ref_genome(reference_fn):
     return ref_id, seq
 
 
+def load_ref_genomes(reference_fn):
+    """Every record of a FASTA -> [(ID, sequence)] in file order; the ID is the first whitespace token of the header, as in
+    load_ref_genome.  An empty record or a repeated ID is an InputError."""
+    if not os.path.isfile(reference_fn):
+        raise InputError("%s: %s" % (ERROR_TEXT_FILE_NOT_FOUND, reference_fn))
+    with open(reference_fn, 'r') as f:
+        lines = f.read().strip().splitlines()
+    if len(lines) < 2 or not lines[0].startswith('>'):
+        raise InputError("%s: %s" % (ERROR_TEXT_INVALID_FASTA, reference_fn))
+    recs = []
+    for l in lines:
+        if l.startswith('>'):
+            head = l[1:].split()
+            if not head:
+                raise InputError("%s: %s" % (ERROR_TEXT_INVALID_FASTA, reference_fn))
+            recs.append((head[0], []))
+        else:
+            recs[-1][1].append(l)
+    out, seen = [], set()
+    for rid, parts in recs:
+        if rid in seen:
+            raise InputError("%s: %s" % (ERROR_TEXT_DUPLICATE_FASTA_ID, rid))
+        seen.add(rid)
+        seq = ''.join(parts)
+        if not seq:
+            raise InputError("%s: %s" % (ERROR_TEXT_EMPTY_FASTA_RECORD, rid))
+        out.append((rid, seq))
+    return out
+
+
+def header_contig_map(refs, contigs):
+    """The sample (= FASTA record index) of every sequence of the alignment header (``refs`` = [(name, length)]), -2 for a
+    sequence that is not in the FASTA; a length that differs from the FASTA record's is an InputError."""
+    index = {rid: k for k, (rid, _) in enumerate(contigs)}
+    out = []
+    for name, ln in refs:
+        k = index.get(name, -2)
+        if k >= 0 and int(ln) != len(contigs[k][1]):
+            raise InputError("%s: %s (%d vs %d)" % (ERROR_TEXT_LENGTH_MISMATCH, name, int(ln), len(contigs[k][1])))
+        out.append(k)
+    return out
+
+
+def sam_read_contigs(aln, contigs):
+    """The sample of every read of a SAM input: RNAME through the @SQ lines, or straight to the FASTA IDs when there are none;
+    '*' = no contig (-1).  A read on a sequence that is not in the FASTA is an InputError naming it."""
+    import numpy as np
+    if aln.refs:
+        m = header_contig_map(aln.refs, contigs)
+        index = {name: m[r] for r, (name, _) in enumerate(aln.refs)}
+    else:
+        index = {rid: k for k, (rid, _) in enumerate(contigs)}
+    sid = np.empty(aln.n, np.int32)
+    for i, f in enumerate(aln.sam_fields):
+        k = -1 if f[2] == '*' else index.get(f[2], -2)
+        if k == -2:
+            raise InputError("%s: %s" % (ERROR_TEXT_UNKNOWN_CONTIG, f[2]))
+        sid[i] = k
+    return sid
+
+
+def bam_read_contigs(aln, contigs):
+    """The sample of every read of a BAM input decoded on the host: its refID through header_contig_map."""
+    import numpy as np
+    m = np.array(header_contig_map(aln.refs, contigs) + [-1], np.int32)
+    if aln.n == 0:
+        return np.zeros(0, np.int32)
+    rid = aln.bam_buf[aln.bam_rec_off[:, None] + 4 + np.arange(4)].copy().view(np.int32).ravel()
+    if ((rid < -1) | (rid >= len(aln.refs))).any():
+        raise InputError(ERROR_TEXT_BAD_REFID)
+    sid = m[rid]
+    if (sid == -2).any():
+        raise InputError("%s: %s" % (ERROR_TEXT_UNKNOWN_CONTIG, aln.refs[int(rid[np.flatnonzero(sid == -2)[0]])][0]))
+    return sid
+
+
+def check_contig_plan(plan, refs=None, ref_map=None):
+    """InputError for what amp_contig_plan_* flags: reads on sequences that are not in the FASTA (named), reads without a
+    reference that are not flagged unmapped, refIDs outside the header."""
+    from .engine import CONTIG_E_BADID, CONTIG_E_NOFLAG4, CONTIG_E_UNKNOWN
+    if plan.errors & CONTIG_E_UNKNOWN:
+        names = [refs[r][0] for r in range(len(refs)) if ref_map[r] == -2 and plan.ref_reads[r]]
+        raise InputError("%s: %s" % (ERROR_TEXT_UNKNOWN_CONTIG, ", ".join(names)))
+    if plan.errors & CONTIG_E_NOFLAG4:
+        raise InputError(ERROR_TEXT_UNMAPPED_NO_FLAG)
+    if plan.errors & CONTIG_E_BADID:
+        raise InputError(ERROR_TEXT_BAD_REFID)
+
+
 def run_amplipy(untrimmed_reads_fn=None, primer_fn=None, reference_fn=None, trimmed_reads_fn=None, variants_fn=None,
                 consensus_fn=None, primer_pos_offset=None, min_length=None, min_quality=None, sliding_window_width=None,
                 min_freq_consensus=None, min_freq_variants=None, min_depth_consensus=None, min_depth_variants=None,
                 unknown_symbol=None, include_no_primer=None, run_trim=False, run_variants=False, run_consensus=False,
-                argv=None, device=0, tsv_fn=None, iupac_threshold=None):
-    """Same keyword arguments and behaviour as the reference's run_amplipy (AmpliPy.py:774-963).  Two additions of this
+                argv=None, device=0, tsv_fn=None, iupac_threshold=None, multi_contig=False):
+    """Same keyword arguments and behaviour as the reference's run_amplipy (AmpliPy.py:774-963).  Additions of this
     project: ``tsv_fn`` (with run_variants) also writes the variants in iVar's TSV format, ``iupac_threshold`` (with
-    run_consensus) writes IUPAC ambiguity codes into the consensus (DESIGN.md 3.7)."""
+    run_consensus) writes IUPAC ambiguity codes into the consensus (DESIGN.md 3.7), ``multi_contig`` takes every record of the
+    reference FASTA as a contig (DESIGN.md 3.8)."""
     argv = list(sys.argv if argv is None else argv)
     try:
         return _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
                     min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
                     min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
-                    tsv_fn if run_variants else None, iupac_threshold if run_consensus else None)
+                    tsv_fn if run_variants else None, iupac_threshold if run_consensus else None, multi_contig)
     except InputError as e:
         error(str(e))
 
 
 def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
          min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
-         unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn=None, iupac_threshold=None):
+         unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn=None, iupac_threshold=None,
+         multi_contig=False):
     # validity checks (AmpliPy.py:837-854)
     if primer_pos_offset is not None and primer_pos_offset < 0:
         error("%s: %s" % (ERROR_TEXT_NEGATIVE_PRIMER_POS_OFFSET, primer_pos_offset))
@@ -200,6 +303,11 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         print_log("Executing AmpliPy All-In-One (v%s)" % VERSION)
 
     print_log("Loading reference genome: %s" % reference_fn)
+    if multi_contig:
+        return _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
+                            min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
+                            min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
+                            tsv_fn, iupac_threshold)
     ref_id, ref_seq = load_ref_genome(reference_fn)
     L = len(ref_seq)
     tables, mpl = None, 0
@@ -366,6 +474,135 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
     return eng
 
 
+def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
+                 min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
+                 unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn, iupac_threshold):
+    """_run with --multi_contig (DESIGN.md 3.8): contig k of the FASTA is sample k of one context, with the BED rows of its chrom as
+    its scheme and its own length; reads go to the contig their reference names.  Outputs follow the FASTA's record order."""
+    contigs = load_ref_genomes(reference_fn)
+    ids = [c[0] for c in contigs]
+    lens = [len(c[1]) for c in contigs]
+    schemes = {c: [] for c in ids}
+    if primer_fn is not None:
+        print_log("Loading primers: %s" % primer_fn)
+        schemes = load_primers_by_contig(primer_fn, ids)
+    in_fn = untrimmed_reads_fn if run_trim else trimmed_reads_fn
+    if run_trim:
+        print_log("Input untrimmed SAM/BAM: %s" % untrimmed_reads_fn)
+        print_log("Output trimmed SAM/BAM: %s" % trimmed_reads_fn)
+        alnio.check_output_path(trimmed_reads_fn)
+    else:
+        print_log("Input trimmed SAM/BAM: %s" % trimmed_reads_fn)
+    if variants_fn is not None:
+        print_log("Output variants VCF: %s" % variants_fn)
+        vcf.check_output_path(variants_fn)
+    if tsv_fn is not None:
+        print_log("Output variants TSV: %s" % tsv_fn)
+        ivar.check_output_path(tsv_fn)
+    from .engine import AmpError, ContigError, Engine, TrimResult
+    qstats = tsv_fn is not None
+    pile = run_variants or run_consensus
+
+    def make_engine(indel_rich):
+        e = Engine(ref_len=max(lens), n_samples=len(contigs),
+                   min_quality=DEFAULT_MIN_QUALITY if min_quality is None else min_quality,
+                   sliding_window_width=DEFAULT_SLIDING_WINDOW_WIDTH if sliding_window_width is None else sliding_window_width,
+                   min_length=DEFAULT_MIN_LENGTH if min_length is None else min_length,
+                   include_no_primer=bool(include_no_primer), device=device,
+                   ins_slots=(1 << 24) if indel_rich else 0, ins_arena_bytes=(1 << 30) if indel_rich else 0)
+        for k, (cid, seq) in enumerate(contigs):
+            # every contig gets a scheme, empty without primers: the coordinate checks then use the contig's own length
+            e.set_scheme(k, schemes[cid], 0 if primer_pos_offset is None else primer_pos_offset, ref_len=len(seq))
+            e.set_sample_reference(k, seq)
+        if qstats or iupac_threshold is not None:
+            e.enable_qstats()
+        return e
+    mode = dict(trim=run_trim, pileup=pile, qstats=qstats)
+    eng = aln = trim = None
+    dev_bam_out = False
+    if in_fn.lower().endswith(".bam") and os.path.isfile(in_fn) and not os.environ.get("AMPLIPY_HOST_DECODE"):
+        with open(in_fn, "rb") as f:
+            raw = f.read()
+        layout = alnio.bam_layout(raw)
+        ref_map = header_contig_map(layout["refs"], contigs)
+        out_header = alnio.header_with_pg(layout["header_text"], argv) if run_trim else None
+        dev_bam_out = run_trim and trimmed_reads_fn.lower().endswith(".bam") and "AMPLIPY_BAM_LEVEL" not in os.environ
+        eng = make_engine(layout["ops_per_read"] > 8)
+        print_log("Processing reads...")
+        try:
+            info = eng.decode_bam(raw, layout)
+        except AmpError:
+            eng.close()
+            eng = None                       # e.g. records straddling BGZF blocks (not written by htslib): host decoder below
+            dev_bam_out = False
+        if eng is not None:
+            check_contig_plan(eng.contig_plan_decoded(ref_map), layout["refs"], ref_map)
+            outs = eng.process_decoded_contigs(download=not dev_bam_out, **mode)
+            eng.raise_on_device_errors()
+            n_reads = info["n"]
+            if run_trim and not dev_bam_out:
+                aln = alnio._read_bam(raw)
+                trim = TrimResult(aln.batch, *outs)
+    if eng is None:
+        aln = alnio.read_alignments(in_fn)
+        out_header = alnio.header_with_pg(aln.header_text, argv) if run_trim else None
+        sid = sam_read_contigs(aln, contigs) if aln.fmt == "sam" else bam_read_contigs(aln, contigs)
+        eng = make_engine(aln.n and (aln.batch.cigar.size / aln.n) > 8)
+        print_log("Processing reads...")
+        try:
+            trim = eng.process_contigs(aln.batch, sid, **mode)
+        except ContigError as e:
+            check_contig_plan(e.plan)
+            raise
+        eng.raise_on_device_errors()
+        n_reads = aln.n
+    for k in range(PROGRESS_NUM_READS, n_reads, PROGRESS_NUM_READS):
+        print_log("Processed %d reads..." % k)
+    if run_trim:
+        if dev_bam_out:
+            data, _ = eng.decoded_write_bam(alnio._bam_header_bytes(out_header, layout["refs"]))
+            with open(trimmed_reads_fn, "wb") as f:
+                f.write(data)
+        else:
+            on_gpu = "AMPLIPY_BAM_LEVEL" not in os.environ
+            alnio.write_alignments(trimmed_reads_fn, aln, out_header, trim, deflater=eng.bgzf_deflate if on_gpu else None)
+    if pile:
+        counts = [eng.counts(k) for k in range(len(contigs))]
+        ins = eng.insertions()
+        res = eng.call(None,
+                       DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
+                       DEFAULT_MIN_FREQ_CONSENSUS if min_freq_consensus is None else min_freq_consensus,
+                       DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
+                       DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants)
+        if run_variants:
+            vcf.write_vcf(variants_fn, ids, VERSION, argv, [calling.variant_records(res, ins, seq, counts[k], k, L=len(seq))
+                                                            for k, (_, seq) in enumerate(contigs)])
+        if tsv_fn is not None:
+            iv = eng.call_ivar(DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
+                               DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants)
+            ivar.write_tsv(tsv_fn, [r for k, (cid, seq) in enumerate(contigs)
+                                    for r in ivar.tsv_rows(res, ins, iv, eng.qstats(k), cid, seq, counts[k], k, L=len(seq))])
+        iupac = None
+        if iupac_threshold is not None:
+            iupac = eng.call_ivar(DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
+                                  DEFAULT_MIN_FREQ_CONSENSUS if min_freq_consensus is None else min_freq_consensus,
+                                  iupac_threshold).iupac
+        if run_consensus:
+            # one record per contig, headed by its ID (a repeated '>sample' would make the IDs ambiguous)
+            text = "".join('>%s\n%s\n' % (cid, calling.consensus_string(res, ins, k, unknown_symbol, iupac=iupac, L=len(seq)))
+                           for k, (cid, seq) in enumerate(contigs))
+            if consensus_fn.lower() == 'stdout':
+                sys.stdout.write(text)
+            elif consensus_fn.lower().endswith('.gz'):
+                with gzip.open(consensus_fn, 'wt') as f:
+                    f.write(text)
+            else:
+                with open(consensus_fn, 'w') as f:
+                    f.write(text)
+    print_log("Finished Processing %d reads" % max(n_reads - 1, 0))
+    return eng
+
+
 def main(argv=None):
     args = parse_args(argv)
     full_argv = list(sys.argv) if argv is None else ["AmpliPy.py"] + list(argv)
@@ -373,15 +610,16 @@ def main(argv=None):
         run_amplipy(untrimmed_reads_fn=args.input, primer_fn=args.primer, reference_fn=args.reference,
                     trimmed_reads_fn=args.output, primer_pos_offset=args.primer_pos_offset, min_length=args.min_length,
                     min_quality=args.min_quality, sliding_window_width=args.sliding_window_width,
-                    include_no_primer=args.include_no_primer, run_trim=True, argv=full_argv)
+                    include_no_primer=args.include_no_primer, run_trim=True, argv=full_argv, multi_contig=args.multi_contig)
     elif args.command == 'variants':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, variants_fn=args.output,
                     min_quality=args.min_quality, min_freq_variants=args.min_freq, min_depth_variants=args.min_depth,
-                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv)
+                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv, multi_contig=args.multi_contig)
     elif args.command == 'consensus':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, consensus_fn=args.output,
                     min_quality=args.min_quality, min_freq_consensus=args.min_freq, min_depth_consensus=args.min_depth,
-                    unknown_symbol=args.unknown_symbol, run_consensus=True, argv=full_argv, iupac_threshold=args.iupac_threshold)
+                    unknown_symbol=args.unknown_symbol, run_consensus=True, argv=full_argv, iupac_threshold=args.iupac_threshold,
+                    multi_contig=args.multi_contig)
     elif args.command == 'aio':
         run_amplipy(untrimmed_reads_fn=args.input, primer_fn=args.primer, reference_fn=args.reference,
                     trimmed_reads_fn=args.output_trimmed_reads, variants_fn=args.output_variants,
@@ -391,7 +629,7 @@ def main(argv=None):
                     min_depth_consensus=args.min_depth_consensus, min_depth_variants=args.min_depth_variants,
                     unknown_symbol=args.unknown_symbol, include_no_primer=args.include_no_primer, run_trim=True,
                     run_variants=True, run_consensus=True, argv=full_argv, tsv_fn=args.output_tsv,
-                    iupac_threshold=args.iupac_threshold)
+                    iupac_threshold=args.iupac_threshold, multi_contig=args.multi_contig)
 
 
 if __name__ == "__main__":

@@ -16,6 +16,7 @@
 #include "amp_ont.cuh"
 #include "amp_deflate.cuh"
 #include "amp_ivar.cuh"
+#include "amp_contig.cuh"
 
 static_assert(AMP_F_TRIM_START == AMP_FLAG_TRIM_START && AMP_F_KEEP == AMP_FLAG_KEEP && AMP_F_SKIPPED == AMP_FLAG_SKIPPED &&
                   AMP_F_ERROR == AMP_FLAG_ERROR && AMP_E_ARENA_FULL == AMP_DEVERR_ARENA_FULL &&
@@ -378,6 +379,36 @@ __global__ void __launch_bounds__(256) amp_bam_scatter_kernel(const uint8_t* raw
     }
 }
 
+// ---- a batch grouped by contig (amp_contig.cuh): plan, stable counting sort, permuted copy, outputs back to input order ----------
+__global__ void __launch_bounds__(AMP_CT_THREADS) amp_contig_plan_kernel(const __grid_constant__ amp::ContigPlanParams P) {
+    __shared__ amp::ContigPlanSmem sm;
+    amp::contig_plan_cta(P, sm, (int)blockIdx.x);
+}
+__global__ void __launch_bounds__(AMP_CT_THREADS) amp_contig_scan_kernel(const __grid_constant__ amp::ContigScanParams P0,
+                                                                        const __grid_constant__ amp::ContigScanParams P1,
+                                                                        const __grid_constant__ amp::ContigScanParams P2) {
+    __shared__ unsigned long long part[AMP_CT_THREADS];
+    amp::contig_scan_cta(blockIdx.y == 0 ? P0 : blockIdx.y == 1 ? P1 : P2, part);
+}
+__global__ void __launch_bounds__(AMP_CT_THREADS) amp_contig_rank_kernel(const __grid_constant__ amp::ContigRankParams P) {
+    __shared__ amp::ContigRankSmem sm;
+    amp::contig_rank_cta(P, sm, (int)blockIdx.x);
+}
+__global__ void __launch_bounds__(AMP_CT_THREADS) amp_contig_tilesum_kernel(const __grid_constant__ amp::ContigGatherParams P) {
+    __shared__ unsigned long long part[AMP_CT_THREADS];
+    amp::contig_tilesum_cta(P, part, (int)blockIdx.x);
+}
+__global__ void __launch_bounds__(AMP_CT_THREADS) amp_contig_gather_kernel(const __grid_constant__ amp::ContigGatherParams P) {
+    __shared__ unsigned long long part[AMP_CT_THREADS];
+    amp::contig_gather_cta(P, part, (int)blockIdx.x);
+}
+__global__ void __launch_bounds__(256) amp_contig_unpermute_kernel(const __grid_constant__ amp::ContigUnpermuteParams P) {
+    amp::contig_unpermute_warp(P, (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5, ((long long)gridDim.x * blockDim.x) >> 5);
+}
+__global__ void __launch_bounds__(256) amp_contig_skip_kernel(const __grid_constant__ amp::ContigSkipParams P) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < P.n; i += (long long)gridDim.x * blockDim.x) amp::contig_skip_read(P, i);
+}
+
 struct DevChunk {   // device staging for one in-flight chunk of amp_process_host
     cudaStream_t stream = nullptr;
     int32_t* pos = nullptr; uint16_t* flag = nullptr; int32_t* tlen = nullptr;
@@ -444,6 +475,19 @@ struct amp_ctx {
     int* d_ins_rev = nullptr; unsigned long long* d_ins_qsum = nullptr; unsigned char* d_ins_head = nullptr;
     unsigned char* d_ivar = nullptr;    // iVar calling outputs (one block, offsets below)
     size_t o_iu = 0, o_fmq = 0, o_fpv = 0, o_imq = 0, o_ipv = 0;
+    // a batch grouped by contig (amp_contig_plan_* / amp_process_contigs; buffers grown at high-water marks)
+    struct Contigs {
+        int source = 0;                                           // the planned batch: 0 none, 1 the decoded one, 2 a device batch
+        amp::BatchPtrs b{}; long long sum_cig = 0; bool grouped = false;   // the planned batch, its CIGAR ops, its plan's verdict
+        int* sid = nullptr; size_t cap_sid = 0; uint32_t* hist = nullptr; size_t cap_hist = 0; uint32_t* hist_off = nullptr; size_t cap_hoff = 0;
+        unsigned long long* table = nullptr; size_t cap_table = 0; std::vector<unsigned long long> h_table;
+        uint32_t* perm = nullptr; size_t cap_perm = 0; uint32_t* tsum = nullptr; size_t cap_tsum = 0; uint32_t* tbase = nullptr; size_t cap_tbase = 0;
+        int32_t* pos = nullptr; size_t cap_pos = 0; uint16_t* flag = nullptr; size_t cap_flag = 0; int32_t* tlen = nullptr; size_t cap_tlen = 0;
+        uint32_t* cig_off = nullptr; size_t cap_coff = 0; uint32_t* seq_off = nullptr; size_t cap_soff = 0; uint32_t* qual_off = nullptr; size_t cap_qoff = 0;
+        uint32_t* cigar = nullptr; size_t cap_cig = 0; uint8_t* seq = nullptr; size_t cap_seq = 0; uint8_t* qual = nullptr; size_t cap_qual = 0;
+        int32_t* o_pos = nullptr; size_t cap_opos = 0; uint16_t* o_ncig = nullptr; size_t cap_oncig = 0; uint8_t* o_flags = nullptr; size_t cap_oflags = 0;
+        uint32_t* o_cigar = nullptr; size_t cap_ocig = 0; uint32_t* scratch = nullptr; size_t cap_scratch = 0;
+    } ct;
 };
 
 namespace {
@@ -688,6 +732,12 @@ int amp_destroy(amp_ctx* c) {
         for (void* q : ps) cudaFree(q);
         for (auto& e : d.ev) if (e) cudaEventDestroy(e);
         for (auto& z : d.zs) if (z) cudaStreamDestroy(z);
+    }
+    {
+        auto& t = c->ct;
+        void* ps[] = {t.sid, t.hist, t.hist_off, t.table, t.perm, t.tsum, t.tbase, t.pos, t.flag, t.tlen, t.cig_off, t.seq_off, t.qual_off, t.cigar,
+                      t.seq, t.qual, t.o_pos, t.o_ncig, t.o_flags, t.o_cigar, t.scratch};
+        for (void* q : ps) cudaFree(q);
     }
     for (auto& ch : c->chunk) {
         cudaFree(ch.pos); cudaFree(ch.flag); cudaFree(ch.tlen); cudaFree(ch.cig_off); cudaFree(ch.seq_off); cudaFree(ch.qual_off);
@@ -1432,6 +1482,7 @@ int amp_bam_decode_host(amp_ctx* c, const uint8_t* bgzf, int64_t n_bytes, const 
     CK(cudaSetDevice(c->cfg.device));
     auto& d = c->dec;
     d.valid = false; d.trimmed = false;
+    if (c->ct.source == 1) c->ct.source = 0;
     cudaStream_t sc = c->chunk[0].stream, sx = c->chunk[1].stream;    // compute / copy
     CK(cudaStreamSynchronize(sc)); CK(cudaStreamSynchronize(sx));
     // host-side tables: block ends, output offsets
@@ -1667,6 +1718,242 @@ int amp_set_sample_reference(amp_ctx* c, int sample, const char* ref_seq, int32_
     }
     CK(cudaMemset(c->d_ref + (size_t)sample * L, 'N', L));
     CK(cudaMemcpy(c->d_ref + (size_t)sample * L, ref_seq, (size_t)len, cudaMemcpyHostToDevice));
+    return AMP_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------
+// a batch grouped by contig (amp_contig.cuh, DESIGN.md 3.8): contig k = sample k of the context
+// ---------------------------------------------------------------------------------------------------
+namespace {
+
+// plan kernel + one copy of its table; P.raw / rec_off / ref_to_sample or P.sample_in set by the caller
+int contig_plan(amp_ctx* c, amp::ContigPlanParams P, const amp::BatchPtrs& b, int source, amp_contig_plan* plan) {
+    auto& t = c->ct;
+    t.source = 0;
+    const int S = c->cfg.n_samples;
+    if (S > AMP_MAX_CONTIGS) return fail(AMP_ERR_ARG, "amp_contig_plan: more contigs than AMP_MAX_CONTIGS (1024)");
+    cudaStream_t sc = c->chunk[0].stream;
+    const long long n = b.n, n_tiles = (n + AMP_CT_TILE - 1) / AMP_CT_TILE;
+    const size_t words = amp::ct_table_words(S, P.n_refs);
+    int rc;
+    if ((rc = dev_grow(&t.sid, &t.cap_sid, (size_t)n + 1))) return rc;
+    if ((rc = dev_grow(&t.hist, &t.cap_hist, (size_t)n_tiles * S + 1))) return rc;
+    if ((rc = dev_grow(&t.table, &t.cap_table, words))) return rc;
+    CK(cudaMemsetAsync(t.table, 0, words * 8, sc));
+    P.n = n; P.flag = b.flag; P.cig_off = b.cig_off; P.qual_off = b.qual_off; P.S = S;
+    P.sid = t.sid; P.tile_hist = t.hist; P.table = t.table;
+    c->last_launches = 0;
+    if (n_tiles) {
+        amp_contig_plan_kernel<<<(unsigned)n_tiles, AMP_CT_THREADS, 0, sc>>>(P);
+        CK(cudaGetLastError());
+        c->last_launches = 1;
+    }
+    t.h_table.assign(words, 0ULL);
+    CK(cudaMemcpyAsync(t.h_table.data(), t.table, words * 8, cudaMemcpyDeviceToHost, sc));
+    CK(cudaStreamSynchronize(sc));
+    const unsigned long long* T = t.h_table.data();
+    int present = T[0] ? 1 : 0;
+    for (int k = 0; k < S; ++k) present += T[AMP_CT_HDR + k] ? 1 : 0;
+    plan->n_reads = n; plan->n_no_contig = (int64_t)T[0]; plan->errors = (uint32_t)T[2];
+    plan->grouped = (n == 0 || T[1] + 1 == (unsigned long long)present) ? 1 : 0;
+    for (int k = 0; k < S; ++k) {
+        const unsigned long long cnt = T[AMP_CT_HDR + k];
+        if (plan->contig_reads) plan->contig_reads[k] = (int64_t)cnt;
+        if (plan->contig_first) plan->contig_first[k] = cnt ? (int64_t)~T[AMP_CT_HDR + 3 * (size_t)S + k] : 0;
+        if (plan->contig_cigar_ops) plan->contig_cigar_ops[k] = (int64_t)T[AMP_CT_HDR + (size_t)S + k];
+        if (plan->contig_qual_bytes) plan->contig_qual_bytes[k] = (int64_t)T[AMP_CT_HDR + 2 * (size_t)S + k];
+    }
+    if (plan->ref_reads) for (int r = 0; r < P.n_refs; ++r) plan->ref_reads[r] = (int64_t)T[AMP_CT_HDR + 5 * (size_t)S + r];
+    t.b = b; t.sum_cig = (long long)T[3]; t.grouped = plan->grouped != 0;
+    t.source = source;
+    return AMP_OK;
+}
+
+// the permuted copy of the planned batch: one range per contig, in contig order, into t.pos ... t.qual
+int contig_permute(amp_ctx* c, cudaStream_t sc) {
+    auto& t = c->ct;
+    const int S = c->cfg.n_samples;
+    const long long n = t.b.n, n_tiles = (n + AMP_CT_TILE - 1) / AMP_CT_TILE;
+    const unsigned long long* T = t.h_table.data();
+    long long sum_seq = 0, sum_qual = 0, n_in = 0;
+    for (int k = 0; k < S; ++k) { n_in += (long long)T[AMP_CT_HDR + k]; sum_qual += (long long)T[AMP_CT_HDR + 2 * (size_t)S + k]; }
+    int rc;
+    if ((rc = dev_grow(&t.hist_off, &t.cap_hoff, (size_t)n_tiles * S + 1))) return rc;
+    if ((rc = dev_grow(&t.perm, &t.cap_perm, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.tsum, &t.cap_tsum, (size_t)n_tiles * 3 + 3))) return rc;
+    if ((rc = dev_grow(&t.tbase, &t.cap_tbase, 3 * ((size_t)n_tiles + 1) + 3))) return rc;
+    // contig-major prefix sums of the tile histograms: the place of each tile's first read of each contig
+    amp::ContigScanParams H{t.hist, (long long)S * n_tiles, n_tiles, (long long)S, 1, t.hist_off};
+    amp_contig_scan_kernel<<<dim3(1, 1), AMP_CT_THREADS, 0, sc>>>(H, H, H);
+    CK(cudaGetLastError());
+    amp::ContigRankParams R{n, S, n_tiles, t.sid, t.hist_off, t.perm};
+    amp_contig_rank_kernel<<<(unsigned)n_tiles, AMP_CT_THREADS, 0, sc>>>(R);
+    CK(cudaGetLastError());
+    // rows of the permuted batch: the seq bytes are not in the plan (they follow from the quality bytes); size them from those
+    sum_seq = sum_qual / 2 + n_in;
+    const long long pt = (n_in + AMP_CT_TILE - 1) / AMP_CT_TILE;
+    if ((rc = dev_grow(&t.pos, &t.cap_pos, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.flag, &t.cap_flag, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.tlen, &t.cap_tlen, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.cig_off, &t.cap_coff, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.seq_off, &t.cap_soff, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.qual_off, &t.cap_qoff, (size_t)n_in + 1))) return rc;
+    if ((rc = dev_grow(&t.cigar, &t.cap_cig, (size_t)t.sum_cig + 8))) return rc;
+    if ((rc = dev_grow(&t.seq, &t.cap_seq, (size_t)sum_seq + 64))) return rc;          // + the 16-byte reads past the end (DESIGN.md 2)
+    if ((rc = dev_grow(&t.qual, &t.cap_qual, (size_t)sum_qual + 64))) return rc;
+    amp::ContigGatherParams G{};
+    G.n = n_in; G.n_tiles = pt; G.perm = t.perm; G.src = t.b; G.src.first = 0;
+    G.pos = t.pos; G.flag = t.flag; G.tlen = t.tlen; G.cig_off = t.cig_off; G.cigar = t.cigar; G.seq_off = t.seq_off; G.seq = t.seq;
+    G.qual_off = t.qual_off; G.qual = t.qual; G.tsum = t.tsum; G.tbase = t.tbase;
+    if (n_in == 0) {
+        CK(cudaMemsetAsync(t.cig_off, 0, 4, sc)); CK(cudaMemsetAsync(t.seq_off, 0, 4, sc)); CK(cudaMemsetAsync(t.qual_off, 0, 4, sc));
+        c->last_launches += 2;
+        return AMP_OK;
+    }
+    amp_contig_tilesum_kernel<<<(unsigned)pt, AMP_CT_THREADS, 0, sc>>>(G);
+    CK(cudaGetLastError());
+    amp::ContigScanParams Q[3];
+    for (int ch = 0; ch < 3; ++ch) Q[ch] = amp::ContigScanParams{t.tsum + ch, pt, pt, 3, 0, t.tbase + (size_t)ch * (pt + 1)};
+    amp_contig_scan_kernel<<<dim3(1, 3), AMP_CT_THREADS, 0, sc>>>(Q[0], Q[1], Q[2]);
+    CK(cudaGetLastError());
+    amp_contig_gather_kernel<<<(unsigned)pt, AMP_CT_THREADS, 0, sc>>>(G);
+    CK(cudaGetLastError());
+    CK(cudaMemsetAsync(t.seq + sum_seq, 0, 64, sc));
+    c->last_launches += 5;
+    return AMP_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int amp_contig_plan_decoded(amp_ctx* c, const int32_t* ref_to_sample, int32_t n_refs, amp_contig_plan* plan) {
+    if (!c || !plan || n_refs < 0 || (n_refs && !ref_to_sample)) return fail(AMP_ERR_ARG, "amp_contig_plan_decoded: bad argument");
+    auto& d = c->dec;
+    if (!d.valid) return fail(AMP_ERR_STATE, "amp_contig_plan_decoded: no decoded batch (amp_bam_decode_host first)");
+    CK(cudaSetDevice(c->cfg.device));
+    int rc;
+    if ((rc = dev_grow(&c->d_xbuf, &c->xbuf_bytes, (size_t)n_refs * 4 + 64))) return rc;
+    int* d_map = (int*)c->d_xbuf;
+    if (n_refs) CK(cudaMemcpyAsync(d_map, ref_to_sample, (size_t)n_refs * 4, cudaMemcpyHostToDevice, c->chunk[0].stream));
+    amp::ContigPlanParams P{};
+    P.raw = d.raw; P.rec_off = d.rec_off; P.ref_to_sample = d_map; P.n_refs = n_refs;
+    amp::BatchPtrs b{0, d.n_reads, d.pos, d.flag, d.tlen, d.cig_off, d.cigar, d.seq_off, d.seq, d.qual_off, d.qual};
+    return contig_plan(c, P, b, 1, plan);
+}
+
+int amp_contig_plan_device(amp_ctx* c, const amp_batch* b, const int32_t* dev_sample_of_read, amp_contig_plan* plan) {
+    if (!c || !b || !plan || (b->n_reads && !dev_sample_of_read) || b->first != 0 || b->n_reads < 0)
+        return fail(AMP_ERR_ARG, "amp_contig_plan_device: bad argument (the batch must start at read 0)");
+    CK(cudaSetDevice(c->cfg.device));
+    amp::ContigPlanParams P{};
+    P.sample_in = dev_sample_of_read;
+    amp::BatchPtrs bp{0, b->n_reads, b->pos, b->flag, b->tlen, b->cig_off, b->cigar, b->seq_off, b->seq, b->qual_off, b->qual};
+    if (plan->ref_reads) return fail(AMP_ERR_ARG, "amp_contig_plan_device: ref_reads is for the decoded plan");
+    return contig_plan(c, P, bp, 2, plan);
+}
+
+int amp_process_contigs(amp_ctx* c, int mode, const amp_trim_out* dev_out, const amp_trim_out* host_out) {
+    if (!c) return fail(AMP_ERR_ARG, "amp_process_contigs: null context");
+    auto& t = c->ct;
+    auto& d = c->dec;
+    if (!t.source || (t.source == 1 && !d.valid)) return fail(AMP_ERR_STATE, "amp_process_contigs: no planned batch (amp_contig_plan_* first)");
+    const int S = c->cfg.n_samples;
+    const unsigned long long* T = t.h_table.data();
+    if (T[2]) return fail(AMP_ERR_DATA, "amp_process_contigs: the plan found reads without a valid contig (amp_contig_plan.errors)");
+    if (!(mode & (AMP_MODE_TRIM | AMP_MODE_PILEUP))) return fail(AMP_ERR_ARG, "amp_process_contigs: empty mode");
+    if (int rc = check_qstats_mode(c, mode, "amp_process_contigs")) return rc;
+    const bool trim = mode & AMP_MODE_TRIM;
+    if (t.source == 1 && dev_out) return fail(AMP_ERR_ARG, "amp_process_contigs: the decoded batch keeps its trim outputs in the context (dev_out must be NULL)");
+    if (t.source == 2 && trim && !dev_out) return fail(AMP_ERR_ARG, "amp_process_contigs: trimming a device batch needs dev_out");
+    for (int k = 0; k < S && trim; ++k)
+        if (T[AMP_CT_HDR + k] && !has_scheme(c, k)) return fail(AMP_ERR_ARG, "amp_process_contigs: trimming needs a scheme for every contig with reads");
+    CK(cudaSetDevice(c->cfg.device));
+    cudaStream_t sc = c->chunk[0].stream;
+    const long long n = t.b.n;
+    const size_t orows = (size_t)t.sum_cig + 3 * (size_t)n;
+    int rc;
+    amp::TrimOut out{};
+    if (trim && t.source == 1) {
+        if ((rc = dev_grow(&d.o_cigar, &d.cap_ocig, orows + 8))) return rc;
+        out.pos = d.o_pos; out.ncig = d.o_ncig; out.flags = d.o_flags; out.cigar = d.o_cigar;
+    } else if (trim) {
+        out.pos = dev_out->pos; out.ncig = dev_out->ncig; out.flags = dev_out->flags; out.cigar = dev_out->cigar;
+    }
+    if (trim && (rc = dev_grow(&t.scratch, &t.cap_scratch, 2 * (orows + 8)))) return rc;
+    {
+        const size_t need = glist_words_for(c, n);
+        if (need > c->glist_words) {
+            CK(cudaStreamSynchronize(sc));
+            if (c->d_glist) CK(cudaFree(c->d_glist));
+            c->d_glist = nullptr; c->glist_words = 0;
+            CK(cudaMalloc((void**)&c->d_glist, need * 4));
+            c->glist_words = need;
+        }
+    }
+    c->last_launches = 0;
+    if (t.grouped) {
+        // one launch per contig over its own range of the batch; scratch rows are addressed like the output rows, from the range start
+        for (int k = 0; k < S; ++k) {
+            const long long cnt = (long long)T[AMP_CT_HDR + k];
+            if (!cnt) continue;
+            const long long first = (long long)~T[AMP_CT_HDR + 3 * (size_t)S + k], cfirst = (long long)T[AMP_CT_HDR + 4 * (size_t)S + k];
+            amp::BatchPtrs bk = t.b;
+            bk.first = first; bk.n = cnt;
+            const long long scig = (long long)T[AMP_CT_HDR + (size_t)S + k], squal = (long long)T[AMP_CT_HDR + 2 * (size_t)S + k];
+            if ((rc = launch_process(c, bk, scig, 0, squal > 0 ? squal : 1, mode, k, out, trim ? t.scratch - (cfirst + 3 * first) : nullptr,
+                                     c->d_glist, sc))) return rc;
+        }
+    } else {
+        if ((rc = contig_permute(c, sc))) return rc;
+        long long n_in = 0;
+        for (int k = 0; k < S; ++k) n_in += (long long)T[AMP_CT_HDR + k];
+        amp::TrimOut po{};
+        if (trim) {
+            if ((rc = dev_grow(&t.o_pos, &t.cap_opos, (size_t)n_in + 1))) return rc;
+            if ((rc = dev_grow(&t.o_ncig, &t.cap_oncig, (size_t)n_in + 1))) return rc;
+            if ((rc = dev_grow(&t.o_flags, &t.cap_oflags, (size_t)n_in + 1))) return rc;
+            if ((rc = dev_grow(&t.o_cigar, &t.cap_ocig, (size_t)t.sum_cig + 3 * (size_t)n_in + 8))) return rc;
+            po.pos = t.o_pos; po.ncig = t.o_ncig; po.flags = t.o_flags; po.cigar = t.o_cigar;
+        }
+        const amp::BatchPtrs pb{0, n_in, t.pos, t.flag, t.tlen, t.cig_off, t.cigar, t.seq_off, t.b.seq ? t.seq : nullptr, t.qual_off, t.qual};
+        long long first = 0, cfirst = 0;
+        for (int k = 0; k < S; ++k) {
+            const long long cnt = (long long)T[AMP_CT_HDR + k];
+            const long long scig = (long long)T[AMP_CT_HDR + (size_t)S + k], squal = (long long)T[AMP_CT_HDR + 2 * (size_t)S + k];
+            if (cnt) {
+                amp::BatchPtrs bk = pb;
+                bk.first = first; bk.n = cnt;
+                if ((rc = launch_process(c, bk, scig, 0, squal > 0 ? squal : 1, mode, k, po, trim ? t.scratch - (cfirst + 3 * first) : nullptr,
+                                         c->d_glist, sc))) return rc;
+            }
+            first += cnt; cfirst += scig;
+        }
+        if (trim && n_in) {
+            amp::ContigUnpermuteParams U{n_in, t.perm, t.cig_off, po, t.b.cig_off, out};
+            const long long grid = std::min<long long>((n_in + 7) / 8, (long long)c->sm_count * 16);
+            amp_contig_unpermute_kernel<<<(unsigned)grid, 256, 0, sc>>>(U);
+            CK(cudaGetLastError());
+            c->last_launches += 1;
+        }
+    }
+    if (trim && T[0]) {
+        amp::ContigSkipParams K{n, t.sid, t.b, out};
+        const long long grid = std::min<long long>((n + 255) / 256, (long long)c->sm_count * 8);
+        amp_contig_skip_kernel<<<(unsigned)grid, 256, 0, sc>>>(K);
+        CK(cudaGetLastError());
+        c->last_launches += 1;
+    }
+    if (trim && t.source == 1) d.trimmed = true;
+    if (trim && host_out && n) {
+        if (host_out->pos) CK(cudaMemcpyAsync(host_out->pos, out.pos, (size_t)n * 4, cudaMemcpyDeviceToHost, sc));
+        if (host_out->ncig) CK(cudaMemcpyAsync(host_out->ncig, out.ncig, (size_t)n * 2, cudaMemcpyDeviceToHost, sc));
+        if (host_out->flags) CK(cudaMemcpyAsync(host_out->flags, out.flags, (size_t)n, cudaMemcpyDeviceToHost, sc));
+        if (host_out->cigar) CK(cudaMemcpyAsync(host_out->cigar, out.cigar, orows * 4, cudaMemcpyDeviceToHost, sc));
+    }
+    CK(cudaStreamSynchronize(sc));
     return AMP_OK;
 }
 

@@ -42,7 +42,7 @@ EXPORTED_SYMBOLS = [
     "amp_ins_slot_bytes", "amp_ins_pack_device", "amp_ins_merge_packed", "amp_reserve", "amp_counts_copy_device",
     "amp_bam_decode_host", "amp_process_decoded", "amp_decoded_copy_host", "amp_counts_upload", "amp_bgzf_deflate_host", "amp_decoded_write_bam",
     "amp_set_scheme", "amp_get_scheme", "amp_set_sample_reference", "amp_qstats_enable", "amp_qstats_host", "amp_call_ivar",
-    "amp_call_ivar_device"]
+    "amp_call_ivar_device", "amp_contig_plan_decoded", "amp_contig_plan_device", "amp_process_contigs"]
 
 
 class AmpConfig(ctypes.Structure):
@@ -72,6 +72,33 @@ class AmpBatchOut(ctypes.Structure):
     _fields_ = [("pos", ctypes.c_void_p), ("flag", ctypes.c_void_p), ("tlen", ctypes.c_void_p), ("cig_off", ctypes.c_void_p),
                 ("cigar", ctypes.c_void_p), ("seq_off", ctypes.c_void_p), ("seq", ctypes.c_void_p), ("qual_off", ctypes.c_void_p),
                 ("qual", ctypes.c_void_p)]
+
+
+class AmpContigPlan(ctypes.Structure):
+    _fields_ = [("n_reads", ctypes.c_int64), ("n_no_contig", ctypes.c_int64), ("grouped", ctypes.c_int32), ("errors", ctypes.c_uint32),
+                ("contig_reads", ctypes.c_void_p), ("contig_first", ctypes.c_void_p), ("contig_cigar_ops", ctypes.c_void_p),
+                ("contig_qual_bytes", ctypes.c_void_p), ("ref_reads", ctypes.c_void_p)]
+
+
+CONTIG_E_NOFLAG4, CONTIG_E_UNKNOWN, CONTIG_E_BADID = 1, 2, 4
+
+
+class ContigPlan:
+    """What amp_contig_plan_* found in a batch: per contig (= sample) its reads, first read, CIGAR ops and quality bytes; the
+    reads without a contig; whether every contig's reads are contiguous; error bits (CONTIG_E_*) and, for a decoded BAM, the
+    reads on each header sequence that is not in the FASTA."""
+
+    def __init__(self, n_samples, n_refs=0):
+        self.reads, self.first = np.zeros(n_samples, np.int64), np.zeros(n_samples, np.int64)
+        self.cigar_ops, self.qual_bytes = np.zeros(n_samples, np.int64), np.zeros(n_samples, np.int64)
+        self.ref_reads = np.zeros(max(n_refs, 1), np.int64)[:n_refs]
+        self.c = AmpContigPlan(0, 0, 0, 0, _ptr(self.reads), _ptr(self.first), _ptr(self.cigar_ops), _ptr(self.qual_bytes),
+                               _ptr(self.ref_reads) if n_refs else None)
+
+    n_reads = property(lambda self: int(self.c.n_reads))
+    n_no_contig = property(lambda self: int(self.c.n_no_contig))
+    grouped = property(lambda self: bool(self.c.grouped))
+    errors = property(lambda self: int(self.c.errors))
 
 
 class AmpCallParams(ctypes.Structure):
@@ -123,6 +150,14 @@ def _check(rc, what):
 
 def _ptr(a):
     return None if a is None else ctypes.c_void_p(a.ctypes.data)
+
+
+class ContigError(AmpError):
+    """amp_contig_plan_* flagged reads without a valid contig (``plan.errors``); nothing was processed."""
+
+    def __init__(self, plan):
+        super().__init__("contig plan error bits 0x%x" % plan.errors)
+        self.plan = plan
 
 
 class TrimResult:
@@ -437,6 +472,61 @@ class Engine:
         _check(self.lib.amp_process_decoded(self._ctx, mode, sample, ctypes.byref(to) if to else None), "amp_process_decoded")
         self.launches += int(self.lib.amp_last_launches(self._ctx))
         return out
+
+    # ---------------------------------------------------------------- multi-contig references (DESIGN.md 3.8): contig k = sample k
+    def contig_plan_decoded(self, ref_to_sample):
+        """Contig of every read of the batch decode_bam left in HBM: its BAM refID through ``ref_to_sample`` (one entry per header
+        sequence: the sample, -1 = no contig, -2 = not in the FASTA).  Returns a ContigPlan."""
+        m = np.ascontiguousarray(ref_to_sample, np.int32)
+        plan = ContigPlan(self.n_samples, m.size)
+        _check(self.lib.amp_contig_plan_decoded(self._ctx, _ptr(m) if m.size else None, int(m.size), ctypes.byref(plan.c)),
+               "amp_contig_plan_decoded")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        self.contig_plan = plan
+        return plan
+
+    def process_decoded_contigs(self, trim=True, pileup=True, qstats=False, download=True, out=None):
+        """The fused kernel once per contig over the planned decoded batch (contig_plan_decoded first): trim outputs in input order,
+        copied to ``out`` (alloc_decoded_trim_out) unless ``download=False`` (decoded_write_bam reads them on the device)."""
+        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0) | (MODE_QSTATS if qstats else 0)
+        to = None
+        if trim and download:
+            if out is None:
+                out = self.alloc_decoded_trim_out()
+            to = AmpTrimOut(_ptr(out[0]), _ptr(out[1]), _ptr(out[2]), _ptr(out[3]))
+        _check(self.lib.amp_process_contigs(self._ctx, mode, None, ctypes.byref(to) if to else None), "amp_process_contigs")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        return out
+
+    def process_contigs(self, batch, sample_of_read, trim=True, pileup=True, qstats=False):
+        """A host batch whose read i belongs to sample_of_read[i] (-1: no contig; such a read must carry flag 4): uploaded, planned
+        (self.contig_plan) and processed by the same device routine as the decoded path.  Returns TrimResult when trim=True; raises
+        ContigError when the plan has error bits."""
+        import torch
+        sid = np.ascontiguousarray(sample_of_read, np.int32)
+        assert sid.shape == (batch.n,)
+        d = self.upload(batch, trim_out=trim)
+        dsid = torch.from_numpy(sid).to(torch.device("cuda", self.device)) if batch.n else torch.zeros(1, dtype=torch.int32,
+                                                                                                    device=torch.device("cuda", self.device))
+        p = lambda t: ctypes.c_void_p(t.data_ptr())
+        db = AmpBatch(0, batch.n, p(d["pos"]), p(d["flag"]), p(d["tlen"]), p(d["cig_off"]), p(d["cigar"]), p(d["seq_off"]), p(d["seq"]),
+                      p(d["qual_off"]), p(d["qual"]))
+        plan = ContigPlan(self.n_samples)
+        _check(self.lib.amp_contig_plan_device(self._ctx, ctypes.byref(db), p(dsid), ctypes.byref(plan.c)), "amp_contig_plan_device")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        self.contig_plan = plan
+        if plan.errors:
+            raise ContigError(plan)
+        mode = (MODE_TRIM if trim else 0) | (MODE_PILEUP if pileup else 0) | (MODE_QSTATS if qstats else 0)
+        dto = hto = out = None
+        if trim:
+            out = self.alloc_trim_out(batch)
+            dto = AmpTrimOut(p(d["o_pos"]), p(d["o_ncig"]), p(d["o_flags"]), p(d["o_cigar"]))
+            hto = AmpTrimOut(_ptr(out[0]), _ptr(out[1]), _ptr(out[2]), _ptr(out[3]))
+        _check(self.lib.amp_process_contigs(self._ctx, mode, ctypes.byref(dto) if dto else None, ctypes.byref(hto) if hto else None),
+               "amp_process_contigs")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        return TrimResult(batch, *out) if trim else None
 
     def decoded_batch(self):
         """The decoded batch copied back to the host as a ReadBatch, plus the offset of every record in the inflated stream."""

@@ -61,11 +61,12 @@ def alt_text(sym, ref_char, head=False):
     return "+" + (sym[:-1] if head else sym[1:])
 
 
-def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0):
+def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None):
     """The TSV rows of one sample: every allele with a p-value (count > 0, symbol != the FASTA character, freq >= min_freq, depth
-    >= min_depth), in position order, then in the reference's allele order (AmpliPy.py:771)."""
-    L = res.L
-    base = sample * L
+    >= min_depth), in position order, then in the reference's allele order (AmpliPy.py:771).  ``L``: the sample's own reference
+    length when it is shorter than the context's (a contig of a multi-record FASTA)."""
+    L = res.L if L is None else L
+    base = sample * res.L
     fpv = iv.fixed_pval[base:base + L]
     ins_rows = {}
     if ins.k:

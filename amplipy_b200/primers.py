@@ -9,32 +9,50 @@ import numpy as np
 ERROR_TEXT_EMPTY_BED = "Empty BED file"
 ERROR_TEXT_FILE_NOT_FOUND = "File not found"
 ERROR_TEXT_INVALID_BED_LINE = "Invalid primer BED line"
+ERROR_TEXT_BED_CHROM_NOT_IN_FASTA = "Primer BED chrom is not a sequence of the reference FASTA"
 
 
 class InputError(Exception):
     """Carries the reference's error text; the CLI prints it the way AmpliPy.py:85-90 does."""
 
 
-def load_primers(primer_fn):
-    """4-column BED -> sorted [(start, end)] (AmpliPy.py:235-258).  Any other column count is an
-    "Invalid primer BED line", as in the reference."""
+def _bed_rows(primer_fn):
+    """4-column BED -> [(chrom, start, end)] in file order.  Any other column count is an "Invalid primer BED line", as in the
+    reference (AmpliPy.py:235-258); no rows is an "Empty BED file"."""
     if not os.path.isfile(primer_fn):
         raise InputError("%s: %s" % (ERROR_TEXT_FILE_NOT_FOUND, primer_fn))
     with open(primer_fn, "r") as f:
         lines = f.read().strip().splitlines()
-    primers = []
+    rows = []
     for l in lines:
         parts = l.split("\t")
         try:
             if len(parts) != 4:
                 raise ValueError
-            primers.append((int(parts[1]), int(parts[2])))
+            rows.append((parts[0], int(parts[1]), int(parts[2])))
         except ValueError:
             raise InputError("%s: %s" % (ERROR_TEXT_INVALID_BED_LINE, l))
-    if len(primers) == 0:
+    if len(rows) == 0:
         raise InputError("%s: %s" % (ERROR_TEXT_EMPTY_BED, primer_fn))
-    primers.sort()
-    return primers
+    return rows
+
+
+def load_primers(primer_fn):
+    """4-column BED -> sorted [(start, end)] (AmpliPy.py:235-258); the chrom column is ignored, as in the reference."""
+    return sorted((s, e) for _, s, e in _bed_rows(primer_fn))
+
+
+def load_primers_by_contig(primer_fn, contig_ids):
+    """4-column BED -> {contig ID: sorted [(start, end)]} for every ID of ``contig_ids`` (an empty list for a contig without
+    primers); a chrom that is not one of them is an InputError."""
+    out = {c: [] for c in contig_ids}
+    for chrom, s, e in _bed_rows(primer_fn):
+        if chrom not in out:
+            raise InputError("%s: %s" % (ERROR_TEXT_BED_CHROM_NOT_IN_FASTA, chrom))
+        out[chrom].append((s, e))
+    for v in out.values():
+        v.sort()
+    return out
 
 
 def find_overlapping_primers(ref_genome_length, primers, primer_pos_offset):

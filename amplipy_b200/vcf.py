@@ -25,12 +25,13 @@ def check_output_path(path):
         raise InputError("%s: %s" % (ERROR_TEXT_INVALID_VCF_EXTENSION, path))
 
 
-def header_text(ref_genome_id, version, argv):
+def header_text(contigs, version, argv):
+    """``contigs``: the reference's ID, or a list of contig IDs (one ##contig line each, in that order)."""
+    ids = [contigs] if isinstance(contigs, str) else list(contigs)
     lines = ["##fileformat=VCFv4.2",
              '##FILTER=<ID=PASS,Description="All filters passed">',
              "##AmpliPyVersion=%s" % version,
-             "##source=%s" % " ".join(argv),
-             "##contig=<ID=%s>" % ref_genome_id,
+             "##source=%s" % " ".join(argv)] + ["##contig=<ID=%s>" % c for c in ids] + [
              '##FORMAT=<ID=GT,Number=1,Type=String,Description="Genotype">',
              '##INFO=<ID=DP,Number=1,Type=Integer,Description="Total Depth">',
              '##INFO=<ID=REF_DP,Number=1,Type=Integer,Description="Depth of reference base">',
@@ -60,8 +61,12 @@ def record_line(ref_genome_id, rec):
     return "\t".join([ref_genome_id, str(pos0 + 1), ".", ref, ",".join(alts), ".", "PASS", info, "GT", "/".join(map(str, gt))])
 
 
-def write_vcf(path, ref_genome_id, version, argv, records):
-    text = header_text(ref_genome_id, version, argv) + "".join(record_line(ref_genome_id, r) + "\n" for r in records)
+def write_vcf(path, contigs, version, argv, records):
+    """``contigs`` = the reference's ID and ``records`` its records, or a list of contig IDs and one list of records per contig
+    (written contig by contig, CHROM = the contig's ID)."""
+    if isinstance(contigs, str):
+        contigs, records = [contigs], [records]
+    text = header_text(contigs, version, argv) + "".join(record_line(c, r) + "\n" for c, recs in zip(contigs, records) for r in recs)
     if path.lower() == "stdout":
         sys.stdout.write(text)
     elif path.lower().endswith(".gz"):

@@ -255,6 +255,37 @@ int amp_set_scheme(amp_ctx* ctx, int sample, int32_t ref_len, const int32_t* pri
 int amp_get_scheme(amp_ctx* ctx, int sample, int32_t* min_primer_start, int32_t* max_primer_end, int32_t* max_primer_len);
 int amp_set_sample_reference(amp_ctx* ctx, int sample, const char* ref_seq, int32_t len);
 
+/* ---- multi-contig references (DESIGN.md 3.8): contig k of the FASTA is sample k of the context, with its own scheme
+ * (amp_set_scheme with ref_len = the contig's length; n_primers may be 0) and reference (amp_set_sample_reference).
+ * A plan call finds every read's contig -- the BAM record's refID through ref_to_sample (-1: no contig, -2: a header sequence
+ * that is not in the FASTA) for the decoded batch, or a per-read sample id in [-1, n_samples) for a device batch -- and
+ * returns per-contig totals.  A read without a contig must carry flag 4; it is trimmed as the fused kernels trim a read that
+ * AmpliPy.py:902 skips and is not piled up.  The context holds at most AMP_MAX_CONTIGS = 1024 samples for this
+ * (AMP_ERR_ARG beyond).  amp_process_contigs then runs the fused kernel (and, with AMP_MODE_QSTATS, the strand / quality pass)
+ * once per contig with reads, over that contig's reads in input order: directly on the batch when it is grouped (every
+ * contig's reads contiguous, as in any coordinate-sorted BAM), else on a copy reordered by a stable counting sort, whose trim
+ * outputs are written back to input order.  Trim outputs: the decoded batch keeps them in the context (dev_out = NULL;
+ * amp_decoded_write_bam reads them), a device batch writes them to dev_out; host_out (may be NULL) receives a copy.
+ * amp_process_contigs returns AMP_ERR_DATA when the plan has error bits, and runs on the batch planned last. */
+#define AMP_CONTIG_E_NOFLAG4 1     /* a read without a contig is not flagged unmapped (flag 4) */
+#define AMP_CONTIG_E_UNKNOWN 2     /* a read on a header sequence that is not in the FASTA (ref_reads says which) */
+#define AMP_CONTIG_E_BADID 4       /* refID outside the header, or a sample id outside [-1, n_samples) */
+typedef struct {
+    int64_t n_reads;            /* out: reads in the batch */
+    int64_t n_no_contig;        /* out: reads without a contig */
+    int32_t grouped;            /* out: 1 = every contig's reads are contiguous */
+    uint32_t errors;            /* out: AMP_CONTIG_E_* */
+    int64_t* contig_reads;      /* [n_samples] out (caller-owned; any of these may be NULL): reads of contig k */
+    int64_t* contig_first;      /*   index of its first read */
+    int64_t* contig_cigar_ops;  /*   CIGAR ops of its reads */
+    int64_t* contig_qual_bytes; /*   quality bytes of its reads */
+    int64_t* ref_reads;         /* [n_refs] out, decoded plan only: reads on header sequence r when ref_to_sample[r] = -2 */
+} amp_contig_plan;
+int amp_contig_plan_decoded(amp_ctx* ctx, const int32_t* ref_to_sample, int32_t n_refs, amp_contig_plan* plan);
+int amp_contig_plan_device(amp_ctx* ctx, const amp_batch* dev_batch /* first = 0 */, const int32_t* dev_sample_of_read,
+                           amp_contig_plan* plan);
+int amp_process_contigs(amp_ctx* ctx, int mode, const amp_trim_out* dev_out, const amp_trim_out* host_out);
+
 /* pinned host memory helpers for callers that want full-speed amp_process_host */
 int amp_host_alloc(void** p, int64_t bytes);
 int amp_host_free(void* p);
