@@ -8,7 +8,7 @@ import os
 import sys
 from datetime import datetime
 
-from . import alnio, calling, ivar, vcf
+from . import alnio, calling, gff, ivar, vcf
 from .primers import InputError, find_overlapping_primers, load_primers, load_primers_by_contig, max_primer_len
 
 VERSION = "0.0.2"
@@ -63,6 +63,9 @@ ERROR_TEXT_LENGTH_MISMATCH = "Sequence length in the alignment header differs fr
 ERROR_TEXT_UNKNOWN_CONTIG = "Reads on a sequence that is not in the reference FASTA"
 ERROR_TEXT_UNMAPPED_NO_FLAG = "Read without a reference sequence is not flagged unmapped (flag 4)"
 ERROR_TEXT_BAD_REFID = "Read reference ID outside the alignment header"
+HELP_TEXT_GFF = ("GFF3 file whose CDS features fill the GFF_FEATURE / codon / amino-acid columns of the TSV (optional; needs "
+                 "--output_tsv)")
+ERROR_TEXT_GFF_NEEDS_TSV = "--gff needs --output_tsv"
 HELP_TEXT_IUPAC_THRESHOLD = ("Write IUPAC ambiguity codes: the shortest prefix of the sorted alleles whose frequencies reach this "
                              "threshold (0-1) is coded (optional; 0 = the plain consensus)")
 
@@ -106,6 +109,7 @@ def parse_args(argv=None):
     v.add_argument('-mf', '--min_freq', required=False, type=float, default=DEFAULT_MIN_FREQ_VARIANTS, help=HELP_TEXT_MIN_FREQ_VARIANTS)
     v.add_argument('-md', '--min_depth', required=False, type=int, default=DEFAULT_MIN_DEPTH_VARIANTS, help=HELP_TEXT_MIN_DEPTH_VARIANTS)
     v.add_argument('--output_tsv', required=False, type=str, default=None, help=HELP_TEXT_TSV)
+    v.add_argument('--gff', required=False, type=str, default=None, help=HELP_TEXT_GFF)
 
     c = sub.add_parser("consensus", description=DESCRIPTION, formatter_class=F)
     c.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_TRIMMED)
@@ -137,6 +141,7 @@ def parse_args(argv=None):
     a.add_argument('-n', '--unknown_symbol', required=False, type=str, default=DEFAULT_UNKNOWN_SYMBOL, help=HELP_TEXT_UNKNOWN_SYMBOL)
     a.add_argument('-e', '--include_no_primer', action='store_true', help=HELP_TEXT_TRIM_INCLUDE_READS_NO_PRIMER)
     a.add_argument('--output_tsv', required=False, type=str, default=None, help=HELP_TEXT_TSV)
+    a.add_argument('--gff', required=False, type=str, default=None, help=HELP_TEXT_GFF)
     a.add_argument('--iupac_threshold', required=False, type=float, default=None, help=HELP_TEXT_IUPAC_THRESHOLD)
     return parser.parse_args(argv)
 
@@ -249,17 +254,19 @@ def run_amplipy(untrimmed_reads_fn=None, primer_fn=None, reference_fn=None, trim
                 consensus_fn=None, primer_pos_offset=None, min_length=None, min_quality=None, sliding_window_width=None,
                 min_freq_consensus=None, min_freq_variants=None, min_depth_consensus=None, min_depth_variants=None,
                 unknown_symbol=None, include_no_primer=None, run_trim=False, run_variants=False, run_consensus=False,
-                argv=None, device=0, tsv_fn=None, iupac_threshold=None, multi_contig=False):
+                argv=None, device=0, tsv_fn=None, iupac_threshold=None, multi_contig=False, gff_fn=None):
     """Same keyword arguments and behaviour as the reference's run_amplipy (AmpliPy.py:774-963).  Additions of this
     project: ``tsv_fn`` (with run_variants) also writes the variants in iVar's TSV format, ``iupac_threshold`` (with
     run_consensus) writes IUPAC ambiguity codes into the consensus (DESIGN.md 3.7), ``multi_contig`` takes every record of the
-    reference FASTA as a contig (DESIGN.md 3.8)."""
+    reference FASTA as a contig (DESIGN.md 3.8), ``gff_fn`` (with ``tsv_fn``) fills the TSV's codon columns from the CDS
+    features of a GFF3 file (DESIGN.md 3.9)."""
     argv = list(sys.argv if argv is None else argv)
     try:
         return _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
                     min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
                     min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
-                    tsv_fn if run_variants else None, iupac_threshold if run_consensus else None, multi_contig)
+                    tsv_fn if run_variants else None, iupac_threshold if run_consensus else None, multi_contig,
+                    gff_fn if run_variants else None)
     except InputError as e:
         error(str(e))
 
@@ -267,7 +274,7 @@ def run_amplipy(untrimmed_reads_fn=None, primer_fn=None, reference_fn=None, trim
 def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
          min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
          unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn=None, iupac_threshold=None,
-         multi_contig=False):
+         multi_contig=False, gff_fn=None):
     # validity checks (AmpliPy.py:837-854)
     if primer_pos_offset is not None and primer_pos_offset < 0:
         error("%s: %s" % (ERROR_TEXT_NEGATIVE_PRIMER_POS_OFFSET, primer_pos_offset))
@@ -289,6 +296,8 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         error("%s: %s" % (ERROR_TEXT_INVALID_UNKNOWN_SYMBOL_LENGTH, unknown_symbol))
     if iupac_threshold is not None and not (0 <= iupac_threshold <= 1):
         error("%s: %s" % (ivar.ERROR_TEXT_INVALID_IUPAC_THRESHOLD, iupac_threshold))
+    if gff_fn is not None and tsv_fn is None:
+        error(ERROR_TEXT_GFF_NEEDS_TSV)
 
     # mode banner (AmpliPy.py:857-866)
     if not (run_trim or run_variants or run_consensus):
@@ -307,7 +316,7 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         return _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
                             min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
                             min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
-                            tsv_fn, iupac_threshold)
+                            tsv_fn, iupac_threshold, gff_fn)
     ref_id, ref_seq = load_ref_genome(reference_fn)
     L = len(ref_seq)
     tables, mpl = None, 0
@@ -330,6 +339,10 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
     if tsv_fn is not None:
         print_log("Output variants TSV: %s" % tsv_fn)
         ivar.check_output_path(tsv_fn)
+    features = None
+    if gff_fn is not None:
+        print_log("Loading GFF: %s" % gff_fn)
+        features = gff.features_by_contig(gff.load_gff(gff_fn), [(ref_id, ref_seq)], False)[0]
     import threading
     import time as _time
     tm = {}
@@ -445,7 +458,11 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         if tsv_fn is not None:
             iv = eng.call_ivar(DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
                                DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants)
-            ivar.write_tsv(tsv_fn, ivar.tsv_rows(res, ins, iv, eng.qstats(0), ref_id, ref_seq, counts))
+            ann = names = None
+            if features is not None:
+                eng.set_features(0, features)     # after call: the context holds the reference now
+                ann, names = eng.annotate(), [f.name for f in features]
+            ivar.write_tsv(tsv_fn, ivar.tsv_rows(res, ins, iv, eng.qstats(0), ref_id, ref_seq, counts, ann=ann, names=names))
         iupac = None
         if iupac_threshold is not None:
             iupac = eng.call_ivar(DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
@@ -476,7 +493,7 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
 
 def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
                  min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
-                 unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn, iupac_threshold):
+                 unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn, iupac_threshold, gff_fn=None):
     """_run with --multi_contig (DESIGN.md 3.8): contig k of the FASTA is sample k of one context, with the BED rows of its chrom as
     its scheme and its own length; reads go to the contig their reference names.  Outputs follow the FASTA's record order."""
     contigs = load_ref_genomes(reference_fn)
@@ -499,6 +516,10 @@ def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, 
     if tsv_fn is not None:
         print_log("Output variants TSV: %s" % tsv_fn)
         ivar.check_output_path(tsv_fn)
+    features = None
+    if gff_fn is not None:
+        print_log("Loading GFF: %s" % gff_fn)
+        features = gff.features_by_contig(gff.load_gff(gff_fn), contigs, True)
     from .engine import AmpError, ContigError, Engine, TrimResult
     qstats = tsv_fn is not None
     pile = run_variants or run_consensus
@@ -580,8 +601,14 @@ def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, 
         if tsv_fn is not None:
             iv = eng.call_ivar(DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
                                DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants)
+            ann = None
+            if features is not None:
+                for k, fk in enumerate(features):
+                    eng.set_features(k, fk)
+                ann = eng.annotate()
             ivar.write_tsv(tsv_fn, [r for k, (cid, seq) in enumerate(contigs)
-                                    for r in ivar.tsv_rows(res, ins, iv, eng.qstats(k), cid, seq, counts[k], k, L=len(seq))])
+                                    for r in ivar.tsv_rows(res, ins, iv, eng.qstats(k), cid, seq, counts[k], k, L=len(seq), ann=ann,
+                                                           names=[f.name for f in features[k]] if features is not None else None)])
         iupac = None
         if iupac_threshold is not None:
             iupac = eng.call_ivar(DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
@@ -614,7 +641,7 @@ def main(argv=None):
     elif args.command == 'variants':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, variants_fn=args.output,
                     min_quality=args.min_quality, min_freq_variants=args.min_freq, min_depth_variants=args.min_depth,
-                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv, multi_contig=args.multi_contig)
+                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv, multi_contig=args.multi_contig, gff_fn=args.gff)
     elif args.command == 'consensus':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, consensus_fn=args.output,
                     min_quality=args.min_quality, min_freq_consensus=args.min_freq, min_depth_consensus=args.min_depth,
@@ -629,7 +656,7 @@ def main(argv=None):
                     min_depth_consensus=args.min_depth_consensus, min_depth_variants=args.min_depth_variants,
                     unknown_symbol=args.unknown_symbol, include_no_primer=args.include_no_primer, run_trim=True,
                     run_variants=True, run_consensus=True, argv=full_argv, tsv_fn=args.output_tsv,
-                    iupac_threshold=args.iupac_threshold, multi_contig=args.multi_contig)
+                    iupac_threshold=args.iupac_threshold, multi_contig=args.multi_contig, gff_fn=args.gff)
 
 
 if __name__ == "__main__":

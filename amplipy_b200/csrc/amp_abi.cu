@@ -17,6 +17,7 @@
 #include "amp_deflate.cuh"
 #include "amp_ivar.cuh"
 #include "amp_contig.cuh"
+#include "amp_annot.cuh"
 
 static_assert(AMP_F_TRIM_START == AMP_FLAG_TRIM_START && AMP_F_KEEP == AMP_FLAG_KEEP && AMP_F_SKIPPED == AMP_FLAG_SKIPPED &&
                   AMP_F_ERROR == AMP_FLAG_ERROR && AMP_E_ARENA_FULL == AMP_DEVERR_ARENA_FULL &&
@@ -409,6 +410,36 @@ __global__ void __launch_bounds__(256) amp_contig_skip_kernel(const __grid_const
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < P.n; i += (long long)gridDim.x * blockDim.x) amp::contig_skip_read(P, i);
 }
 
+// ---- codon annotation (amp_annot.cuh): counts and per-tile sums, a scan of the tile sums (amp_contig_scan_kernel), then the
+// offsets and the entries ----------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(AMP_AN_THREADS) amp_annot_count_kernel(const __grid_constant__ amp::AnnotParams P, uint32_t* tsum) {
+    __shared__ unsigned int s;
+    if (threadIdx.x == 0) s = 0;
+    __syncthreads();
+    const long long gp = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (gp < (long long)P.n_samples * P.L) {
+        const unsigned int n = amp::annot_count(P, gp);
+        P.off[gp] = n;
+        if (n) atomicAdd(&s, n);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) tsum[blockIdx.x] = s;
+}
+__global__ void __launch_bounds__(AMP_AN_THREADS) amp_annot_fill_kernel(const __grid_constant__ amp::AnnotParams P, const uint32_t* tbase,
+                                                                        unsigned int n_tiles) {
+    __shared__ unsigned long long part[AMP_AN_THREADS];
+    const long long SL = (long long)P.n_samples * P.L;
+    const long long gp = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    const unsigned int n = gp < SL ? P.off[gp] : 0u;
+    unsigned long long total;
+    const unsigned int o = tbase[blockIdx.x] + (unsigned int)amp::cta_excl_scan(n, part, &total);
+    if (gp < SL) {
+        P.off[gp] = o;
+        if (n) amp::annot_fill(P, gp, o);
+    }
+    if (gp == 0) P.off[SL] = tbase[n_tiles];
+}
+
 struct DevChunk {   // device staging for one in-flight chunk of amp_process_host
     cudaStream_t stream = nullptr;
     int32_t* pos = nullptr; uint16_t* flag = nullptr; int32_t* tlen = nullptr;
@@ -488,6 +519,14 @@ struct amp_ctx {
         int32_t* o_pos = nullptr; size_t cap_opos = 0; uint16_t* o_ncig = nullptr; size_t cap_oncig = 0; uint8_t* o_flags = nullptr; size_t cap_oflags = 0;
         uint32_t* o_cigar = nullptr; size_t cap_ocig = 0; uint32_t* scratch = nullptr; size_t cap_scratch = 0;
     } ct;
+    std::vector<int> ref_len_s;         // per-sample reference lengths (amp_set_sample_reference)
+    // codon annotation (amp_set_features / amp_annotate; buffers grown at high-water marks)
+    struct Annot {
+        std::vector<amp::AnnotFeatures> feat; bool built = false; long long n = 0;
+        int* tables = nullptr; size_t cap_tables = 0; uint32_t* off = nullptr; size_t cap_off = 0;
+        uint32_t* tsum = nullptr; size_t cap_tsum = 0; uint32_t* tbase = nullptr; size_t cap_tbase = 0;
+        int* e_int = nullptr; size_t cap_eint = 0; unsigned char* e_chr = nullptr; size_t cap_echr = 0;   // feat, pos_aa | off, codons, aas
+    } an;
 };
 
 namespace {
@@ -739,6 +778,7 @@ int amp_destroy(amp_ctx* c) {
                       t.seq, t.qual, t.o_pos, t.o_ncig, t.o_flags, t.o_cigar, t.scratch};
         for (void* q : ps) cudaFree(q);
     }
+    cudaFree(c->an.tables); cudaFree(c->an.off); cudaFree(c->an.tsum); cudaFree(c->an.tbase); cudaFree(c->an.e_int); cudaFree(c->an.e_chr);
     for (auto& ch : c->chunk) {
         cudaFree(ch.pos); cudaFree(ch.flag); cudaFree(ch.tlen); cudaFree(ch.cig_off); cudaFree(ch.seq_off); cudaFree(ch.qual_off);
         cudaFree(ch.cigar); cudaFree(ch.seq); cudaFree(ch.qual); cudaFree(ch.o_pos); cudaFree(ch.o_ncig); cudaFree(ch.o_flags);
@@ -1024,7 +1064,8 @@ int amp_ins_merge(amp_ctx* c, int64_t n, const int32_t* sample, const int32_t* p
 int amp_set_reference(amp_ctx* c, const char* ref_seq) {
     if (!c || !ref_seq) return fail(AMP_ERR_ARG, "amp_set_reference: null argument");
     CK(cudaSetDevice(c->cfg.device));
-    if (c->ref_per_sample) { CK(cudaFree(c->d_ref)); c->d_ref = nullptr; c->ref_per_sample = false; }
+    if (c->ref_per_sample) { CK(cudaFree(c->d_ref)); c->d_ref = nullptr; c->ref_per_sample = false; c->ref_len_s.clear(); }
+    c->an.built = false;
     if (!c->d_ref) CK(cudaMalloc((void**)&c->d_ref, (size_t)c->cfg.ref_len + 16));
     CK(cudaMemcpy(c->d_ref, ref_seq, (size_t)c->cfg.ref_len, cudaMemcpyHostToDevice));
     return AMP_OK;
@@ -1718,6 +1759,9 @@ int amp_set_sample_reference(amp_ctx* c, int sample, const char* ref_seq, int32_
     }
     CK(cudaMemset(c->d_ref + (size_t)sample * L, 'N', L));
     CK(cudaMemcpy(c->d_ref + (size_t)sample * L, ref_seq, (size_t)len, cudaMemcpyHostToDevice));
+    if (c->ref_len_s.size() != S) c->ref_len_s.assign(S, (int)L);
+    c->ref_len_s[sample] = len;
+    c->an.built = false;
     return AMP_OK;
 }
 
@@ -1954,6 +1998,112 @@ int amp_process_contigs(amp_ctx* c, int mode, const amp_trim_out* dev_out, const
         if (host_out->cigar) CK(cudaMemcpyAsync(host_out->cigar, out.cigar, orows * 4, cudaMemcpyDeviceToHost, sc));
     }
     CK(cudaStreamSynchronize(sc));
+    return AMP_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------
+// codon annotation of the iVar TSV (amp_annot.cuh, DESIGN.md 3.9)
+// ---------------------------------------------------------------------------------------------------
+namespace {
+int sample_ref_len(const amp_ctx* c, int sample) {
+    return c->ref_per_sample && (size_t)sample < c->ref_len_s.size() ? c->ref_len_s[sample] : c->cfg.ref_len;
+}
+}  // namespace
+
+extern "C" {
+
+int amp_set_features(amp_ctx* c, int sample, int32_t n_features, const int32_t* strand, const int32_t* phase, const int32_t* seg_off,
+                     const int32_t* seg_start, const int32_t* seg_end) {
+    if (!c || sample < 0 || sample >= c->cfg.n_samples) return fail(AMP_ERR_ARG, "amp_set_features: bad sample");
+    if (!c->d_ref) return fail(AMP_ERR_STATE, "amp_set_features: no reference (amp_set_reference / amp_set_sample_reference first)");
+    amp::AnnotFeatures f;
+    if (!amp::annot_features(sample_ref_len(c, sample), n_features, strand, phase, seg_off, seg_start, seg_end, f))
+        return fail(AMP_ERR_ARG, "amp_set_features: bad feature (strand +1 / -1, phase 0..2, at least one segment, 0 <= start < end <= the sample's length)");
+    if (c->an.feat.size() < (size_t)c->cfg.n_samples) c->an.feat.resize((size_t)c->cfg.n_samples);
+    c->an.feat[sample] = std::move(f);
+    c->an.built = false;
+    return AMP_OK;
+}
+
+int amp_annotate(amp_ctx* c, int64_t* n_entries) {
+    if (!c) return fail(AMP_ERR_ARG, "amp_annotate: null context");
+    auto& a = c->an;
+    bool any = false;
+    for (size_t s = 0; s < a.feat.size(); ++s) {
+        any |= !a.feat[s].lo.empty();
+        for (int e : a.feat[s].hi)
+            if (e > sample_ref_len(c, (int)s)) return fail(AMP_ERR_ARG, "amp_annotate: a segment ends past its sample's reference");
+    }
+    if (!any) return fail(AMP_ERR_STATE, "amp_annotate: no features (amp_set_features first)");
+    if (!c->d_ref) return fail(AMP_ERR_STATE, "amp_annotate: no reference");
+    CK(cudaSetDevice(c->cfg.device));
+    a.built = false;
+    const int S = c->cfg.n_samples, L = c->cfg.ref_len;
+    const long long SL = (long long)S * L, n_tiles = (SL + AMP_AN_THREADS - 1) / AMP_AN_THREADS;
+    std::vector<amp::AnnotFeatures> all(a.feat);
+    all.resize((size_t)S);
+    amp::AnnotTables T;
+    amp::annot_tables(all, T);
+    const std::vector<int>* parts[] = {&T.samp_seg, &T.sg_lo, &T.sg_max, &T.sg_key, &T.fs_lo, &T.fs_hi, &T.fs_cum, &T.fs_feat, &T.ft_fs,
+                                       &T.ft_len, &T.ft_local, &T.ft_info};
+    size_t words = 0;
+    for (auto* v : parts) words += v->size();
+    std::vector<int> packed;
+    packed.reserve(words);
+    for (auto* v : parts) packed.insert(packed.end(), v->begin(), v->end());
+    int rc;
+    if ((rc = dev_grow(&a.tables, &a.cap_tables, words)) || (rc = dev_grow(&a.off, &a.cap_off, (size_t)SL + 1)) ||
+        (rc = dev_grow(&a.tsum, &a.cap_tsum, (size_t)n_tiles)) || (rc = dev_grow(&a.tbase, &a.cap_tbase, (size_t)n_tiles + 1)))
+        return rc;
+    cudaStream_t st = c->chunk[0].stream;
+    CK(cudaDeviceSynchronize());
+    CK(cudaMemcpyAsync(a.tables, packed.data(), words * 4, cudaMemcpyHostToDevice, st));
+    amp::AnnotParams P{};
+    P.L = L; P.n_samples = S; P.ref = c->d_ref; P.ref_stride = c->ref_per_sample ? (long long)L : 0;
+    const int** dst[] = {&P.samp_seg, &P.sg_lo, &P.sg_max, &P.sg_key, &P.fs_lo, &P.fs_hi, &P.fs_cum, &P.fs_feat, &P.ft_fs, &P.ft_len,
+                         &P.ft_local, &P.ft_info};
+    size_t o = 0;
+    for (int k = 0; k < 12; ++k) { *dst[k] = a.tables + o; o += parts[k]->size(); }
+    P.off = a.off;
+    amp_annot_count_kernel<<<(unsigned)n_tiles, AMP_AN_THREADS, 0, st>>>(P, a.tsum);
+    CK(cudaGetLastError());
+    amp::ContigScanParams H{a.tsum, n_tiles, n_tiles, 1, 0, a.tbase};
+    amp_contig_scan_kernel<<<dim3(1, 1), AMP_CT_THREADS, 0, st>>>(H, H, H);
+    CK(cudaGetLastError());
+    uint32_t total = 0;
+    CK(cudaMemcpyAsync(&total, a.tbase + n_tiles, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const size_t E = total;
+    if ((rc = dev_grow(&a.e_int, &a.cap_eint, 2 * E + 1)) || (rc = dev_grow(&a.e_chr, &a.cap_echr, 25 * E + 1))) return rc;
+    P.e_feat = a.e_int; P.e_pos_aa = a.e_int + E;
+    P.e_off = a.e_chr; P.e_codon = a.e_chr + E; P.e_aa = a.e_chr + 19 * E;
+    amp_annot_fill_kernel<<<(unsigned)n_tiles, AMP_AN_THREADS, 0, st>>>(P, a.tbase, (unsigned)n_tiles);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    c->last_launches = 3;
+    a.n = (long long)E; a.built = true;
+    if (n_entries) *n_entries = a.n;
+    return AMP_OK;
+}
+
+int amp_annot_host(amp_ctx* c, uint32_t* off, int32_t* feat, int32_t* pos_aa, uint8_t* codon_off, char* codons, char* aas) {
+    if (!c) return fail(AMP_ERR_ARG, "amp_annot_host: null context");
+    if (!c->an.built) return fail(AMP_ERR_STATE, "amp_annot_host: no annotation (amp_annotate first, after the last change of features or reference)");
+    CK(cudaSetDevice(c->cfg.device));
+    auto& a = c->an;
+    const size_t SL = (size_t)c->cfg.n_samples * c->cfg.ref_len, E = (size_t)a.n;
+    cudaStream_t st = c->chunk[0].stream;
+    if (off) CK(cudaMemcpyAsync(off, a.off, (SL + 1) * 4, cudaMemcpyDeviceToHost, st));
+    if (E) {
+        if (feat) CK(cudaMemcpyAsync(feat, a.e_int, E * 4, cudaMemcpyDeviceToHost, st));
+        if (pos_aa) CK(cudaMemcpyAsync(pos_aa, a.e_int + E, E * 4, cudaMemcpyDeviceToHost, st));
+        if (codon_off) CK(cudaMemcpyAsync(codon_off, a.e_chr, E, cudaMemcpyDeviceToHost, st));
+        if (codons) CK(cudaMemcpyAsync(codons, a.e_chr + E, E * 18, cudaMemcpyDeviceToHost, st));
+        if (aas) CK(cudaMemcpyAsync(aas, a.e_chr + 19 * E, E * 6, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
     return AMP_OK;
 }
 

@@ -18,7 +18,7 @@ import numpy as np
 
 from .batch import ReadBatch
 from .calling import CallResult, Insertions
-from .ivar import IvarResult, QStats
+from .ivar import Annotation, IvarResult, QStats
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AMP_LIB_OVERRIDE") or os.path.join(_HERE, "csrc", "libamplipy_b200.so")   # override: tuning experiments only
@@ -42,7 +42,8 @@ EXPORTED_SYMBOLS = [
     "amp_ins_slot_bytes", "amp_ins_pack_device", "amp_ins_merge_packed", "amp_reserve", "amp_counts_copy_device",
     "amp_bam_decode_host", "amp_process_decoded", "amp_decoded_copy_host", "amp_counts_upload", "amp_bgzf_deflate_host", "amp_decoded_write_bam",
     "amp_set_scheme", "amp_get_scheme", "amp_set_sample_reference", "amp_qstats_enable", "amp_qstats_host", "amp_call_ivar",
-    "amp_call_ivar_device", "amp_contig_plan_decoded", "amp_contig_plan_device", "amp_process_contigs"]
+    "amp_call_ivar_device", "amp_contig_plan_decoded", "amp_contig_plan_device", "amp_process_contigs", "amp_set_features",
+    "amp_annotate", "amp_annot_host"]
 
 
 class AmpConfig(ctypes.Structure):
@@ -635,6 +636,33 @@ class Engine:
         _check(self.lib.amp_call_ivar_device(self._ctx, ctypes.byref(p), ctypes.c_void_p(stream) if stream else None),
                "amp_call_ivar_device")
         self.launches += int(self.lib.amp_last_launches(self._ctx))
+
+    # ---------------------------------------------------------------- codon annotation of the iVar TSV (DESIGN.md 3.9)
+    def set_features(self, sample, features):
+        """The CDS features of one sample (gff.Feature: strand, phase, segments); checked against the sample's reference, which
+        has to be set first (set_reference / set_sample_reference / call).  An empty list clears the sample."""
+        strand = np.ascontiguousarray([f.strand for f in features], np.int32)
+        phase = np.ascontiguousarray([f.phase for f in features], np.int32)
+        seg_off = np.zeros(len(features) + 1, np.int32)
+        np.cumsum([len(f.segments) for f in features], out=seg_off[1:])
+        start = np.ascontiguousarray([s for f in features for s, _ in f.segments], np.int32)
+        end = np.ascontiguousarray([e for f in features for _, e in f.segments], np.int32)
+        _check(self.lib.amp_set_features(self._ctx, int(sample), len(features), _ptr(strand), _ptr(phase), _ptr(seg_off), _ptr(start),
+                                         _ptr(end)), "amp_set_features")
+
+    def annotate(self):
+        """The occurrences of every (sample, position) in the features of set_features, built and translated on the device
+        (amp_annotate + amp_annot_host).  Returns an ivar.Annotation."""
+        n = ctypes.c_int64(0)
+        _check(self.lib.amp_annotate(self._ctx, ctypes.byref(n)), "amp_annotate")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        E = int(n.value)
+        a = Annotation(self.L, np.empty(self.n_samples * self.L + 1, np.uint32), np.empty(max(E, 1), np.int32), np.empty(max(E, 1), np.int32),
+                       np.empty(max(E, 1), np.uint8), np.empty((max(E, 1), 18), np.uint8), np.empty((max(E, 1), 6), np.uint8))
+        _check(self.lib.amp_annot_host(self._ctx, _ptr(a.off), _ptr(a.feat), _ptr(a.pos_aa), _ptr(a.codon_off), _ptr(a.codons), _ptr(a.aas)),
+               "amp_annot_host")
+        a.feat, a.pos_aa, a.codon_off, a.codons, a.aas = a.feat[:E], a.pos_aa[:E], a.codon_off[:E], a.codons[:E], a.aas[:E]
+        return a
 
     def _call_buffers(self, n_ins, pinned):
         """Result arrays of ``call``: fresh numpy arrays, or (``pinned``) page-locked arrays owned by the engine and reused."""

@@ -40,6 +40,31 @@ class IvarResult:
     ins_pval: np.ndarray    # f64[K]
 
 
+@dataclass
+class Annotation:
+    """``amp_annotate`` outputs (DESIGN.md 3.9): the occurrences of (sample, position) gp = sample * L + p, each a (feature, codon)
+    pair the position belongs to, are entries [off[gp], off[gp + 1]), in feature order, then in spliced order."""
+    L: int
+    off: np.ndarray         # u32[S*L + 1]
+    feat: np.ndarray        # i32[E] index of the feature in its sample's list
+    pos_aa: np.ndarray      # i32[E] 1-based codon index
+    codon_off: np.ndarray   # u8[E] offset of the position in the codon
+    codons: np.ndarray      # u8[E, 18] REF_CODON, then ALT_CODON for A C G T N at that offset
+    aas: np.ndarray         # u8[E, 6] REF_AA, then ALT_AA for A C G T N
+
+    def columns(self, sample, p, alt, names):
+        """The six annotation columns of a TSV row at position p with ALT ``alt``, one tuple per occurrence; ALT_CODON / ALT_AA
+        are NA for '-' and '+' rows."""
+        gp = sample * self.L + p
+        out = []
+        for e in range(int(self.off[gp]), int(self.off[gp + 1])):
+            c, a = self.codons[e].tobytes().decode("latin-1"), self.aas[e].tobytes().decode("latin-1")
+            k = "ACGTN".find(alt) if len(alt) == 1 else -1
+            out.append((names[int(self.feat[e])], c[:3], a[0], c[3 + 3 * k:6 + 3 * k] if k >= 0 else "NA", a[1 + k] if k >= 0 else "NA",
+                        int(self.pos_aa[e])))
+        return out
+
+
 def check_output_path(path):
     """The TSV refuses to overwrite, like the other outputs."""
     if path.lower() != "stdout" and os.path.isfile(path):
@@ -61,10 +86,12 @@ def alt_text(sym, ref_char, head=False):
     return "+" + (sym[:-1] if head else sym[1:])
 
 
-def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None):
+def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None, ann=None, names=None):
     """The TSV rows of one sample: every allele with a p-value (count > 0, symbol != the FASTA character, freq >= min_freq, depth
     >= min_depth), in position order, then in the reference's allele order (AmpliPy.py:771).  ``L``: the sample's own reference
-    length when it is shorter than the context's (a contig of a multi-record FASTA)."""
+    length when it is shorter than the context's (a contig of a multi-record FASTA).  ``ann`` (an Annotation) and ``names`` (the
+    sample's feature names): a row at a position with k >= 1 occurrences is written k times in a row, once per occurrence, with
+    the six annotation columns appended."""
     L = res.L if L is None else L
     base = sample * res.L
     fpv = iv.fixed_pval[base:base + L]
@@ -93,14 +120,18 @@ def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None):
                          int(qs.ins_rev[k]), int(iv.ins_mq[k]), float(iv.ins_pval[k])))
         alts.sort(key=lambda a: a[0])
         for _, alt, c, rv, mq, pv in alts:
-            out.append((ref_id, p + 1, ref_char, alt, ref_dp, ref_rv, ref_q, c, rv, mq, c / D, D, pv, pv <= PASS_PVAL))
+            row = (ref_id, p + 1, ref_char, alt, ref_dp, ref_rv, ref_q, c, rv, mq, c / D, D, pv, pv <= PASS_PVAL)
+            cols = ann.columns(sample, p, alt, names) if ann is not None else ()
+            out.extend([row + a for a in cols] if cols else [row])
     return out
 
 
 def format_row(r):
-    ref_id, pos, ref, alt, ref_dp, ref_rv, ref_q, c, rv, mq, freq, D, pv, ok = r
+    """A row of tsv_rows: 14 fields, and the six annotation columns when it has them (else NA)."""
+    ref_id, pos, ref, alt, ref_dp, ref_rv, ref_q, c, rv, mq, freq, D, pv, ok = r[:14]
+    ann = [str(x) for x in r[14:]] if len(r) > 14 else ["NA"] * 6
     return "\t".join([ref_id, str(pos), ref, alt, str(ref_dp), str(ref_rv), str(ref_q), str(c), str(rv), str(mq), repr(freq), str(D),
-                      repr(pv), "TRUE" if ok else "FALSE"] + ["NA"] * 6)
+                      repr(pv), "TRUE" if ok else "FALSE"] + ann)
 
 
 def write_tsv(path, rows):

@@ -286,6 +286,24 @@ int amp_contig_plan_device(amp_ctx* ctx, const amp_batch* dev_batch /* first = 0
                            amp_contig_plan* plan);
 int amp_process_contigs(amp_ctx* ctx, int mode, const amp_trim_out* dev_out, const amp_trim_out* host_out);
 
+/* ---- codon annotation of the iVar TSV (DESIGN.md 3.9): the CDS features of a GFF3 file, per sample.
+ * amp_set_features gives sample `sample` its features: feature f has strand[f] (+1 / -1), phase[f] (0..2: bases skipped before
+ * its first codon), and the segments [seg_off[f], seg_off[f + 1]) of seg_start / seg_end (0-based, half-open, in any order: they
+ * are spliced 5' to 3').  Checked against the sample's reference length (amp_set_reference / amp_set_sample_reference first,
+ * else AMP_ERR_STATE); bad input is AMP_ERR_ARG.  n_features = 0 clears the sample.
+ * amp_annotate builds, on the device, the occurrences of every (sample, position): the (feature, codon) pairs it belongs to,
+ * in feature order, then in spliced order, as CSR over S*L positions, with each one's reference codon and amino acid and the
+ * codon and amino acid of every substitution A C G T N at the position (standard code, table 1; '*' stop, 'X' any codon with
+ * a character other than ACGT).  *n_entries = the number of occurrences.  AMP_ERR_STATE without features.
+ * amp_annot_host copies the result: off[S*L + 1] (occurrences of position gp: [off[gp], off[gp + 1])), and per occurrence the
+ * feature's index in its sample, the 1-based codon index, the position's offset in the codon, 18 codon characters (REF, then
+ * ALT for A C G T N) and 6 amino acids (the same order); any pointer may be NULL.  AMP_ERR_STATE unless amp_annotate ran after
+ * the last change of features or reference. */
+int amp_set_features(amp_ctx* ctx, int sample, int32_t n_features, const int32_t* strand, const int32_t* phase, const int32_t* seg_off,
+                     const int32_t* seg_start, const int32_t* seg_end);
+int amp_annotate(amp_ctx* ctx, int64_t* n_entries);
+int amp_annot_host(amp_ctx* ctx, uint32_t* off, int32_t* feat, int32_t* pos_aa, uint8_t* codon_off, char* codons, char* aas);
+
 /* pinned host memory helpers for callers that want full-speed amp_process_host */
 int amp_host_alloc(void** p, int64_t bytes);
 int amp_host_free(void* p);
