@@ -171,7 +171,8 @@ __global__ void amp_merge_kernel(amp::InsTable tab, long long n, const int* gpos
 // slot = { u64 n_alleles, u64 arena_words, {u64 arena word offset, u64 count}[cap_entries], arena bytes [cap_arena] }
 __global__ void amp_ins_pack_kernel(amp::InsTable tab, unsigned long long* slot, unsigned long long cap_entries,
                                     unsigned long long cap_arena_words) {
-    const unsigned long long words = tab.cursor[0], n = tab.cursor[1];
+    // cursor[0] runs past the arena when a reservation failed (AMP_E_ARENA_FULL); no slot names such a record
+    const unsigned long long words = tab.cursor[0] < tab.arena_words ? tab.cursor[0] : tab.arena_words, n = tab.cursor[1];
     const bool fits = n <= cap_entries && words <= cap_arena_words;
     const unsigned long long tid = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x, nth = (unsigned long long)gridDim.x * blockDim.x;
     if (tid == 0) {
@@ -998,7 +999,7 @@ int amp_ins_count(amp_ctx* c, int64_t* n_alleles, int64_t* n_chars) {
     unsigned long long cur[2];
     CK(cudaMemcpy(cur, c->tab.cursor, 16, cudaMemcpyDeviceToHost));
     *n_alleles = (int64_t)cur[1];
-    *n_chars = (int64_t)(cur[0] * 8);   // upper bound (records incl. headers and padding)
+    *n_chars = (int64_t)(std::min(cur[0], c->tab.arena_words) * 8);   // upper bound (records incl. headers and padding)
     return AMP_OK;
 }
 
@@ -1009,6 +1010,8 @@ int amp_ins_export(amp_ctx* c, int32_t* sample, int32_t* pos, int32_t* count, in
     unsigned long long cur[2];
     CK(cudaMemcpy(cur, c->tab.cursor, 16, cudaMemcpyDeviceToHost));
     const unsigned long long n = cur[1];
+    // a failed reservation leaves cursor[0] past the arena (AMP_E_ARENA_FULL); the stored records all lie below arena_words
+    const unsigned long long words = std::min(cur[0], c->tab.arena_words);
     str_off[0] = 0;
     if (n == 0) return AMP_OK;
     {
@@ -1020,10 +1023,10 @@ int amp_ins_export(amp_ctx* c, int32_t* sample, int32_t* pos, int32_t* count, in
     amp_gather_entries_kernel<<<(unsigned)std::min<unsigned long long>((n + 255) / 256, 1184), 256>>>(c->tab.slots, c->tab.entries, n, d_count, d_off);
     CK(cudaGetLastError());
     std::vector<unsigned long long> off(n);
-    std::vector<unsigned char> arena(cur[0] * 8);
+    std::vector<unsigned char> arena(words * 8);
     CK(cudaMemcpy(count, d_count, n * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(off.data(), d_off, n * 8, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(arena.data(), c->tab.arena, cur[0] * 8, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(arena.data(), c->tab.arena, words * 8, cudaMemcpyDeviceToHost));
     int64_t o = 0;
     for (unsigned long long k = 0; k < n; ++k) {
         const unsigned char* rec = arena.data() + off[k] * 8;

@@ -164,6 +164,14 @@ void* emu_create(int L, int n_samples, const int32_t* mn, const int32_t* mx, int
 }
 void emu_destroy(void* h) { delete (EmuCtx*)h; }
 unsigned int emu_error_flags(void* h) { return ((EmuCtx*)h)->err; }
+// as amp_reset_kernel: zero counts, the slots listed in entries[0, cursor[1]), both cursors and the error word; the arena
+// keeps its bytes
+void emu_reset(void* h) {
+    EmuCtx* c = (EmuCtx*)h;
+    std::fill(c->counts.begin(), c->counts.end(), 0);
+    for (unsigned long long k = 0; k < c->cursor[1]; ++k) c->slots[c->entries[k]] = amp::InsSlot{0, 0, 0};
+    c->cursor[0] = c->cursor[1] = 0; c->err = 0;
+}
 
 // grid / threads / reads_per_tile overrides (0 = what the product's launch code would choose)
 int emu_process(void* h, long long first, long long n, const int32_t* pos, const uint16_t* flag, const int32_t* tlen,
@@ -305,7 +313,10 @@ void emu_counts(void* h, int sample, int32_t* out) {
 int* emu_counts_ptr(void* h) { return ((EmuCtx*)h)->counts.data(); }
 int emu_lpad(void* h) { return ((EmuCtx*)h)->Lpad; }
 long long emu_ins_count(void* h) { return (long long)((EmuCtx*)h)->cursor[1]; }
-long long emu_ins_chars(void* h) { return (long long)((EmuCtx*)h)->cursor[0] * 8; }
+long long emu_ins_chars(void* h) {   // as amp_ins_count: a failed reservation leaves cursor[0] past the arena
+    EmuCtx* c = (EmuCtx*)h;
+    return (long long)std::min(c->cursor[0], c->tab.arena_words) * 8;
+}
 void emu_ins_export(void* h, int32_t* sample, int32_t* pos, int32_t* count, int64_t* str_off, char* chars) {
     EmuCtx* c = (EmuCtx*)h;
     int64_t o = 0; str_off[0] = 0;
@@ -326,6 +337,13 @@ struct RawText {
         return w;
     }
 };
+// the 64-bit hash ins_table_add computes for the key text[0, len) at gpos (home slot h & mask, tag (h >> 40) | 0x800000)
+unsigned long long emu_ins_hash(int gpos, const char* text, int len) {
+    const RawText t{text};
+    unsigned long long h = amp::ins_hash_init(gpos);
+    for (int i = 0; i < len; i += 4) h = amp::ins_hash_word(h, t.word(i, len));
+    return amp::ins_hash_final(h, len);
+}
 void emu_ins_merge(void* h, long long n, const int32_t* sample, const int32_t* pos, const int32_t* count, const int64_t* str_off,
                    const char* chars) {
     EmuCtx* c = (EmuCtx*)h;

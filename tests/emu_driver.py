@@ -38,7 +38,15 @@ def lib():
         _lib.emu_ins_count.restype = ctypes.c_longlong
         _lib.emu_ins_chars.restype = ctypes.c_longlong
         _lib.emu_error_flags.restype = ctypes.c_uint
+        _lib.emu_ins_hash.restype = ctypes.c_ulonglong
+        _lib.emu_ins_hash.argtypes = [ctypes.c_int, ctypes.c_char_p, ctypes.c_int]
     return _lib
+
+
+def ins_hash(gpos, text):
+    """The 64-bit hash ins_table_add computes for the insertion key ``text`` at ``gpos`` (sample * lpad + pos)."""
+    raw = text.encode("latin-1")
+    return int(lib().emu_ins_hash(int(gpos), raw, len(raw)))
 
 
 def v7_stats(reset=True):
@@ -77,6 +85,9 @@ class EmuEngine:
 
     def error_flags(self):
         return int(lib().emu_error_flags(self._h))
+
+    def reset(self):
+        lib().emu_reset(self._h)
 
     def raise_on_device_errors(self):
         assert self.error_flags() == 0, self.error_flags()
