@@ -18,6 +18,7 @@
 #include "amp_ivar.cuh"
 #include "amp_contig.cuh"
 #include "amp_annot.cuh"
+#include "amp_exchange.cuh"
 
 static_assert(AMP_F_TRIM_START == AMP_FLAG_TRIM_START && AMP_F_KEEP == AMP_FLAG_KEEP && AMP_F_SKIPPED == AMP_FLAG_SKIPPED &&
                   AMP_F_ERROR == AMP_FLAG_ERROR && AMP_E_ARENA_FULL == AMP_DEVERR_ARENA_FULL &&
@@ -189,15 +190,6 @@ __global__ void amp_ins_pack_kernel(amp::InsTable tab, unsigned long long* slot,
     const unsigned long long* src = (const unsigned long long*)tab.arena;
     for (unsigned long long k = tid; k < words; k += nth) dst[k] = src[k];
 }
-struct ArenaText {   // key characters of a packed record
-    const unsigned char* p;
-    __device__ char operator()(int i) const { return (char)p[i]; }
-    __device__ uint32_t word(int i, int len) const {
-        uint32_t w = *(const uint32_t*)(p + i);                 // records are padded to 8 bytes
-        if (len - i < 4) w &= (1u << (8 * (len - i))) - 1u;
-        return w;
-    }
-};
 __global__ void amp_ins_merge_packed_kernel(amp::InsTable tab, const unsigned long long* slots, unsigned long long slot_words,
                                             unsigned long long cap_entries, int my_rank) {
     const int r = (int)blockIdx.y;
@@ -210,9 +202,32 @@ __global__ void amp_ins_merge_packed_kernel(amp::InsTable tab, const unsigned lo
         const unsigned char* rec = arena + ent[2 * k] * 8;
         const int gpos = ((const int*)rec)[0];
         const int len = (int)((const unsigned int*)rec)[1];
-        ArenaText t{rec + 8};
+        amp::ArenaText t{rec + 8};
         amp::ins_table_add(tab, gpos, len, t, (int)ent[2 * k + 1]);
     }
+}
+
+// The same two steps for a context with the strand / quality sums (amp_exchange.cuh): every entry carries its allele's sums.
+__global__ void amp_ins_pack_qstats_kernel(amp::InsTable tab, amp::QStatsSlots q, unsigned long long* slot, unsigned long long cap_entries,
+                                           unsigned long long cap_arena_words) {
+    unsigned long long n, words;
+    const bool fits = amp::xq_pack_size(tab, cap_entries, cap_arena_words, n, words);
+    const unsigned long long tid = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x, nth = (unsigned long long)gridDim.x * blockDim.x;
+    if (tid == 0) amp::xq_pack_header(tab, slot, fits, n, words, cap_entries);
+    if (!fits) return;
+    for (unsigned long long k = tid; k < n; k += nth) amp::xq_pack_entry(tab, q, slot, k);
+    unsigned long long* dst = amp::xq_slot_arena(slot, cap_entries);
+    const unsigned long long* src = (const unsigned long long*)tab.arena;
+    for (unsigned long long k = tid; k < words; k += nth) dst[k] = src[k];
+}
+__global__ void amp_ins_merge_packed_qstats_kernel(amp::InsTable tab, amp::QStatsSlots q, const unsigned long long* slots,
+                                                   unsigned long long slot_words, unsigned long long cap_entries, int my_rank) {
+    const int r = (int)blockIdx.y;
+    if (r == my_rank) return;
+    const unsigned long long* slot = slots + (unsigned long long)r * slot_words;
+    const unsigned long long n = slot[0];
+    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n; k += (unsigned long long)gridDim.x * blockDim.x)
+        amp::xq_merge_entry(tab, q, slot, cap_entries, k);
 }
 
 // ---- BGZF deflate on the device (amp_deflate.cuh) --------------------------------------------------------------------------
@@ -1447,7 +1462,7 @@ int amp_nccl_allgather(void* comm, const void* dev_send, void* dev_recv, int64_t
 // one ncclAllReduce(sum, int32) over the whole [n_samples][6][lpad] block, in place, asynchronous on `stream`
 int amp_allreduce_counts(amp_ctx* c, void* comm, void* stream) {
     if (!c || !comm) return fail(AMP_ERR_ARG, "amp_allreduce_counts: null argument");
-    if (c->d_rev) return fail(AMP_ERR_STATE, "amp_allreduce_counts: the strand / quality stats are not exchanged across ranks");
+    if (c->d_rev) return fail(AMP_ERR_STATE, "amp_allreduce_counts: the context has the strand / quality sums (amp_allreduce_qstats carries them)");
     NCCL_OR_FAIL(a);
     CK(cudaSetDevice(c->cfg.device));
     const size_t n = (size_t)c->cfg.n_samples * AMP_NCH * (size_t)c->Lpad;
@@ -1462,7 +1477,7 @@ int64_t amp_ins_slot_bytes(int64_t cap_entries, int64_t cap_arena_bytes) {
 }
 int amp_ins_pack_device(amp_ctx* c, void* dev_slot, int64_t cap_entries, int64_t cap_arena_bytes, void* stream) {
     if (!c || !dev_slot || cap_entries < 0 || cap_arena_bytes < 0) return fail(AMP_ERR_ARG, "amp_ins_pack_device: bad argument");
-    if (c->d_rev) return fail(AMP_ERR_STATE, "amp_ins_pack_device: the strand / quality stats are not exchanged across ranks");
+    if (c->d_rev) return fail(AMP_ERR_STATE, "amp_ins_pack_device: the context has the strand / quality sums (amp_ins_pack_qstats_device carries them)");
     CK(cudaSetDevice(c->cfg.device));
     amp_ins_pack_kernel<<<c->sm_count * 2, 512, 0, (cudaStream_t)stream>>>(c->tab, (unsigned long long*)dev_slot, (unsigned long long)cap_entries,
                                                                           (unsigned long long)((cap_arena_bytes + 7) / 8));
@@ -1477,6 +1492,52 @@ int amp_ins_merge_packed(amp_ctx* c, const void* dev_slots, int n_ranks, int my_
     dim3 grid((unsigned)c->sm_count, (unsigned)n_ranks);
     amp_ins_merge_packed_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(c->tab, (const unsigned long long*)dev_slots, slot_words,
                                                                        (unsigned long long)cap_entries, my_rank);
+    CK(cudaGetLastError());
+    return AMP_OK;
+}
+
+// The exchange of a context with the strand / quality sums (amp_qstats_enable): the entry points above refuse it, these carry the
+// sums.  Three ncclAllReduce(sum) over [n_samples][6][lpad] blocks, in place, asynchronous on `stream`: counts and rev (int32), qsum
+// (uint64).
+int amp_allreduce_qstats(amp_ctx* c, void* comm, void* stream) {
+    if (!c || !comm) return fail(AMP_ERR_ARG, "amp_allreduce_qstats: null argument");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, "amp_allreduce_qstats: amp_qstats_enable has not been called");
+    NCCL_OR_FAIL(a);
+    CK(cudaSetDevice(c->cfg.device));
+    const size_t n = (size_t)c->cfg.n_samples * AMP_NCH * (size_t)c->Lpad;
+    int rc = a->AllReduce(c->d_counts, c->d_counts, n, /*ncclInt32*/ 2, /*ncclSum*/ 0, comm, (cudaStream_t)stream);
+    if (!rc) rc = a->AllReduce(c->d_rev, c->d_rev, n, /*ncclInt32*/ 2, /*ncclSum*/ 0, comm, (cudaStream_t)stream);
+    if (!rc) rc = a->AllReduce(c->d_qsum, c->d_qsum, n, /*ncclUint64*/ 5, /*ncclSum*/ 0, comm, (cudaStream_t)stream);
+    if (rc) return nccl_fail(a, rc, "ncclAllReduce");
+    return AMP_OK;
+}
+
+int64_t amp_ins_slot_bytes_qstats(int64_t cap_entries, int64_t cap_arena_bytes) {
+    if (cap_entries < 0 || cap_arena_bytes < 0) return -1;
+    return 16 + 8 * AMP_XQ_WORDS * cap_entries + ((cap_arena_bytes + 7) & ~(int64_t)7);
+}
+int amp_ins_pack_qstats_device(amp_ctx* c, void* dev_slot, int64_t cap_entries, int64_t cap_arena_bytes, void* stream) {
+    if (!c || !dev_slot || cap_entries < 0 || cap_arena_bytes < 0) return fail(AMP_ERR_ARG, "amp_ins_pack_qstats_device: bad argument");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, "amp_ins_pack_qstats_device: amp_qstats_enable has not been called");
+    CK(cudaSetDevice(c->cfg.device));
+    const amp::QStatsSlots q{c->d_ins_rev, c->d_ins_qsum, c->d_ins_head};
+    amp_ins_pack_qstats_kernel<<<c->sm_count * 2, 512, 0, (cudaStream_t)stream>>>(c->tab, q, (unsigned long long*)dev_slot,
+                                                                                 (unsigned long long)cap_entries,
+                                                                                 (unsigned long long)((cap_arena_bytes + 7) / 8));
+    CK(cudaGetLastError());
+    return AMP_OK;
+}
+int amp_ins_merge_packed_qstats(amp_ctx* c, const void* dev_slots, int n_ranks, int my_rank, int64_t cap_entries, int64_t cap_arena_bytes,
+                                void* stream) {
+    if (!c || !dev_slots || n_ranks < 1 || cap_entries < 0 || cap_arena_bytes < 0)
+        return fail(AMP_ERR_ARG, "amp_ins_merge_packed_qstats: bad argument");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, "amp_ins_merge_packed_qstats: amp_qstats_enable has not been called");
+    CK(cudaSetDevice(c->cfg.device));
+    const amp::QStatsSlots q{c->d_ins_rev, c->d_ins_qsum, c->d_ins_head};
+    const unsigned long long slot_words = (unsigned long long)amp_ins_slot_bytes_qstats(cap_entries, cap_arena_bytes) / 8;
+    dim3 grid((unsigned)c->sm_count, (unsigned)n_ranks);
+    amp_ins_merge_packed_qstats_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(c->tab, q, (const unsigned long long*)dev_slots, slot_words,
+                                                                              (unsigned long long)cap_entries, my_rank);
     CK(cudaGetLastError());
     return AMP_OK;
 }

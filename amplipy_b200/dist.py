@@ -11,7 +11,10 @@ Two natural partitions (SURVEY.md section 8e):
 
 On CUDA engines the exchange runs through the C ABI (amp_allreduce_counts, amp_ins_pack_device, amp_nccl_allgather,
 amp_ins_merge_packed) on a communicator made by ``DeepExchange``; engines without that entry point (the CPU emulation
-used by the gloo tests) take the torch.distributed form of the same two steps.
+used by the gloo tests) take the torch.distributed form of the same two steps.  An engine with the strand / quality sums
+(``enable_qstats``) exchanges them too: the all-reduce also sums its rev / qsum matrices and every exchanged insertion
+allele carries its ins_rev / ins_qsum / ins_head (the *_qstats entry points), so the iVar outputs of every rank are those
+of one GPU over all the reads.
 
 The reference has no counterpart (single sequential loop, AmpliPy.py:896)."""
 import numpy as np
@@ -34,7 +37,8 @@ class DeepExchange:
     through the C ABI; the id travels over the torch.distributed group once) and the two slot buffers, allocated once.
 
     cap_entries / cap_arena_bytes: capacity of a rank's slot (distinct insertion alleles / bytes of their records); a
-    table that does not fit raises the engine's TABLE_FULL / ARENA_FULL error flag."""
+    table that does not fit raises the engine's TABLE_FULL / ARENA_FULL error flag.  The engine's strand / quality sums,
+    when it has them at construction (``engine.qstats_enabled``), travel with the counts and the alleles."""
 
     def __init__(self, engine, group=None, cap_entries=1 << 16, cap_arena_bytes=4 << 20):
         import torch
@@ -43,7 +47,9 @@ class DeepExchange:
         self.engine = engine
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         self.cap_entries, self.cap_arena = int(cap_entries), int(cap_arena_bytes)
-        self.slot_bytes = engine.ins_slot_bytes(self.cap_entries, self.cap_arena)
+        self.qstats = engine.qstats_enabled
+        slot_bytes = engine.ins_slot_bytes_qstats if self.qstats else engine.ins_slot_bytes
+        self.slot_bytes = slot_bytes(self.cap_entries, self.cap_arena)
         dev = torch.device("cuda", engine.device)
         self.send = torch.zeros(self.slot_bytes, dtype=torch.uint8, device=dev)
         self.recv = torch.zeros(self.slot_bytes * self.world, dtype=torch.uint8, device=dev)
@@ -52,23 +58,31 @@ class DeepExchange:
     def run(self, stream=None):
         """all-reduce of the counts + exchange of the insertion tables, asynchronous on ``stream`` (a raw cudaStream_t)."""
         e = self.engine
-        e.allreduce_counts(self.comm, stream)
-        e.ins_pack_device(self.send.data_ptr(), self.cap_entries, self.cap_arena, stream)
+        if self.qstats:
+            allreduce, pack, merge = e.allreduce_qstats, e.ins_pack_qstats_device, e.ins_merge_packed_qstats
+        else:
+            allreduce, pack, merge = e.allreduce_counts, e.ins_pack_device, e.ins_merge_packed
+        allreduce(self.comm, stream)
+        pack(self.send.data_ptr(), self.cap_entries, self.cap_arena, stream)
         self.comm.allgather(self.send.data_ptr(), self.recv.data_ptr(), self.slot_bytes, stream)
-        e.ins_merge_packed(self.recv.data_ptr(), self.world, self.rank, self.cap_entries, self.cap_arena, stream)
+        merge(self.recv.data_ptr(), self.world, self.rank, self.cap_entries, self.cap_arena, stream)
 
     def close(self):
         self.comm.close()
 
 
 def allreduce_counts(engine, group=None):
-    """torch.distributed form: sum the per-rank count matrices in place (every rank ends up with the total)."""
+    """torch.distributed form: sum the per-rank count matrices in place (every rank ends up with the total), and the rev /
+    qsum matrices of an engine with the strand / quality sums."""
     import torch.distributed as dist
     t = engine.counts_tensor()
     if t.is_cuda:
         import torch
         torch.cuda.synchronize(t.device)
     dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    if getattr(engine, "qstats_enabled", False):
+        for s in engine.qstats_tensors():
+            dist.all_reduce(s, op=dist.ReduceOp.SUM, group=group)
     return t
 
 
@@ -80,22 +94,27 @@ def allgather_insertions(engine, group=None):
     world = dist.get_world_size(group)
     ins = engine.insertions()
     mine = (np.asarray(ins.sample), np.asarray(ins.pos), np.asarray(ins.count), np.asarray(ins.str_off), np.asarray(ins.chars))
+    if getattr(engine, "qstats_enabled", False):     # each allele's strand / quality sums travel with it
+        qs = engine.qstats()
+        mine += (np.asarray(qs.ins_rev), np.asarray(qs.ins_qsum), np.asarray(qs.ins_head))
     gathered = [None] * world
     dist.all_gather_object(gathered, mine, group=group)
-    for r, (sample, pos, count, off, chars) in enumerate(gathered):
-        if r != rank and len(pos):
-            engine.merge_insertions(sample, pos, count, off, chars)
+    for r, part in enumerate(gathered):
+        if r != rank and len(part[1]):
+            engine.merge_insertions(*part)
     return engine.insertions()
 
 
-def process_deep_sample(engine, batch, trim=True, pileup=True, sample=0, group=None, exchange=None):
+def process_deep_sample(engine, batch, trim=True, pileup=True, sample=0, group=None, exchange=None, qstats=False):
     """Read-sharded processing of one sample: local kernel on this rank's read range, then the exchange step.
     Returns this rank's TrimResult (valid for its own range of reads only; the other reads' flags are 0).
-    ``exchange``: a DeepExchange to reuse (CUDA engines); one is created and closed when it is None."""
+    ``exchange``: a DeepExchange to reuse (CUDA engines); one is created and closed when it is None.
+    ``qstats``: the strand / quality pass runs on the same reads (engine.enable_qstats first); the exchange carries the sums
+    whenever the engine has them.  Without it, engine.process is called as before, so engines without the pass work unchanged."""
     import torch.distributed as dist
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     first, count = read_range(batch.n, rank, world)
-    t = engine.process(batch, trim=trim, pileup=pileup, sample=sample, first=first, n=count)
+    t = engine.process(batch, trim=trim, pileup=pileup, sample=sample, first=first, n=count, **({"qstats": True} if qstats else {}))
     if pileup and world > 1:
         if hasattr(engine, "ins_pack_device"):
             import torch

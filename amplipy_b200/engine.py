@@ -43,7 +43,8 @@ EXPORTED_SYMBOLS = [
     "amp_bam_decode_host", "amp_process_decoded", "amp_decoded_copy_host", "amp_counts_upload", "amp_bgzf_deflate_host", "amp_decoded_write_bam",
     "amp_set_scheme", "amp_get_scheme", "amp_set_sample_reference", "amp_qstats_enable", "amp_qstats_host", "amp_call_ivar",
     "amp_call_ivar_device", "amp_contig_plan_decoded", "amp_contig_plan_device", "amp_process_contigs", "amp_set_features",
-    "amp_annotate", "amp_annot_host"]
+    "amp_annotate", "amp_annot_host", "amp_allreduce_qstats", "amp_ins_slot_bytes_qstats", "amp_ins_pack_qstats_device",
+    "amp_ins_merge_packed_qstats"]
 
 
 class AmpConfig(ctypes.Structure):
@@ -130,6 +131,7 @@ def load_library():
         lib = ctypes.CDLL(LIB_PATH)
         lib.amp_last_error.restype = ctypes.c_char_p
         lib.amp_ins_slot_bytes.restype = ctypes.c_int64
+        lib.amp_ins_slot_bytes_qstats.restype = ctypes.c_int64
         for name in EXPORTED_SYMBOLS:
             try:
                 getattr(lib, name)   # AttributeError if the build is stale
@@ -222,6 +224,7 @@ class Engine:
         self.lpad = int(self.lib.amp_lpad(self._ctx))
         self.device = device
         self.launches = 0
+        self._qstats = False
 
     def close(self):
         if getattr(self, "_ctx", None) is not None and self._ctx.value:
@@ -597,10 +600,38 @@ class Engine:
                                              ctypes.c_void_p(stream) if stream else None), "amp_ins_merge_packed")
         self.launches += 1
 
+    # the same exchange for a context with the strand / quality sums (enable_qstats): the methods above refuse such a context
+    def allreduce_qstats(self, comm, stream=None):
+        """ncclAllReduce(sum) of the counts, rev and qsum matrices, in place (``comm``: NcclComm or a raw ncclComm_t value)."""
+        h = comm.handle if hasattr(comm, "handle") else comm
+        _check(self.lib.amp_allreduce_qstats(self._ctx, ctypes.c_void_p(h), ctypes.c_void_p(stream) if stream else None),
+               "amp_allreduce_qstats")
+
+    def ins_slot_bytes_qstats(self, cap_entries, cap_arena_bytes):
+        return int(self.lib.amp_ins_slot_bytes_qstats(ctypes.c_int64(cap_entries), ctypes.c_int64(cap_arena_bytes)))
+
+    def ins_pack_qstats_device(self, dev_ptr, cap_entries, cap_arena_bytes, stream=None):
+        _check(self.lib.amp_ins_pack_qstats_device(self._ctx, ctypes.c_void_p(dev_ptr), ctypes.c_int64(cap_entries),
+                                                   ctypes.c_int64(cap_arena_bytes), ctypes.c_void_p(stream) if stream else None),
+               "amp_ins_pack_qstats_device")
+        self.launches += 1
+
+    def ins_merge_packed_qstats(self, dev_ptr, n_ranks, my_rank, cap_entries, cap_arena_bytes, stream=None):
+        _check(self.lib.amp_ins_merge_packed_qstats(self._ctx, ctypes.c_void_p(dev_ptr), int(n_ranks), int(my_rank),
+                                                    ctypes.c_int64(cap_entries), ctypes.c_int64(cap_arena_bytes),
+                                                    ctypes.c_void_p(stream) if stream else None), "amp_ins_merge_packed_qstats")
+        self.launches += 1
+
     # ---------------------------------------------------------------- iVar-format outputs (DESIGN.md 3.7)
     def enable_qstats(self):
         """Allocate the strand / quality sums (amp_qstats_enable); process(..., qstats=True) fills them."""
         _check(self.lib.amp_qstats_enable(self._ctx), "amp_qstats_enable")
+        self._qstats = True
+
+    @property
+    def qstats_enabled(self):
+        """True once enable_qstats has succeeded: the context holds the strand / quality sums."""
+        return self._qstats
 
     def qstats(self, sample=0):
         """The strand / quality sums of one sample: rev / qsum [6, L] and, in insertions() order (all samples), ins_rev /

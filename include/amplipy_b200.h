@@ -160,8 +160,9 @@ int amp_call_device(amp_ctx* ctx, const amp_call_params* p, void* stream);
  * position), rev = the count matrix's increments from reverse-strand reads (flag & 0x10) and qsum = the phred qualities of the
  * counted A C G T N bases ('-' carries none), plus the same two sums per insertion allele (an event's quality = that of the first
  * inserted base past the gates 718 / 722).  amp_process_* with AMP_MODE_PILEUP | AMP_MODE_QSTATS then runs a second pass over the
- * same reads after the fused kernel; amp_reset / amp_reset_async zero the sums.  The sums are not exchanged across ranks:
- * amp_allreduce_counts and amp_ins_pack_device return AMP_ERR_STATE on a context with them enabled.
+ * same reads after the fused kernel; amp_reset / amp_reset_async zero the sums.  Across ranks the sums travel through the
+ * *_qstats entry points of the deep-sample mode below; amp_allreduce_counts and amp_ins_pack_device, which would leave them
+ * behind, return AMP_ERR_STATE on a context with them enabled.
  * amp_qstats_host: host arrays rev [6][L], qsum [6][L] of one sample, and ins_rev / ins_qsum / ins_head [n_alleles] in
  * amp_ins_export order (ins_head[k] = 1: an event of allele k is the key of AmpliPy.py:735-736); any pointer may be NULL.
  * amp_call_ivar (after amp_call): per allele mean quality mq = floor(qsum / count) ('-': the position's mean base quality) and,
@@ -200,6 +201,21 @@ int64_t amp_ins_slot_bytes(int64_t cap_entries, int64_t cap_arena_bytes);
 int amp_ins_pack_device(amp_ctx* ctx, void* dev_slot, int64_t cap_entries, int64_t cap_arena_bytes, void* stream);
 int amp_ins_merge_packed(amp_ctx* ctx, const void* dev_slots, int n_ranks, int my_rank, int64_t cap_entries,
                          int64_t cap_arena_bytes, void* stream);
+/* The same exchange for a context with the strand / quality sums (amp_qstats_enable); each returns AMP_ERR_STATE on a context
+ * without them (and amp_allreduce_qstats does so before it calls NCCL).  Afterwards every rank holds what one context over all the
+ * reads would hold: counts, insertion alleles, rev / qsum and each allele's ins_rev / ins_qsum / ins_head.
+ *   amp_allreduce_qstats         three ncclAllReduce(sum), in place: counts and rev (int32), qsum (uint64)
+ *   amp_ins_slot_bytes_qstats    16 + 32 * cap_entries + cap_arena_bytes rounded up to 8
+ *   amp_ins_pack_qstats_device   { u64 n_alleles, u64 arena_words,
+ *                                  {u64 arena offset, u64 count, u64 ins_qsum, u64 ins_rev | ins_head << 32}[cap_entries],
+ *                                  arena[cap_arena_bytes] }; the same overflow contract as amp_ins_pack_device
+ *   amp_ins_merge_packed_qstats  the other ranks' alleles with their sums; an allele the table cannot take gets no sums (the
+ *                                TABLE_FULL / ARENA_FULL bit reports the loss) */
+int amp_allreduce_qstats(amp_ctx* ctx, void* comm, void* stream);
+int64_t amp_ins_slot_bytes_qstats(int64_t cap_entries, int64_t cap_arena_bytes);
+int amp_ins_pack_qstats_device(amp_ctx* ctx, void* dev_slot, int64_t cap_entries, int64_t cap_arena_bytes, void* stream);
+int amp_ins_merge_packed_qstats(amp_ctx* ctx, const void* dev_slots, int n_ranks, int my_rank, int64_t cap_entries,
+                                int64_t cap_arena_bytes, void* stream);
 
 /* pre-size what amp_process_device would otherwise grow on demand (it synchronises `stream` when it has to allocate) */
 int amp_reserve(amp_ctx* ctx, int64_t max_reads, int64_t max_cigar_ops);
