@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libamplipy_b200.so")
 SOURCES = ["amp_abi.cu"]
-HEADERS = ["amp_core.cuh", "amp_kernels.cuh", "amp_warp.cuh", "amp_call.cuh", "amp_bgzf.cuh", "amp_ont.cuh", "amp_deflate.cuh", "amp_ivar.cuh", "amp_contig.cuh", "amp_annot.cuh", "amp_exchange.cuh", os.path.join("..", "..", "include", "amplipy_b200.h")]
+HEADERS = ["amp_core.cuh", "amp_kernels.cuh", "amp_warp.cuh", "amp_call.cuh", "amp_bgzf.cuh", "amp_ont.cuh", "amp_deflate.cuh", "amp_ivar.cuh", "amp_contig.cuh", "amp_annot.cuh", "amp_exchange.cuh", "amp_dels.cuh", os.path.join("..", "..", "include", "amplipy_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

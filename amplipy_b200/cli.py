@@ -66,6 +66,9 @@ ERROR_TEXT_BAD_REFID = "Read reference ID outside the alignment header"
 HELP_TEXT_GFF = ("GFF3 file whose CDS features fill the GFF_FEATURE / codon / amino-acid columns of the TSV (optional; needs "
                  "--output_tsv)")
 ERROR_TEXT_GFF_NEEDS_TSV = "--gff needs --output_tsv"
+HELP_TEXT_IVAR_DELETIONS = ("Write deletions in the TSV as iVar does: one row per deletion allele at the aligned base before it, ALT = '-' + "
+                            "the deleted bases, instead of one '-' row per deleted base (optional; needs --output_tsv)")
+ERROR_TEXT_DELS_NEEDS_TSV = "--ivar_deletions needs --output_tsv"
 HELP_TEXT_IUPAC_THRESHOLD = ("Write IUPAC ambiguity codes: the shortest prefix of the sorted alleles whose frequencies reach this "
                              "threshold (0-1) is coded (optional; 0 = the plain consensus)")
 
@@ -110,6 +113,7 @@ def parse_args(argv=None):
     v.add_argument('-md', '--min_depth', required=False, type=int, default=DEFAULT_MIN_DEPTH_VARIANTS, help=HELP_TEXT_MIN_DEPTH_VARIANTS)
     v.add_argument('--output_tsv', required=False, type=str, default=None, help=HELP_TEXT_TSV)
     v.add_argument('--gff', required=False, type=str, default=None, help=HELP_TEXT_GFF)
+    v.add_argument('--ivar_deletions', action='store_true', help=HELP_TEXT_IVAR_DELETIONS)
 
     c = sub.add_parser("consensus", description=DESCRIPTION, formatter_class=F)
     c.add_argument('-i', '--input', required=False, type=str, default='stdin', help=HELP_TEXT_READS_TRIMMED)
@@ -142,6 +146,7 @@ def parse_args(argv=None):
     a.add_argument('-e', '--include_no_primer', action='store_true', help=HELP_TEXT_TRIM_INCLUDE_READS_NO_PRIMER)
     a.add_argument('--output_tsv', required=False, type=str, default=None, help=HELP_TEXT_TSV)
     a.add_argument('--gff', required=False, type=str, default=None, help=HELP_TEXT_GFF)
+    a.add_argument('--ivar_deletions', action='store_true', help=HELP_TEXT_IVAR_DELETIONS)
     a.add_argument('--iupac_threshold', required=False, type=float, default=None, help=HELP_TEXT_IUPAC_THRESHOLD)
     return parser.parse_args(argv)
 
@@ -250,23 +255,30 @@ def check_contig_plan(plan, refs=None, ref_map=None):
         raise InputError(ERROR_TEXT_BAD_REFID)
 
 
+def dels_slots(sum_cigar_ops):
+    """Slots of the anchored deletion table for a batch of ``sum_cigar_ops`` CIGAR ops: every allele comes from a D op of the input
+    (trimming merges or drops D ops, it adds none), so twice their total, rounded up to a power of two, never fills."""
+    return max(1024, 1 << int(2 * max(int(sum_cigar_ops), 1) - 1).bit_length())
+
+
 def run_amplipy(untrimmed_reads_fn=None, primer_fn=None, reference_fn=None, trimmed_reads_fn=None, variants_fn=None,
                 consensus_fn=None, primer_pos_offset=None, min_length=None, min_quality=None, sliding_window_width=None,
                 min_freq_consensus=None, min_freq_variants=None, min_depth_consensus=None, min_depth_variants=None,
                 unknown_symbol=None, include_no_primer=None, run_trim=False, run_variants=False, run_consensus=False,
-                argv=None, device=0, tsv_fn=None, iupac_threshold=None, multi_contig=False, gff_fn=None):
+                argv=None, device=0, tsv_fn=None, iupac_threshold=None, multi_contig=False, gff_fn=None, ivar_deletions=False):
     """Same keyword arguments and behaviour as the reference's run_amplipy (AmpliPy.py:774-963).  Additions of this
     project: ``tsv_fn`` (with run_variants) also writes the variants in iVar's TSV format, ``iupac_threshold`` (with
     run_consensus) writes IUPAC ambiguity codes into the consensus (DESIGN.md 3.7), ``multi_contig`` takes every record of the
     reference FASTA as a contig (DESIGN.md 3.8), ``gff_fn`` (with ``tsv_fn``) fills the TSV's codon columns from the CDS
-    features of a GFF3 file (DESIGN.md 3.9)."""
+    features of a GFF3 file (DESIGN.md 3.9), ``ivar_deletions`` (with ``tsv_fn``) writes the TSV's deletions as iVar does, one
+    row per anchored deletion allele (DESIGN.md 3.7)."""
     argv = list(sys.argv if argv is None else argv)
     try:
         return _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
                     min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
                     min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
                     tsv_fn if run_variants else None, iupac_threshold if run_consensus else None, multi_contig,
-                    gff_fn if run_variants else None)
+                    gff_fn if run_variants else None, bool(ivar_deletions) and run_variants)
     except InputError as e:
         error(str(e))
 
@@ -274,7 +286,7 @@ def run_amplipy(untrimmed_reads_fn=None, primer_fn=None, reference_fn=None, trim
 def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
          min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
          unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn=None, iupac_threshold=None,
-         multi_contig=False, gff_fn=None):
+         multi_contig=False, gff_fn=None, ivar_deletions=False):
     # validity checks (AmpliPy.py:837-854)
     if primer_pos_offset is not None and primer_pos_offset < 0:
         error("%s: %s" % (ERROR_TEXT_NEGATIVE_PRIMER_POS_OFFSET, primer_pos_offset))
@@ -298,6 +310,8 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         error("%s: %s" % (ivar.ERROR_TEXT_INVALID_IUPAC_THRESHOLD, iupac_threshold))
     if gff_fn is not None and tsv_fn is None:
         error(ERROR_TEXT_GFF_NEEDS_TSV)
+    if ivar_deletions and tsv_fn is None:
+        error(ERROR_TEXT_DELS_NEEDS_TSV)
 
     # mode banner (AmpliPy.py:857-866)
     if not (run_trim or run_variants or run_consensus):
@@ -316,7 +330,7 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         return _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset,
                             min_length, min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus,
                             min_depth_variants, unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device,
-                            tsv_fn, iupac_threshold, gff_fn)
+                            tsv_fn, iupac_threshold, gff_fn, ivar_deletions)
     ref_id, ref_seq = load_ref_genome(reference_fn)
     L = len(ref_seq)
     tables, mpl = None, 0
@@ -390,6 +404,8 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         print_log("Processing reads...")
         try:
             info = eng.decode_bam(raw, layout)
+            if ivar_deletions:
+                eng.enable_dels(dels_slots(info["sum_cig"]))
             outs = eng.process_decoded(trim=run_trim, pileup=pile, download=not dev_bam_out, **({"qstats": True} if qstats else {}))
             n_reads = info["n"]
         except AmpError:
@@ -415,6 +431,8 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
         out_header = alnio.header_with_pg(aln.header_text, argv) if run_trim else None
         indel_rich = aln.n and (aln.batch.cigar.size / aln.n) > 8
         eng = make_engine(indel_rich)
+        if ivar_deletions:
+            eng.enable_dels(dels_slots(aln.batch.cigar.size))
         print_log("Processing reads...")
         _t = _time.perf_counter()
         trim = eng.process(aln.batch, trim=run_trim, pileup=pile, **({"qstats": True} if qstats else {}))
@@ -462,7 +480,9 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
             if features is not None:
                 eng.set_features(0, features)     # after call: the context holds the reference now
                 ann, names = eng.annotate(), [f.name for f in features]
-            ivar.write_tsv(tsv_fn, ivar.tsv_rows(res, ins, iv, eng.qstats(0), ref_id, ref_seq, counts, ann=ann, names=names))
+            dels = eng.call_ivar_dels(DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
+                                      DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants) if ivar_deletions else None
+            ivar.write_tsv(tsv_fn, ivar.tsv_rows(res, ins, iv, eng.qstats(0), ref_id, ref_seq, counts, ann=ann, names=names, dels=dels))
         iupac = None
         if iupac_threshold is not None:
             iupac = eng.call_ivar(DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
@@ -493,7 +513,8 @@ def _run(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants
 
 def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, variants_fn, consensus_fn, primer_pos_offset, min_length,
                  min_quality, sliding_window_width, min_freq_consensus, min_freq_variants, min_depth_consensus, min_depth_variants,
-                 unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn, iupac_threshold, gff_fn=None):
+                 unknown_symbol, include_no_primer, run_trim, run_variants, run_consensus, argv, device, tsv_fn, iupac_threshold, gff_fn=None,
+                 ivar_deletions=False):
     """_run with --multi_contig (DESIGN.md 3.8): contig k of the FASTA is sample k of one context, with the BED rows of its chrom as
     its scheme and its own length; reads go to the contig their reference names.  Outputs follow the FASTA's record order."""
     contigs = load_ref_genomes(reference_fn)
@@ -558,6 +579,8 @@ def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, 
             dev_bam_out = False
         if eng is not None:
             check_contig_plan(eng.contig_plan_decoded(ref_map), layout["refs"], ref_map)
+            if ivar_deletions:
+                eng.enable_dels(dels_slots(info["sum_cig"]))
             outs = eng.process_decoded_contigs(download=not dev_bam_out, **mode)
             eng.raise_on_device_errors()
             n_reads = info["n"]
@@ -569,6 +592,8 @@ def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, 
         out_header = alnio.header_with_pg(aln.header_text, argv) if run_trim else None
         sid = sam_read_contigs(aln, contigs) if aln.fmt == "sam" else bam_read_contigs(aln, contigs)
         eng = make_engine(aln.n and (aln.batch.cigar.size / aln.n) > 8)
+        if ivar_deletions:
+            eng.enable_dels(dels_slots(aln.batch.cigar.size))
         print_log("Processing reads...")
         try:
             trim = eng.process_contigs(aln.batch, sid, **mode)
@@ -606,9 +631,12 @@ def _run_contigs(untrimmed_reads_fn, primer_fn, reference_fn, trimmed_reads_fn, 
                 for k, fk in enumerate(features):
                     eng.set_features(k, fk)
                 ann = eng.annotate()
+            dels = eng.call_ivar_dels(DEFAULT_MIN_DEPTH_VARIANTS if min_depth_variants is None else min_depth_variants,
+                                      DEFAULT_MIN_FREQ_VARIANTS if min_freq_variants is None else min_freq_variants) if ivar_deletions else None
             ivar.write_tsv(tsv_fn, [r for k, (cid, seq) in enumerate(contigs)
                                     for r in ivar.tsv_rows(res, ins, iv, eng.qstats(k), cid, seq, counts[k], k, L=len(seq), ann=ann,
-                                                           names=[f.name for f in features[k]] if features is not None else None)])
+                                                           names=[f.name for f in features[k]] if features is not None else None,
+                                                           dels=dels)])
         iupac = None
         if iupac_threshold is not None:
             iupac = eng.call_ivar(DEFAULT_MIN_DEPTH_CONSENSUS if min_depth_consensus is None else min_depth_consensus,
@@ -641,7 +669,8 @@ def main(argv=None):
     elif args.command == 'variants':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, variants_fn=args.output,
                     min_quality=args.min_quality, min_freq_variants=args.min_freq, min_depth_variants=args.min_depth,
-                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv, multi_contig=args.multi_contig, gff_fn=args.gff)
+                    run_variants=True, argv=full_argv, tsv_fn=args.output_tsv, multi_contig=args.multi_contig, gff_fn=args.gff,
+                    ivar_deletions=args.ivar_deletions)
     elif args.command == 'consensus':
         run_amplipy(trimmed_reads_fn=args.input, reference_fn=args.reference, consensus_fn=args.output,
                     min_quality=args.min_quality, min_freq_consensus=args.min_freq, min_depth_consensus=args.min_depth,
@@ -656,7 +685,8 @@ def main(argv=None):
                     min_depth_consensus=args.min_depth_consensus, min_depth_variants=args.min_depth_variants,
                     unknown_symbol=args.unknown_symbol, include_no_primer=args.include_no_primer, run_trim=True,
                     run_variants=True, run_consensus=True, argv=full_argv, tsv_fn=args.output_tsv,
-                    iupac_threshold=args.iupac_threshold, multi_contig=args.multi_contig, gff_fn=args.gff)
+                    iupac_threshold=args.iupac_threshold, multi_contig=args.multi_contig, gff_fn=args.gff,
+                    ivar_deletions=args.ivar_deletions)
 
 
 if __name__ == "__main__":

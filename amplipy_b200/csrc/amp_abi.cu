@@ -22,9 +22,9 @@
 
 static_assert(AMP_F_TRIM_START == AMP_FLAG_TRIM_START && AMP_F_KEEP == AMP_FLAG_KEEP && AMP_F_SKIPPED == AMP_FLAG_SKIPPED &&
                   AMP_F_ERROR == AMP_FLAG_ERROR && AMP_E_ARENA_FULL == AMP_DEVERR_ARENA_FULL &&
-                  AMP_E_QSTATS_MISS == AMP_DEVERR_QSTATS_MISS,
+                  AMP_E_QSTATS_MISS == AMP_DEVERR_QSTATS_MISS && AMP_E_DELS_FULL == AMP_DEVERR_DELS_FULL,
               "flag constants out of sync with include/amplipy_b200.h");
-static_assert(sizeof(amp::Seg) == 16 && sizeof(amp::InsSlot) == 16, "layout");
+static_assert(sizeof(amp::Seg) == 16 && sizeof(amp::InsSlot) == 16 && sizeof(amp::DelSlot) == 24, "layout");
 
 namespace {
 
@@ -97,10 +97,50 @@ __global__ void __launch_bounds__(AMP_QS_READS) amp_qstats_kernel(const __grid_c
     amp::cta_qstats(P, trev, tq, &lo, (int)blockIdx.x, (int)blockDim.x);
 }
 
+// The same pass on a context with the deletion-allele table (amp_dels_enable): the anchored deletion events go to the table too
+__global__ void __launch_bounds__(AMP_QS_READS) amp_qstats_dels_kernel(const __grid_constant__ amp::QStatsParams P) {
+    __shared__ int trev[AMP_NCH * AMP_QS_WT], tq[AMP_NCH * AMP_QS_WT];
+    __shared__ int lo;
+    amp::cta_qstats<true>(P, trev, tq, &lo, (int)blockIdx.x, (int)blockDim.x);
+}
+
 // iVar calling (amp_ivar.cuh): one thread per (sample, position), after amp_call_kernel on its outputs
 __global__ void __launch_bounds__(256) amp_ivar_kernel(const __grid_constant__ amp::IvarParams P) {
     const long long gp = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (gp < (long long)P.n_samples * P.L) amp::ivar_position(P, gp);
+}
+
+// iVar calling of the deletion alleles (amp_ivar.cuh): one thread per listed allele
+__global__ void __launch_bounds__(256) amp_ivar_dels_kernel(const __grid_constant__ amp::IvarDelParams P) {
+    const unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x;
+    if (k < P.n) amp::ivar_del(P, k);
+}
+
+// the deletion alleles in list order: key, count | rev << 32, qsum
+__global__ void amp_dels_gather_kernel(amp::DelTable T, unsigned long long n, unsigned long long* o) {
+    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n; k += (unsigned long long)gridDim.x * blockDim.x) {
+        const amp::DelSlot s = T.slots[T.entries[k]];
+        o[3 * k] = s.key; o[3 * k + 1] = s.cr; o[3 * k + 2] = s.qsum;
+    }
+}
+
+// alleles given as {key, count | rev << 32, qsum} added to the table (amp_dels_merge)
+__global__ void amp_dels_merge_kernel(amp::DelTable T, unsigned long long n, const unsigned long long* in) {
+    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n; k += (unsigned long long)gridDim.x * blockDim.x)
+        amp::del_table_add(T, (int)(in[3 * k] >> 32), (int)(in[3 * k] & 0xFFFFFFFFu), (unsigned int)in[3 * k + 1],
+                           (unsigned int)(in[3 * k + 1] >> 32), in[3 * k + 2]);
+}
+
+// Reset of the deletion table, one block: its listed slots, then its cursor.  Runs on the stream of amp_reset_kernel, which
+// clears the error word.
+__global__ void __launch_bounds__(1024) amp_dels_reset_kernel(amp::DelTable T) {
+    const unsigned long long n = T.cursor[0];
+    for (unsigned long long k = threadIdx.x; k < n; k += blockDim.x) {
+        amp::DelSlot z; z.key = 0; z.cr = 0; z.qsum = 0;
+        T.slots[T.entries[k]] = z;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) T.cursor[0] = 0;
 }
 
 // the per-slot stats of the insertion alleles in amp_ins_export order
@@ -228,6 +268,24 @@ __global__ void amp_ins_merge_packed_qstats_kernel(amp::InsTable tab, amp::QStat
     const unsigned long long n = slot[0];
     for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n; k += (unsigned long long)gridDim.x * blockDim.x)
         amp::xq_merge_entry(tab, q, slot, cap_entries, k);
+}
+
+// The deletion table of a rank packed into one fixed-size slot and the other ranks' slots merged (amp_exchange.cuh)
+__global__ void amp_dels_pack_kernel(amp::DelTable T, unsigned long long* slot, unsigned long long cap_entries) {
+    unsigned long long n;
+    const bool fits = amp::xd_pack_size(T, cap_entries, n);
+    const unsigned long long tid = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x, nth = (unsigned long long)gridDim.x * blockDim.x;
+    if (tid == 0) amp::xd_pack_header(T, slot, fits, n);
+    if (!fits) return;
+    for (unsigned long long k = tid; k < n; k += nth) amp::xd_pack_entry(T, slot, k);
+}
+__global__ void amp_dels_merge_packed_kernel(amp::DelTable T, const unsigned long long* slots, unsigned long long slot_words, int my_rank) {
+    const int r = (int)blockIdx.y;
+    if (r == my_rank) return;
+    const unsigned long long* slot = slots + (unsigned long long)r * slot_words;
+    const unsigned long long n = slot[0];
+    for (unsigned long long k = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; k < n; k += (unsigned long long)gridDim.x * blockDim.x)
+        amp::xd_merge_entry(T, slot, k);
 }
 
 // ---- BGZF deflate on the device (amp_deflate.cuh) --------------------------------------------------------------------------
@@ -522,6 +580,9 @@ struct amp_ctx {
     int* d_ins_rev = nullptr; unsigned long long* d_ins_qsum = nullptr; unsigned char* d_ins_head = nullptr;
     unsigned char* d_ivar = nullptr;    // iVar calling outputs (one block, offsets below)
     size_t o_iu = 0, o_fmq = 0, o_fpv = 0, o_imq = 0, o_ipv = 0;
+    // anchored deletion alleles (amp_dels_enable): the table, and the calling outputs (mq, then pval; grown at high-water marks)
+    amp::DelTable dels{}; unsigned long long dels_nslots = 0;
+    unsigned long long* d_dels_out = nullptr; size_t dels_out_words = 0;
     // a batch grouped by contig (amp_contig_plan_* / amp_process_contigs; buffers grown at high-water marks)
     struct Contigs {
         int source = 0;                                           // the planned batch: 0 none, 1 the decoded one, 2 a device batch
@@ -706,7 +767,9 @@ int launch_process(amp_ctx* c, const amp::BatchPtrs& b, long long sum_cig, long 
     Q.Lpad = c->Lpad; Q.minq = c->cfg.min_quality; Q.gpos_base = sample * c->Lpad;
     Q.rev = c->d_rev + (size_t)sample * AMP_NCH * c->Lpad; Q.qsum = c->d_qsum + (size_t)sample * AMP_NCH * c->Lpad;
     Q.tab = c->tab; Q.ins_rev = c->d_ins_rev; Q.ins_qsum = c->d_ins_qsum; Q.ins_head = c->d_ins_head; Q.err = c->d_err;
-    amp_qstats_kernel<<<(unsigned)((b.n + AMP_QS_READS - 1) / AMP_QS_READS), AMP_QS_READS, 0, st>>>(Q);
+    const unsigned grid = (unsigned)((b.n + AMP_QS_READS - 1) / AMP_QS_READS);
+    if (c->dels.slots) { Q.dels = c->dels; amp_qstats_dels_kernel<<<grid, AMP_QS_READS, 0, st>>>(Q); }
+    else amp_qstats_kernel<<<grid, AMP_QS_READS, 0, st>>>(Q);
     CK(cudaGetLastError());
     c->last_launches += 1;
     return AMP_OK;
@@ -779,6 +842,7 @@ int amp_destroy(amp_ctx* c) {
     if (c->defl.stream) cudaStreamDestroy(c->defl.stream);
     cudaFree(c->defl.in); cudaFree(c->defl.slots); cudaFree(c->defl.out); cudaFree(c->defl.bstart); cudaFree(c->defl.off); cudaFree(c->defl.clen); cudaFree(c->defl.crc); cudaFree(c->defl.ctr); cudaFree(c->defl.toks);
     cudaFree(c->d_rev); cudaFree(c->d_qsum); cudaFree(c->d_ins_rev); cudaFree(c->d_ins_qsum); cudaFree(c->d_ins_head); cudaFree(c->d_ivar);
+    cudaFree(c->dels.slots); cudaFree(c->dels.entries); cudaFree(c->dels.cursor); cudaFree(c->d_dels_out);
     cudaFree(c->d_err); cudaFree(c->d_reset_done); cudaFree(c->d_scratch); cudaFree(c->d_glist); cudaFree(c->d_ref); cudaFree(c->d_call); cudaFree(c->d_xbuf);
     {
         auto& d = c->dec;
@@ -820,6 +884,10 @@ int amp_reset(amp_ctx* c) {
         CK(cudaMemsetAsync(c->d_ins_rev, 0, c->nslots * 4, 0)); CK(cudaMemsetAsync(c->d_ins_qsum, 0, c->nslots * 8, 0));
         CK(cudaMemsetAsync(c->d_ins_head, 0, c->nslots, 0));
     }
+    if (c->dels.slots) {
+        CK(cudaMemsetAsync(c->dels.slots, 0, c->dels_nslots * sizeof(amp::DelSlot), 0));
+        CK(cudaMemsetAsync(c->dels.cursor, 0, 8, 0));
+    }
     CK(cudaStreamSynchronize(0));
     return AMP_OK;
 }
@@ -836,6 +904,10 @@ int amp_reset_async(amp_ctx* c, void* stream) {
                                                         c->tab.cursor, c->d_err, c->d_reset_done, (uint4*)c->d_rev, (uint4*)c->d_qsum, counts16,
                                                         c->d_ins_rev, c->d_ins_qsum, c->d_ins_head);
     CK(cudaGetLastError());
+    if (c->dels.slots) {
+        amp_dels_reset_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(c->dels);
+        CK(cudaGetLastError());
+    }
     return AMP_OK;
 }
 
@@ -1248,6 +1320,162 @@ int amp_call_ivar(amp_ctx* c, const amp_ivar_params* p, uint8_t* iupac, int32_t*
     if (K && ins_mq) CK(cudaMemcpyAsync(ins_mq, out + c->o_imq, K * 4, cudaMemcpyDeviceToHost, st));
     if (K && ins_pval) CK(cudaMemcpyAsync(ins_pval, out + c->o_ipv, K * 8, cudaMemcpyDeviceToHost, st));
     if (K) CK(cudaStreamSynchronize(st));
+    return AMP_OK;
+}
+
+// ---- anchored deletion alleles (amp_dels.cuh) ------------------------------------------------------------------------------------
+int amp_dels_enable(amp_ctx* c, int64_t slots) {
+    if (!c || slots < 0 || slots > (1LL << 40)) return fail(AMP_ERR_ARG, "amp_dels_enable: bad argument");
+    if (!c->d_rev) return fail(AMP_ERR_STATE, "amp_dels_enable: amp_qstats_enable has not been called (the strand / quality pass fills the table)");
+    if (c->dels.slots) return AMP_OK;
+    unsigned long long n = slots > 0 ? (unsigned long long)slots : (1ULL << 20);
+    while (n & (n - 1)) n += n & (~n + 1);   // round up to a power of two
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    CK(cudaMalloc((void**)&c->dels.slots, n * sizeof(amp::DelSlot)));
+    CK(cudaMalloc((void**)&c->dels.entries, n * 4));
+    CK(cudaMalloc((void**)&c->dels.cursor, 8));
+    CK(cudaMemset(c->dels.slots, 0, n * sizeof(amp::DelSlot)));
+    CK(cudaMemset(c->dels.cursor, 0, 8));
+    c->dels.mask = n - 1; c->dels.err = c->d_err; c->dels_nslots = n;
+    return AMP_OK;
+}
+
+static int dels_check(amp_ctx* c, const char* who) {
+    if (!c) return fail(AMP_ERR_ARG, who, "null context");
+    if (!c->dels.slots) return fail(AMP_ERR_STATE, who, "amp_dels_enable has not been called");
+    return AMP_OK;
+}
+// the listed alleles on the host: {key, count | rev << 32, qsum} per allele, and the list order sorted by key
+static int dels_download(amp_ctx* c, std::vector<unsigned long long>& rec, std::vector<unsigned long long>& order) {
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    unsigned long long n = 0;
+    CK(cudaMemcpy(&n, c->dels.cursor, 8, cudaMemcpyDeviceToHost));
+    rec.assign(3 * n, 0); order.resize(n);
+    for (unsigned long long k = 0; k < n; ++k) order[k] = k;
+    if (n == 0) return AMP_OK;
+    if (int rc = dev_grow(&c->d_xbuf, &c->xbuf_bytes, (size_t)n * 24 + 64)) return rc;
+    amp_dels_gather_kernel<<<(unsigned)std::min<unsigned long long>((n + 255) / 256, 1184), 256>>>(c->dels, n, (unsigned long long*)c->d_xbuf);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(rec.data(), c->d_xbuf, n * 24, cudaMemcpyDeviceToHost));
+    // LSD radix sort by key, 16 bits a pass; a pass whose digit is the same for every key is skipped (the high bits of a length)
+    std::vector<unsigned long long> tmp(n);
+    std::vector<size_t> hist(1 << 16);
+    for (int shift = 0; shift < 64; shift += 16) {
+        std::fill(hist.begin(), hist.end(), 0);
+        for (unsigned long long k = 0; k < n; ++k) ++hist[(rec[3 * order[k]] >> shift) & 0xFFFF];
+        if (hist[(rec[0] >> shift) & 0xFFFF] == n) continue;
+        size_t sum = 0;
+        for (auto& h : hist) { const size_t t = h; h = sum; sum += t; }
+        for (unsigned long long k = 0; k < n; ++k) tmp[hist[(rec[3 * order[k]] >> shift) & 0xFFFF]++] = order[k];
+        order.swap(tmp);
+    }
+    return AMP_OK;
+}
+
+int amp_dels_count(amp_ctx* c, int64_t* n) {
+    if (int rc = dels_check(c, "amp_dels_count")) return rc;
+    if (!n) return fail(AMP_ERR_ARG, "amp_dels_count: null argument");
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    unsigned long long v = 0;
+    CK(cudaMemcpy(&v, c->dels.cursor, 8, cudaMemcpyDeviceToHost));
+    *n = (int64_t)v;
+    return AMP_OK;
+}
+
+int amp_dels_export(amp_ctx* c, int32_t* sample, int32_t* anchor, int32_t* len, int32_t* count, int32_t* rev, int64_t* qsum) {
+    if (int rc = dels_check(c, "amp_dels_export")) return rc;
+    std::vector<unsigned long long> rec, order;
+    if (int rc = dels_download(c, rec, order)) return rc;
+    for (size_t j = 0; j < order.size(); ++j) {
+        const unsigned long long* r = &rec[3 * order[j]];
+        int s, a, l;
+        amp::del_key_split(r[0], c->Lpad, s, a, l);
+        if (sample) sample[j] = s;
+        if (anchor) anchor[j] = a;
+        if (len) len[j] = l;
+        if (count) count[j] = (int32_t)(r[1] & 0xFFFFFFFFULL);
+        if (rev) rev[j] = (int32_t)(r[1] >> 32);
+        if (qsum) qsum[j] = (int64_t)r[2];
+    }
+    return AMP_OK;
+}
+
+int amp_dels_merge(amp_ctx* c, int64_t n, const int32_t* sample, const int32_t* anchor, const int32_t* len, const int32_t* count,
+                   const int32_t* rev, const int64_t* qsum) {
+    if (int rc = dels_check(c, "amp_dels_merge")) return rc;
+    if (n < 0 || (n > 0 && (!sample || !anchor || !len || !count || !rev || !qsum))) return fail(AMP_ERR_ARG, "amp_dels_merge: bad argument");
+    if (n == 0) return AMP_OK;
+    std::vector<unsigned long long> in(3 * (size_t)n);
+    for (int64_t k = 0; k < n; ++k) {
+        if (sample[k] < 0 || sample[k] >= c->cfg.n_samples || anchor[k] < 0 || anchor[k] >= c->cfg.ref_len || len[k] < 1 || count[k] < 0 ||
+            rev[k] < 0 || rev[k] > count[k] || qsum[k] < 0)
+            return fail(AMP_ERR_ARG, "amp_dels_merge: allele out of range");
+        in[3 * k] = amp::del_key(sample[k] * c->Lpad + anchor[k], len[k]);
+        in[3 * k + 1] = (unsigned long long)(unsigned int)count[k] | ((unsigned long long)(unsigned int)rev[k] << 32);
+        in[3 * k + 2] = (unsigned long long)qsum[k];
+    }
+    CK(cudaSetDevice(c->cfg.device));
+    CK(cudaDeviceSynchronize());
+    if (int rc = dev_grow(&c->d_xbuf, &c->xbuf_bytes, (size_t)n * 24 + 64)) return rc;
+    CK(cudaMemcpy(c->d_xbuf, in.data(), (size_t)n * 24, cudaMemcpyHostToDevice));
+    amp_dels_merge_kernel<<<(unsigned)std::min<long long>((n + 127) / 128, (long long)c->sm_count * 4), 128>>>(c->dels, (unsigned long long)n,
+                                                                                                            (const unsigned long long*)c->d_xbuf);
+    CK(cudaGetLastError());
+    CK(cudaDeviceSynchronize());
+    return AMP_OK;
+}
+
+int amp_call_ivar_dels(amp_ctx* c, const amp_ivar_params* p, int32_t* mq, double* pval) {
+    if (int rc = dels_check(c, "amp_call_ivar_dels")) return rc;
+    if (!p) return fail(AMP_ERR_ARG, "amp_call_ivar_dels: null argument");
+    if (!c->d_call) return fail(AMP_ERR_STATE, "amp_call_ivar_dels: amp_call / amp_call_device has not been called");
+    std::vector<unsigned long long> rec, order;
+    if (int rc = dels_download(c, rec, order)) return rc;
+    const unsigned long long n = order.size();
+    c->last_launches = 0;
+    if (n == 0) return AMP_OK;
+    if (int rc = dev_grow(&c->d_dels_out, &c->dels_out_words, (size_t)n * 2)) return rc;
+    amp::IvarDelParams P{};
+    P.L = c->cfg.ref_len; P.Lpad = c->Lpad; P.dels = c->dels; P.n = n;
+    P.depth = (const int*)(c->d_call + c->o_depth);
+    P.min_depth = p->min_depth; P.min_freq = p->min_freq;
+    P.pval = (double*)c->d_dels_out; P.mq = (int*)(c->d_dels_out + n);
+    amp_ivar_dels_kernel<<<(unsigned)((n + 255) / 256), 256>>>(P);
+    CK(cudaGetLastError());
+    c->last_launches = 1;
+    std::vector<int> h_mq(n); std::vector<double> h_pv(n);
+    CK(cudaMemcpy(h_pv.data(), P.pval, n * 8, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(h_mq.data(), P.mq, n * 4, cudaMemcpyDeviceToHost));
+    for (unsigned long long j = 0; j < n; ++j) {
+        if (mq) mq[j] = h_mq[order[j]];
+        if (pval) pval[j] = h_pv[order[j]];
+    }
+    return AMP_OK;
+}
+
+int64_t amp_dels_slot_bytes(int64_t cap_entries) {
+    if (cap_entries < 0) return -1;
+    return 8 + 8 * AMP_XD_WORDS * cap_entries;
+}
+int amp_dels_pack_device(amp_ctx* c, void* dev_slot, int64_t cap_entries, void* stream) {
+    if (int rc = dels_check(c, "amp_dels_pack_device")) return rc;
+    if (!dev_slot || cap_entries < 0) return fail(AMP_ERR_ARG, "amp_dels_pack_device: bad argument");
+    CK(cudaSetDevice(c->cfg.device));
+    amp_dels_pack_kernel<<<c->sm_count, 256, 0, (cudaStream_t)stream>>>(c->dels, (unsigned long long*)dev_slot, (unsigned long long)cap_entries);
+    CK(cudaGetLastError());
+    return AMP_OK;
+}
+int amp_dels_merge_packed(amp_ctx* c, const void* dev_slots, int n_ranks, int my_rank, int64_t cap_entries, void* stream) {
+    if (int rc = dels_check(c, "amp_dels_merge_packed")) return rc;
+    if (!dev_slots || n_ranks < 1 || cap_entries < 0) return fail(AMP_ERR_ARG, "amp_dels_merge_packed: bad argument");
+    CK(cudaSetDevice(c->cfg.device));
+    dim3 grid((unsigned)c->sm_count, (unsigned)n_ranks);
+    amp_dels_merge_packed_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(c->dels, (const unsigned long long*)dev_slots,
+                                                                        (unsigned long long)amp_dels_slot_bytes(cap_entries) / 8, my_rank);
+    CK(cudaGetLastError());
     return AMP_OK;
 }
 

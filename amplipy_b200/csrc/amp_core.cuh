@@ -945,7 +945,8 @@ AMP_HD int ins_table_find(const InsTable& T, int gpos, int len, const Text& text
 
 // ---- pileup plan: walk the (trimmed) CIGAR exactly as update_base_counts walks get_aligned_pairs() ----
 // Sink interface:  match(rpos, q, len)   aligned run (quality filter applied when counting)
-//                  del(rpos, len)        D / N run -> '-' channel, unconditional (714-715)
+//                  del(rpos, len, qa)    D / N run -> '-' channel, unconditional (714-715); qa = query index of the anchor
+//                                        base of a D directly after M / = / X (the op's last base), -1 otherwise (N too)
 //                  ins(pos, s_begin, s_len, q0)   insertion allele = query_seq[s_begin : s_begin + s_len]; q0 = the first
 //                                        inserted base that passed the gates 718 / 722 (s_begin == q0: the key of 735-736)
 // Returns AMP_E_* bits (0 = ok).
@@ -960,6 +961,7 @@ AMP_HD int plan_read(const uint32_t* c, int nc, int pos, int l_seq, const uint8_
     if (pos < 0) return AMP_E_COORD;
     for (int k = 0; k < nc; ++k) if (c_op(c[k]) > OP_X) return AMP_E_CIGAR;
     int q = 0, r = pos, q0 = -1;   // q0 >= 0: an insertion event is open (730-734)
+    bool after_m = false;          // the previous op walked (H and empty ops are skipped) was M / = / X
     // key slice [q0-1 : end) with python's negative-index wrap for q0 == 0
 #define AMP_KEY(end_, at_) do { int b_ = q0 - 1; if (b_ < 0) { b_ += l_seq; if (b_ < 0) b_ = 0; } \
         int e_ = (end_) < l_seq ? (end_) : l_seq; int n_ = e_ - b_; if (n_ < 0) n_ = 0; \
@@ -976,13 +978,15 @@ AMP_HD int plan_read(const uint32_t* c, int nc, int pos, int l_seq, const uint8_
             }
             sink.match(r, q, n);
             q += n; r += n;
+            after_m = true;
+            continue;
         } else if (op == OP_D || op == OP_N) {
             if (r + n > L) return AMP_E_COORD;
             if (q0 >= 0) {                                    // exit (B): key runs to the end of the read
                 if (r == 0) return AMP_E_INS_END;             // None + 1 -> TypeError in the reference
                 AMP_KEY(l_seq, r);
             }
-            sink.del(r, n);
+            sink.del(r, n, op == OP_D && after_m ? q - 1 : -1);
             r += n;
         } else {                                              // I, S, P: pairs (q, None)
             int j = q; const int hi = q + n;
@@ -1002,6 +1006,7 @@ AMP_HD int plan_read(const uint32_t* c, int nc, int pos, int l_seq, const uint8_
             }
             q += n;
         }
+        after_m = false;
     }
 #undef AMP_KEY
     if (q0 >= 0) return AMP_E_INS_END;                        // IndexError at 734

@@ -5,8 +5,11 @@
 //   stats slot = { u64 n_alleles, u64 arena_words,
 //                  {u64 arena word offset, u64 count, u64 ins_qsum, u64 ins_rev | ins_head << 32}[cap_entries],
 //                  arena bytes [cap_arena] }
+//
+//   deletion slot = { u64 n_alleles, {u64 key, u64 count, u64 rev, u64 qsum}[cap_entries] }   (the table of amp_dels.cuh)
 #pragma once
 #include "amp_core.cuh"
+#include "amp_dels.cuh"
 
 namespace amp {
 
@@ -78,6 +81,30 @@ AMP_HD void xq_merge_entry(const InsTable& T, const QStatsSlots& Q, const unsign
     const int len = (int)((const unsigned int*)rec)[1];
     ArenaText t{rec + 8};
     ins_merge_qstats(T, Q, gpos, len, t, (int)e[1], (int)(unsigned int)e[3], e[2], (e[3] >> 32) != 0);
+}
+
+#define AMP_XD_WORDS 4   // u64 words per entry of a deletion slot
+
+// The deletion table as the pack sees it: n alleles.  Returns whether they fit the slot.
+AMP_HD bool xd_pack_size(const DelTable& T, unsigned long long cap_entries, unsigned long long& n) {
+    n = T.cursor[0];
+    return n <= cap_entries;
+}
+// The slot's header word, by one thread.  A table that does not fit packs as empty and sets AMP_E_DELS_FULL.
+AMP_HD void xd_pack_header(const DelTable& T, unsigned long long* slot, bool fits, unsigned long long n) {
+    slot[0] = fits ? n : 0ULL;
+    if (!fits) atomic_or(T.err, AMP_E_DELS_FULL);
+}
+// Entry k of the slot: allele k of the table with its sums.
+AMP_HD void xd_pack_entry(const DelTable& T, unsigned long long* slot, unsigned long long k) {
+    const DelSlot& s = T.slots[T.entries[k]];
+    unsigned long long* e = slot + 1 + AMP_XD_WORDS * k;
+    e[0] = s.key; e[1] = s.cr & 0xFFFFFFFFULL; e[2] = s.cr >> 32; e[3] = s.qsum;
+}
+// Entry k of another rank's slot added to this rank's table.
+AMP_HD void xd_merge_entry(const DelTable& T, const unsigned long long* slot, unsigned long long k) {
+    const unsigned long long* e = slot + 1 + AMP_XD_WORDS * k;
+    del_table_add(T, (int)(e[0] >> 32), (int)(e[0] & 0xFFFFFFFFu), (unsigned int)e[1], (unsigned int)e[2], e[3]);
 }
 
 }  // namespace amp

@@ -7,11 +7,14 @@
 //                  received, 1 to rev when the read is on the reverse strand and the base's phred quality to qsum (A C G T N; the
 //                  '-' row carries no quality, 714-715).  A privatised tile over the CTA's reference window takes what falls in
 //                  it and is flushed with global atomics; whatever falls outside goes straight to global memory.
+//                  cta_qstats<true> also adds every anchored deletion event to the deletion-allele table (amp_dels.cuh).
 //   ivar_position  one thread per (sample, position), after amp_call on its outputs.
+//   ivar_del       one thread per deletion allele, after amp_call on its depths.
 #pragma once
 #include <math.h>
 
 #include "amp_kernels.cuh"
+#include "amp_dels.cuh"
 
 namespace amp {
 
@@ -27,8 +30,11 @@ struct QStatsParams {
     int* ins_rev; unsigned long long* ins_qsum; // per slot
     unsigned char* ins_head;                    // per slot: 1 = an event of this allele is the key of 735-736
     unsigned int* err;
+    DelTable dels;                              // cta_qstats<true> only: the anchored deletion alleles
 };
 
+// DELS: anchored deletion events also go to P->dels (a separate instance, so the pass without the table is unchanged)
+template <bool DELS = false>
 struct QStatsSink {
     const QStatsParams* P; int* trev; int* tq; int wbase;
     const uint8_t* seq; const uint8_t* qual; bool rev; unsigned int errs;
@@ -52,7 +58,13 @@ struct QStatsSink {
             if (ch >= 0) add(ch, rpos + j, qv);                                   // 752-753 (a KeyError is the pileup's to raise)
         }
     }
-    AMP_HD void del(int rpos, int n) { if (rev) for (int j = 0; j < n; ++j) add(5, rpos + j, 0); }   // 714-715
+    AMP_HD void del(int rpos, int n, int qa) {
+        if (rev) for (int j = 0; j < n; ++j) add(5, rpos + j, 0);                                      // 714-715
+        if (DELS && qa >= 0) {                                                    // an anchored deletion (DESIGN.md 3.7)
+            const int aq = qual[qa];
+            if (aq >= P->minq) del_table_add(P->dels, P->gpos_base + rpos - 1, n, 1u, rev ? 1u : 0u, (unsigned long long)aq);
+        }
+    }
     AMP_HD void ins(int pos, int b, int n, int q0) {
         const int eq = qual[q0];                                                  // the first inserted base past 718 / 722
         if (n == 1) {
@@ -81,6 +93,7 @@ AMP_HD bool qstats_row(const QStatsParams& P, long long i, const uint32_t*& cig,
 }
 
 // trev / tq: the tile, 6 x AMP_QS_WT ints each; lo: one shared int
+template <bool DELS = false>
 AMP_HD void cta_qstats(const QStatsParams& P, int* trev, int* tq, int* lo, int block, int nthreads) {
     const long long r0 = P.b.first + (long long)block * AMP_QS_READS;
     long long r1 = r0 + AMP_QS_READS; if (r1 > P.b.first + P.b.n) r1 = P.b.first + P.b.n;
@@ -102,7 +115,7 @@ AMP_HD void cta_qstats(const QStatsParams& P, int* trev, int* tq, int* lo, int b
         for (long long i = r0 + tid; i < r1; i += nthreads) {
             const uint32_t* cig; int nc, pos;
             if (!qstats_row(P, i, cig, nc, pos)) continue;
-            QStatsSink s;
+            QStatsSink<DELS> s;
             s.P = &P; s.trev = trev; s.tq = tq; s.wbase = wbase;
             s.seq = P.b.seq + P.b.seq_off[i]; s.qual = P.b.qual + P.b.qual_off[i];
             s.rev = (P.b.flag[i] & 16) != 0; s.errs = 0;
@@ -292,6 +305,28 @@ AMP_HD void ivar_position(const IvarParams& P, long long gp) {
         if (n > 1) code = has_n ? (unsigned char)'N' : (unsigned char)AMP_IUPAC_CODES[mask];
     }
     P.iupac[gp] = code;
+}
+
+struct IvarDelParams {
+    int L, Lpad;
+    DelTable dels; unsigned long long n;           // the first n listed alleles
+    const int* depth;                              // amp_call's, [n_samples * L]
+    int min_depth; double min_freq;
+    int* mq; double* pval;                         // [n] in list order; pval NaN = no TSV row
+};
+
+// Deletion allele k: mq = floor(qsum / count) and, when it gets a TSV row (D > 0, D >= min_depth, count / D >= min_freq, D the
+// depth at the anchor), PVAL = fisher_less(D, count, mq).
+AMP_HD void ivar_del(const IvarDelParams& P, unsigned long long k) {
+    const DelSlot& s = P.dels.slots[P.dels.entries[k]];
+    int sample, a, len;
+    del_key_split(s.key, P.Lpad, sample, a, len);
+    const long long c = (long long)(s.cr & 0xFFFFFFFFULL);
+    const long long D = P.depth[(size_t)sample * P.L + a];
+    const int mq = c ? (int)(s.qsum / (unsigned long long)c) : 0;
+    P.mq[k] = mq;
+    const bool row = D > 0 && D >= P.min_depth && c && (double)c / (double)D >= P.min_freq;
+    P.pval[k] = row ? fisher_less(D, c, mq) : (double)NAN;
 }
 
 }  // namespace amp

@@ -180,7 +180,7 @@ struct TileSink {
         }
     }
     AMP_HD void match(int rpos, int q, int n) { push(rpos, n, q); }
-    AMP_HD void del(int rpos, int n) { push(rpos, (int)(0x80000000u | (unsigned)n), 0); }
+    AMP_HD void del(int rpos, int n, int /*qa*/) { push(rpos, (int)(0x80000000u | (unsigned)n), 0); }
     struct Text {
         const uint8_t* seq; int b;
         AMP_HD char operator()(int i) const { return nib_char(nib_at(seq, (uint32_t)(b + i))); }
@@ -257,7 +257,7 @@ struct DirectSink {
             }
         }
     }
-    AMP_HD void del(int rpos, int n) { for (int j = 0; j < n; ++j) count_add(*P, sm.cnt, wbase, 5, rpos + j); }   // 714-715
+    AMP_HD void del(int rpos, int n, int /*qa*/ = -1) { for (int j = 0; j < n; ++j) count_add(*P, sm.cnt, wbase, 5, rpos + j); }   // 714-715
     AMP_HD void ins(int pos, int b, int n, int /*q0*/ = 0) {
         if (n == 1) {
             int ch = nib_channel(nib_at(seq_read, (uint32_t)b));
@@ -288,7 +288,7 @@ struct RecordSink {
         if (nrun < AMP_REC_RUNS && q < 65536 && n < 32768) { rp[nrun] = rpos; ql[nrun] = ((uint32_t)q << 16) | (uint32_t)n; ++nrun; steps += n; }
         else d.match(rpos, q, n);
     }
-    AMP_HD void del(int rpos, int n) {
+    AMP_HD void del(int rpos, int n, int /*qa*/) {
         if (nrun < AMP_REC_RUNS && n < 32768) { rp[nrun] = rpos; ql[nrun] = 0x8000u | (uint32_t)n; ++nrun; steps += n; }
         else d.del(rpos, n);
     }

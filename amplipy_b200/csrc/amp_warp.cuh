@@ -467,7 +467,7 @@ struct WarpSink7 {
         }
     }
     AMP_HD void match(int rpos, int q, int n) { push(rpos, n, q); }
-    AMP_HD void del(int rpos, int n) { push(rpos, (int)(0x80000000u | (unsigned)n), 0); }
+    AMP_HD void del(int rpos, int n, int /*qa*/) { push(rpos, (int)(0x80000000u | (unsigned)n), 0); }
     AMP_WD void ins(int pos, int b, int n, int /*q0*/) { ins_defer(*P, wm.ctrl, so0, pos, b, n); }
 };
 

@@ -14,7 +14,8 @@ amp_ins_merge_packed) on a communicator made by ``DeepExchange``; engines withou
 used by the gloo tests) take the torch.distributed form of the same two steps.  An engine with the strand / quality sums
 (``enable_qstats``) exchanges them too: the all-reduce also sums its rev / qsum matrices and every exchanged insertion
 allele carries its ins_rev / ins_qsum / ins_head (the *_qstats entry points), so the iVar outputs of every rank are those
-of one GPU over all the reads.
+of one GPU over all the reads.  An engine with the anchored deletion table (``enable_dels``) also packs, gathers and merges
+that table (amp_dels_pack_device, amp_nccl_allgather, amp_dels_merge_packed; its sums are integers too).
 
 The reference has no counterpart (single sequential loop, AmpliPy.py:896)."""
 import numpy as np
@@ -38,9 +39,10 @@ class DeepExchange:
 
     cap_entries / cap_arena_bytes: capacity of a rank's slot (distinct insertion alleles / bytes of their records); a
     table that does not fit raises the engine's TABLE_FULL / ARENA_FULL error flag.  The engine's strand / quality sums,
-    when it has them at construction (``engine.qstats_enabled``), travel with the counts and the alleles."""
+    when it has them at construction (``engine.qstats_enabled``), travel with the counts and the alleles.  So does its anchored
+    deletion table (``engine.dels_enabled``), in slots of cap_dels alleles; a table that does not fit raises DELS_FULL."""
 
-    def __init__(self, engine, group=None, cap_entries=1 << 16, cap_arena_bytes=4 << 20):
+    def __init__(self, engine, group=None, cap_entries=1 << 16, cap_arena_bytes=4 << 20, cap_dels=1 << 16):
         import torch
         import torch.distributed as dist
         from .engine import NcclComm
@@ -53,6 +55,12 @@ class DeepExchange:
         dev = torch.device("cuda", engine.device)
         self.send = torch.zeros(self.slot_bytes, dtype=torch.uint8, device=dev)
         self.recv = torch.zeros(self.slot_bytes * self.world, dtype=torch.uint8, device=dev)
+        self.dels = getattr(engine, "dels_enabled", False)
+        if self.dels:
+            self.cap_dels = int(cap_dels)
+            self.dels_bytes = engine.dels_slot_bytes(self.cap_dels)
+            self.dels_send = torch.zeros(self.dels_bytes, dtype=torch.uint8, device=dev)
+            self.dels_recv = torch.zeros(self.dels_bytes * self.world, dtype=torch.uint8, device=dev)
         self.comm = NcclComm.from_torch_group(engine.device, group)
 
     def run(self, stream=None):
@@ -66,6 +74,10 @@ class DeepExchange:
         pack(self.send.data_ptr(), self.cap_entries, self.cap_arena, stream)
         self.comm.allgather(self.send.data_ptr(), self.recv.data_ptr(), self.slot_bytes, stream)
         merge(self.recv.data_ptr(), self.world, self.rank, self.cap_entries, self.cap_arena, stream)
+        if self.dels:
+            e.dels_pack_device(self.dels_send.data_ptr(), self.cap_dels, stream)
+            self.comm.allgather(self.dels_send.data_ptr(), self.dels_recv.data_ptr(), self.dels_bytes, stream)
+            e.dels_merge_packed(self.dels_recv.data_ptr(), self.world, self.rank, self.cap_dels, stream)
 
     def close(self):
         self.comm.close()
@@ -105,6 +117,19 @@ def allgather_insertions(engine, group=None):
     return engine.insertions()
 
 
+def allgather_dels(engine, group=None):
+    """torch.distributed form (host arrays) of the deletion-table exchange: every rank's anchored deletion alleles gathered, the
+    others' merged into the local table (engines with ``dels_enabled``)."""
+    import torch.distributed as dist
+    rank = dist.get_rank(group)
+    gathered = [None] * dist.get_world_size(group)
+    dist.all_gather_object(gathered, engine.dels(), group=group)
+    for r, part in enumerate(gathered):
+        if r != rank and len(part.count):
+            engine.merge_dels(part)
+    return engine.dels()
+
+
 def process_deep_sample(engine, batch, trim=True, pileup=True, sample=0, group=None, exchange=None, qstats=False):
     """Read-sharded processing of one sample: local kernel on this rank's read range, then the exchange step.
     Returns this rank's TrimResult (valid for its own range of reads only; the other reads' flags are 0).
@@ -126,4 +151,6 @@ def process_deep_sample(engine, batch, trim=True, pileup=True, sample=0, group=N
         else:
             allreduce_counts(engine, group)
             allgather_insertions(engine, group)
+            if getattr(engine, "dels_enabled", False):
+                allgather_dels(engine, group)
     return t, (first, count)

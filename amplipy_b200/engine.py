@@ -18,7 +18,7 @@ import numpy as np
 
 from .batch import ReadBatch
 from .calling import CallResult, Insertions
-from .ivar import Annotation, IvarResult, QStats
+from .ivar import Annotation, Deletions, IvarResult, QStats
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AMP_LIB_OVERRIDE") or os.path.join(_HERE, "csrc", "libamplipy_b200.so")   # override: tuning experiments only
@@ -31,7 +31,8 @@ DEVERR_NAMES = {1: "read outside the reference (IndexError in AmpliPy.py:450-451
                 8: "CIGAR consumes more query than l_seq / unsupported op",
                 16: "insertion hash table full (raise ins_slots)",
                 32: "insertion string arena full (raise ins_arena_bytes)",
-                64: "strand / quality pass met an insertion allele the pileup did not add"}
+                64: "strand / quality pass met an insertion allele the pileup did not add",
+                128: "anchored deletion table full (raise the slots of enable_dels)"}
 
 EXPORTED_SYMBOLS = [
     "amp_last_error", "amp_abi_version", "amp_create", "amp_destroy", "amp_reset", "amp_error_flags", "amp_lpad",
@@ -44,7 +45,8 @@ EXPORTED_SYMBOLS = [
     "amp_set_scheme", "amp_get_scheme", "amp_set_sample_reference", "amp_qstats_enable", "amp_qstats_host", "amp_call_ivar",
     "amp_call_ivar_device", "amp_contig_plan_decoded", "amp_contig_plan_device", "amp_process_contigs", "amp_set_features",
     "amp_annotate", "amp_annot_host", "amp_allreduce_qstats", "amp_ins_slot_bytes_qstats", "amp_ins_pack_qstats_device",
-    "amp_ins_merge_packed_qstats"]
+    "amp_ins_merge_packed_qstats", "amp_dels_enable", "amp_dels_count", "amp_dels_export", "amp_dels_merge", "amp_call_ivar_dels",
+    "amp_dels_slot_bytes", "amp_dels_pack_device", "amp_dels_merge_packed"]
 
 
 class AmpConfig(ctypes.Structure):
@@ -132,6 +134,8 @@ def load_library():
         lib.amp_last_error.restype = ctypes.c_char_p
         lib.amp_ins_slot_bytes.restype = ctypes.c_int64
         lib.amp_ins_slot_bytes_qstats.restype = ctypes.c_int64
+        if hasattr(lib, "amp_dels_slot_bytes"):       # A/B runs may load a library from before the deletion table
+            lib.amp_dels_slot_bytes.restype = ctypes.c_int64
         for name in EXPORTED_SYMBOLS:
             try:
                 getattr(lib, name)   # AttributeError if the build is stale
@@ -225,6 +229,7 @@ class Engine:
         self.device = device
         self.launches = 0
         self._qstats = False
+        self._dels = False
 
     def close(self):
         if getattr(self, "_ctx", None) is not None and self._ctx.value:
@@ -242,7 +247,7 @@ class Engine:
 
     def reset_async(self, stream=None):
         _check(self.lib.amp_reset_async(self._ctx, ctypes.c_void_p(stream) if stream else None), "amp_reset_async")
-        self.launches += 1            # amp_reset_kernel
+        self.launches += 2 if self._dels else 1      # amp_reset_kernel (+ amp_dels_reset_kernel)
 
     def set_reference(self, ref_seq):
         ref = ref_seq.encode("latin-1") if isinstance(ref_seq, str) else bytes(ref_seq)
@@ -667,6 +672,60 @@ class Engine:
         _check(self.lib.amp_call_ivar_device(self._ctx, ctypes.byref(p), ctypes.c_void_p(stream) if stream else None),
                "amp_call_ivar_device")
         self.launches += int(self.lib.amp_last_launches(self._ctx))
+
+    # ---------------------------------------------------------------- anchored deletion alleles of the iVar TSV (DESIGN.md 3.7)
+    def enable_dels(self, slots=0):
+        """Allocate the anchored deletion table (amp_dels_enable; ``slots`` a power of two, 0 = 2^20) after enable_qstats;
+        process(..., qstats=True) fills it."""
+        _check(self.lib.amp_dels_enable(self._ctx, ctypes.c_int64(int(slots))), "amp_dels_enable")
+        self._dels = True
+
+    @property
+    def dels_enabled(self):
+        """True once enable_dels has succeeded."""
+        return self._dels
+
+    def dels(self, sample=None):
+        """The anchored deletion alleles sorted by (sample, anchor, len) (amp_dels_export); ``sample``: only that sample's."""
+        n = ctypes.c_int64(0)
+        _check(self.lib.amp_dels_count(self._ctx, ctypes.byref(n)), "amp_dels_count")
+        k = int(n.value)
+        d = Deletions(*[np.zeros(max(k, 1), t) for t in (np.int32,) * 5 + (np.int64,)])
+        _check(self.lib.amp_dels_export(self._ctx, _ptr(d.sample), _ptr(d.anchor), _ptr(d.len), _ptr(d.count), _ptr(d.rev), _ptr(d.qsum)),
+               "amp_dels_export")
+        d = d.take(np.arange(k))
+        return d if sample is None else d.take(np.flatnonzero(d.sample == sample))
+
+    def merge_dels(self, d):
+        """Add the alleles of a Deletions (e.g. another rank's) to the table: the host form of the exchange."""
+        a = [np.ascontiguousarray(x, t) for x, t in ((d.sample, np.int32), (d.anchor, np.int32), (d.len, np.int32), (d.count, np.int32),
+                                                     (d.rev, np.int32), (d.qsum, np.int64))]
+        _check(self.lib.amp_dels_merge(self._ctx, ctypes.c_int64(len(a[0])), *[_ptr(x) for x in a]), "amp_dels_merge")
+        self.launches += 1
+
+    def call_ivar_dels(self, min_depth=1, min_freq=0.03):
+        """The alleles of ``dels()`` with mq and PVAL (amp_call_ivar_dels; NaN = no TSV row), on the depths of the last ``call``."""
+        d = self.dels()
+        k = len(d.count)
+        mq, pval = np.zeros(max(k, 1), np.int32), np.full(max(k, 1), np.nan)
+        p = AmpIvarParams(int(min_depth), float(min_freq), 0.0)
+        _check(self.lib.amp_call_ivar_dels(self._ctx, ctypes.byref(p), _ptr(mq), _ptr(pval)), "amp_call_ivar_dels")
+        self.launches += int(self.lib.amp_last_launches(self._ctx))
+        d.mq, d.pval = mq[:k], pval[:k]
+        return d
+
+    def dels_slot_bytes(self, cap_entries):
+        return int(self.lib.amp_dels_slot_bytes(ctypes.c_int64(cap_entries)))
+
+    def dels_pack_device(self, dev_ptr, cap_entries, stream=None):
+        _check(self.lib.amp_dels_pack_device(self._ctx, ctypes.c_void_p(dev_ptr), ctypes.c_int64(cap_entries),
+                                             ctypes.c_void_p(stream) if stream else None), "amp_dels_pack_device")
+        self.launches += 1
+
+    def dels_merge_packed(self, dev_ptr, n_ranks, my_rank, cap_entries, stream=None):
+        _check(self.lib.amp_dels_merge_packed(self._ctx, ctypes.c_void_p(dev_ptr), int(n_ranks), int(my_rank), ctypes.c_int64(cap_entries),
+                                              ctypes.c_void_p(stream) if stream else None), "amp_dels_merge_packed")
+        self.launches += 1
 
     # ---------------------------------------------------------------- codon annotation of the iVar TSV (DESIGN.md 3.9)
     def set_features(self, sample, features):

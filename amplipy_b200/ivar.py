@@ -41,6 +41,24 @@ class IvarResult:
 
 
 @dataclass
+class Deletions:
+    """Anchored deletion alleles (DESIGN.md 3.7, ``Engine.dels``), sorted by (sample, anchor, len); ``mq`` / ``pval`` are filled by
+    ``Engine.call_ivar_dels`` (pval NaN = no TSV row)."""
+    sample: np.ndarray      # i32[K]
+    anchor: np.ndarray      # i32[K] 0-based reference position of the base before the deletion
+    len: np.ndarray         # i32[K] deleted bases
+    count: np.ndarray       # i32[K]
+    rev: np.ndarray         # i32[K] events from reverse-strand reads
+    qsum: np.ndarray        # i64[K] anchor qualities
+    mq: np.ndarray = None   # i32[K] floor(qsum / count)
+    pval: np.ndarray = None  # f64[K]
+
+    def take(self, idx):
+        f = lambda a: None if a is None else a[idx]
+        return Deletions(f(self.sample), f(self.anchor), f(self.len), f(self.count), f(self.rev), f(self.qsum), f(self.mq), f(self.pval))
+
+
+@dataclass
 class Annotation:
     """``amp_annotate`` outputs (DESIGN.md 3.9): the occurrences of (sample, position) gp = sample * L + p, each a (feature, codon)
     pair the position belongs to, are entries [off[gp], off[gp + 1]), in feature order, then in spliced order."""
@@ -86,21 +104,29 @@ def alt_text(sym, ref_char, head=False):
     return "+" + (sym[:-1] if head else sym[1:])
 
 
-def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None, ann=None, names=None):
+def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None, ann=None, names=None, dels=None):
     """The TSV rows of one sample: every allele with a p-value (count > 0, symbol != the FASTA character, freq >= min_freq, depth
     >= min_depth), in position order, then in the reference's allele order (AmpliPy.py:771).  ``L``: the sample's own reference
     length when it is shorter than the context's (a contig of a multi-record FASTA).  ``ann`` (an Annotation) and ``names`` (the
     sample's feature names): a row at a position with k >= 1 occurrences is written k times in a row, once per occurrence, with
-    the six annotation columns appended."""
+    the six annotation columns appended.  ``dels`` (a Deletions from ``Engine.call_ivar_dels``): deletions are written as iVar
+    writes them (DESIGN.md 3.7): the '-' channel gets no rows, and each anchored deletion with a p-value gets one row at its anchor,
+    after the position's ranked alleles, in ascending length."""
     L = res.L if L is None else L
     base = sample * res.L
     fpv = iv.fixed_pval[base:base + L]
+    del_rows = {}
+    if dels is not None:
+        fpv = fpv.copy()
+        fpv[:, 5] = np.nan
+        for k in np.flatnonzero((dels.sample == sample) & ~np.isnan(dels.pval)).tolist():
+            del_rows.setdefault(int(dels.anchor[k]), []).append(k)
     ins_rows = {}
     if ins.k:
         sel = np.flatnonzero((ins.sample == sample) & ~np.isnan(iv.ins_pval[:ins.k]))
         for k in sel.tolist():
             ins_rows.setdefault(int(ins.pos[k]), []).append(k)
-    pos = sorted(set(np.flatnonzero(~np.isnan(fpv).all(axis=1)).tolist()) | set(ins_rows))
+    pos = sorted(set(np.flatnonzero(~np.isnan(fpv).all(axis=1)).tolist()) | set(ins_rows) | set(del_rows))
     out = []
     for p in pos:
         gp = base + p
@@ -119,6 +145,9 @@ def tsv_rows(res, ins, iv, qs, ref_id, ref_seq, counts, sample=0, L=None, ann=No
             alts.append((int(res.ins_rank[k]), alt_text(ins.strs[k], ref_char, bool(qs.ins_head[k])), int(ins.count[k]),
                          int(qs.ins_rev[k]), int(iv.ins_mq[k]), float(iv.ins_pval[k])))
         alts.sort(key=lambda a: a[0])
+        for k in del_rows.get(p, ()):         # dels are sorted by length within a position
+            n = int(dels.len[k])
+            alts.append((None, "-" + ref_seq[p + 1:p + 1 + n], int(dels.count[k]), int(dels.rev[k]), int(dels.mq[k]), float(dels.pval[k])))
         for _, alt, c, rv, mq, pv in alts:
             row = (ref_id, p + 1, ref_char, alt, ref_dp, ref_rv, ref_q, c, rv, mq, c / D, D, pv, pv <= PASS_PVAL)
             cols = ann.columns(sample, p, alt, names) if ann is not None else ()

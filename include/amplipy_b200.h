@@ -52,6 +52,7 @@ extern "C" {
 #define AMP_DEVERR_TABLE_FULL 16
 #define AMP_DEVERR_ARENA_FULL 32
 #define AMP_DEVERR_QSTATS_MISS 64   /* strand / quality pass: an insertion allele the pileup did not add (never expected) */
+#define AMP_DEVERR_DELS_FULL 128    /* anchored deletion table full (amp_dels_enable); the alleles it could not take are lost */
 
 /* mode bits for amp_process_* */
 #define AMP_MODE_TRIM 1      /* trim_read, AmpliPy.py:426-687 (+ gate 902/910) */
@@ -180,6 +181,35 @@ int amp_call_ivar(amp_ctx* ctx, const amp_ivar_params* p, uint8_t* iupac /* [S*L
                   double* fixed_pval /* [S*L*6] */, int32_t* ins_mq, double* ins_pval);
 /* the same kernel on the outputs amp_call_device left in HBM; results stay in context-owned buffers; asynchronous on `stream` */
 int amp_call_ivar_device(amp_ctx* ctx, const amp_ivar_params* p, void* stream);
+
+/* ---- anchored deletion alleles of the iVar TSV (DESIGN.md 3.7, --ivar_deletions).  An allele is (sample, anchor, len): a D op of
+ * len bases directly after an M / = / X op of a read the pileup counted, in the CIGAR row it walked, whose last base (the anchor, at
+ * reference position anchor = the D's start - 1) has quality >= min_quality.  Each carries count, rev (events from reads with flag &
+ * 0x10) and qsum (the anchor qualities).  N ops and a D after S / I / P are not alleles; the '-' channel is unchanged.
+ *   amp_dels_enable        allocate and zero an open-addressing table of `slots` slots (a power of two, rounded up; 0 = 2^20).
+ *                          AMP_ERR_STATE without amp_qstats_enable: the strand / quality pass (AMP_MODE_QSTATS) fills it.  A
+ *                          second call changes nothing.  A full table raises AMP_DEVERR_DELS_FULL.  amp_reset / amp_reset_async
+ *                          clear it.
+ *   amp_dels_count         the number of alleles
+ *   amp_dels_export        the alleles sorted by (sample, anchor, len); any pointer may be NULL
+ *   amp_dels_merge         host alleles added to the table (sums added to an existing allele's); AMP_ERR_ARG when one is out of range
+ *   amp_call_ivar_dels     after amp_call: per allele in export order, mq = floor(qsum / count) and, when it gets a TSV row
+ *                          (D > 0, D >= min_depth, count / D >= min_freq, D = depth at the anchor), PVAL as amp_call_ivar computes
+ *                          it; NaN otherwise.  p->iupac_threshold is not used.
+ * Every entry point returns AMP_ERR_STATE on a context without the table.  The deep-sample exchange of the table:
+ *   amp_dels_slot_bytes    8 + 32 * cap_entries
+ *   amp_dels_pack_device   { u64 n_alleles, {u64 key = (sample * lpad + anchor) << 32 | len, u64 count, u64 rev, u64 qsum}[cap_entries] };
+ *                          a table of more than cap_entries alleles raises AMP_DEVERR_DELS_FULL and packs as empty
+ *   amp_dels_merge_packed  the other ranks' alleles added to this rank's table (amp_nccl_allgather moves the slots) */
+int amp_dels_enable(amp_ctx* ctx, int64_t slots);
+int amp_dels_count(amp_ctx* ctx, int64_t* n_alleles);
+int amp_dels_export(amp_ctx* ctx, int32_t* sample, int32_t* anchor, int32_t* len, int32_t* count, int32_t* rev, int64_t* qsum);
+int amp_dels_merge(amp_ctx* ctx, int64_t n, const int32_t* sample, const int32_t* anchor, const int32_t* len, const int32_t* count,
+                   const int32_t* rev, const int64_t* qsum);
+int amp_call_ivar_dels(amp_ctx* ctx, const amp_ivar_params* p, int32_t* mq, double* pval);
+int64_t amp_dels_slot_bytes(int64_t cap_entries);
+int amp_dels_pack_device(amp_ctx* ctx, void* dev_slot, int64_t cap_entries, void* stream);
+int amp_dels_merge_packed(amp_ctx* ctx, const void* dev_slots, int n_ranks, int my_rank, int64_t cap_entries, void* stream);
 
 /* ---- deep-sample mode: one sample's reads sharded over ranks (SURVEY.md 8e; the reference has no counterpart, its loop
  * AmpliPy.py:896-915 is sequential).  After every rank has processed its read range:
